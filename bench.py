@@ -285,7 +285,11 @@ def main():
     ap.add_argument("--queries", type=int, default=0, help="queries per GPU (default: the configs[1] size, 4096)")
     ap.add_argument("--config5-queries", type=int, default=1 << 20,
                     help="total queries of the sharded config-5 run (strong scaling, part of every line; 0 skips it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's plan records and chains) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     global Q_PER_GPU
     if args.queries > 0:
         Q_PER_GPU = args.queries
@@ -352,6 +356,8 @@ def main():
     sampler.join()
     rec = planner.records_numpy()
     ok = int((rec["status"] == 0).sum())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, rec, planner.chain[:planner.n].cpu().numpy())
 
     # ---- end to end through the host-buffer C ABI (host arrays in, records + chains out)
     e2e_steps = max(2, min(args.steps, 3))
@@ -449,6 +455,26 @@ def main():
     print(json.dumps(line))
     if world_size > 1:
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 63 << 20        # array data of --dump-outputs: under 64 MiB with the .npy headers
+
+
+def dump_outputs(out_dir, rec, chain):
+    """The planner's outputs of the last timed step, one float64 .npy per record field plus `chain` (the stream
+    positions of each plan's nodes, exact in float64) and `query` (the query index of each row).  Above DUMP_BYTES a
+    fixed seeded sample of the queries is written, so that two builds can be compared file for file."""
+    fields = {name: rec[name] for name in rec.dtype.names}
+    fields["chain"] = chain.view(np.uint32)
+    row_bytes = 8 * (1 + sum(int(np.prod(a.shape[1:])) for a in fields.values()))
+    rows = np.arange(len(rec))
+    if len(rows) * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.RandomState(0).choice(len(rows), DUMP_BYTES // row_bytes, replace=False))
+    out = {name: a[rows] for name, a in fields.items()}
+    out["query"] = rows
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 def catalina_parents(world, n, dev, seed=3):

@@ -139,6 +139,17 @@ def stream_block(seed: int, start: int, n: int, f32u: bool = False) -> np.ndarra
     return (z >> np.uint64(11)).astype(np.float64) * (2.0 ** -53)
 
 
+def steer_arc_uniforms(i: int, n: int) -> np.ndarray:
+    """The n uniforms RRT.steer drew in case i of tests/golden/steer_arc.npz (oracle/make_golden.py): Python's own
+    Mersenne Twister seeded with i for i % 5 == 4, else stream 1000 + i from position 0.  Both are exact functions
+    of (i, n), so the golden file stores only the counts."""
+    i = int(i)          # numpy integers overflow in stream_key's arithmetic
+    if i % 5 == 4:
+        r = RecordingRandom(i)
+        return np.array([r.random() for _ in range(n)], dtype=np.float64)
+    return stream_block(1000 + i, 0, n)
+
+
 class StreamPlayer:
     """Stands in for the `random` module inside the reference: plays u_0, u_1, ...
 

@@ -12,10 +12,12 @@ fixture here is an output of the reference's own functions under oracle/harness.
   nn.npz              RRT.get_closest_mps (rrt_dubins.py:505-513) incl. exact ties
   exploring.npz       RRT.exploring traces (rrt_dubins.py:92-176), time-bin mode and NN mode
 """
+import io
 import json
 import math
 import os
 import sys
+import zipfile
 
 import numpy as np
 
@@ -34,6 +36,15 @@ def ragged(list_of_arrays, width):
                             for a in list_of_arrays], axis=0)
             if list_of_arrays else np.zeros((0, width)))
     return off, flat
+
+
+def savez_lzma(path, **arrays):
+    """np.savez with LZMA instead of deflate (np.load reads both): keeps the larger fixtures under 1 MB"""
+    with zipfile.ZipFile(path, "w", compression=zipfile.ZIP_LZMA) as zf:
+        for name, a in arrays.items():
+            buf = io.BytesIO()
+            np.lib.format.write_array(buf, np.asanyarray(a), allow_pickle=False)
+            zf.writestr(name + ".npy", buf.getvalue())
 
 
 def random_state_in_polygon(ref, poly, rs):
@@ -85,6 +96,7 @@ def main():
             new = rrt.steer(parent, 2, 0.5, 30, 0.5, v, True)
             used = (np.array(player.log) if isinstance(player, H.RecordingRandom)
                     else H.stream_block(1000 + i, 0, player.pos))
+            assert np.array_equal(used, H.steer_arc_uniforms(i, len(used)))   # so only the counts are stored
             parents.append([x, y, th, t0, ln])
             velocities.append(v)
             ustreams.append(used.reshape(-1, 1))
@@ -97,9 +109,9 @@ def main():
         mod.random, mod.time = saved
     uoff, uflat = ragged(ustreams, 1)
     woff, wflat = ragged(wps, 6)
-    np.savez_compressed(
+    savez_lzma(
         os.path.join(OUT, "steer_arc.npz"), parents=np.array(parents), velocity=np.array(velocities),
-        params=np.array([2.0, 0.5, 30.0, 0.5]), uoff=uoff, u=uflat[:, 0], leaf=np.array(leaves),
+        params=np.array([2.0, 0.5, 30.0, 0.5]), uoff=uoff, leaf=np.array(leaves),
         nwp=np.array(nwp, dtype=np.int32), woff=woff, wp=wflat,
         safe_fwd=np.array(safe_fwd, dtype=np.uint8), safe_rev=np.array(safe_rev, dtype=np.uint8))
     print("steer: %d edges, %d uniforms, %d waypoints, safe %d / %d (rev %d)" % (
@@ -224,7 +236,7 @@ def main():
                      "cost": None if res is None else res["cost"][0]})
         print(meta[-1])
     ex["meta"] = np.array(json.dumps(meta))
-    np.savez_compressed(os.path.join(OUT, "exploring.npz"), **ex)
+    savez_lzma(os.path.join(OUT, "exploring.npz"), **ex)
 
     # ---- cost ---------------------------------------------------------------------------------
     cost_mod = ref.cost

@@ -41,3 +41,20 @@ def test_main_arm_line():
     assert e["value"] > 0 and e["value"] < d["value"] * 1.05 and e["h2d_bytes_per_step"] > 0 and e["d2h_bytes_per_step"] > 0
     assert d["gpu_launches"] == 3 and d["clocks"]["sm_mhz"] > 0 and isinstance(d["clocks"]["reasons"], list)
     assert "workload" in d["config"] and d["data"] == "synthetic"
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_reproducible(tmp_path):
+    """--dump-outputs writes the last timed step's records and chains as float64 .npy files; two runs with the same
+    arguments write the same arrays"""
+    import numpy as np
+    for run in ("a", "b"):
+        d = _run(["--steps", "2", "--warmup", "0", "--no-extras", "--dump-outputs", str(tmp_path / run)], 900)
+        assert d["steps"] == 2
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and {"chain.npy", "cost.npy", "status.npy", "query.npy"} <= set(names)
+    assert sum(os.path.getsize(tmp_path / "a" / n) for n in names) <= 64 << 20
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float64 and len(a) == 4096 and np.array_equal(a, b), n
+    assert (np.load(tmp_path / "a" / "status.npy") == 0).mean() > 0.9

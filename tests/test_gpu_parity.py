@@ -54,11 +54,12 @@ def test_stream_matches_oracle(api):
 
 # ------------------------------------------------------------------------------------ steer (arc)
 def test_steer_arc_f64_golden(api, golden_dir):
+    from oracle import harness as H
     z = np.load(os.path.join(golden_dir, "steer_arc.npz"))
     n = len(z["parents"])
     for v in np.unique(z["velocity"]):
         sel = np.where(z["velocity"] == v)[0]
-        us = [z["u"][z["uoff"][i]:z["uoff"][i + 1]] for i in sel]
+        us = [H.steer_arc_uniforms(i, int(z["uoff"][i + 1] - z["uoff"][i])) for i in sel]
         uoff = np.concatenate([[0], np.cumsum([len(u) for u in us])])
         params = list(z["params"]) + [v]
         leaf, counts, wp, used, status = api.steer_arc(z["parents"][sel], np.concatenate(us), uoff, params, "f64")

@@ -14,6 +14,7 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 
+import envelope_worlds as ew  # noqa: E402
 from oracle import orc  # noqa: E402  (the checker)
 
 RTOL32 = 1e-5      # fp32 fast build, relative (absolute floor 1e-5 * map scale of 1 m .. 500 m below)
@@ -37,6 +38,22 @@ def env(api, catalina_map, shark_grid):
 def oworld(catalina_map, shark_grid):
     bins, probs = shark_grid
     return orc.OracleWorld.from_map(catalina_map, bins, probs)
+
+
+@pytest.fixture(scope="module")
+def worlds(api, env, oworld):
+    """(Env, OracleWorld, origin) of an envelope world (envelope_worlds.py), built once per module"""
+    cache = {"catalina": (env, oworld, np.zeros(2))}
+
+    def get(name):
+        if name not in cache:
+            w = ew.assert_flags(name)
+            cache[name] = (api.Env(**w), orc.OracleWorld(**w), ew.origin(name))
+        return cache[name]
+    yield get
+    for name, (e, _, _) in cache.items():
+        if name != "catalina":
+            e.close()
 
 
 def close(a, b, rtol, scale=1.0):
@@ -363,10 +380,12 @@ def edge_variant(request, monkeypatch):
     return request.param
 
 
-def test_edges_arc_vs_oracle(api, env, oworld, edge_variant):
+@pytest.mark.parametrize("world", ew.NAMES)
+def test_edges_arc_vs_oracle(api, worlds, world, edge_variant):
+    env, oworld, (ox, oy) = worlds(world)
     rs = np.random.RandomState(8)
     n = 20000
-    parents = np.stack([rs.uniform(-300, -100, n), rs.uniform(-60, 100, n), rs.uniform(-6, 6, n),
+    parents = np.stack([rs.uniform(-300, -100, n) + ox, rs.uniform(-60, 100, n) + oy, rs.uniform(-6, 6, n),
                         rs.uniform(0, 400, n), rs.uniform(0, 500, n)], 1)
     seeds = np.arange(n) + 77
     want_safe, want_nwp, want_leaf = orc.edges_arc_batch(oworld, parents, seeds, velocity=2.0)
@@ -522,13 +541,15 @@ def _flat_steer_draws(u, dist_to_end, diff_max, freq):
     return np.array(flat)
 
 
-def test_edges_arc_cost_vs_oracle(api, env, oworld, edge_variant):
+@pytest.mark.parametrize("world", ew.NAMES)
+def test_edges_arc_cost_vs_oracle(api, worlds, world, edge_variant):
     """config 4 "cost on": the fused steer + collide + cost edge kernel; per-edge cost terms against
     cost.habitat_shark_cost_func restated by the oracle on the oracle's own waypoints"""
     from oracle import harness as H
+    env, oworld, (ox, oy) = worlds(world)
     rs = np.random.RandomState(18)
     n = 1500
-    parents = np.stack([rs.uniform(-300, -100, n), rs.uniform(-60, 100, n), rs.uniform(-6, 6, n),
+    parents = np.stack([rs.uniform(-300, -100, n) + ox, rs.uniform(-60, 100, n) + oy, rs.uniform(-6, 6, n),
                         rs.uniform(0, 520, n), rs.uniform(0, 500, n)], 1)
     seeds = np.arange(n) + 4242
     w3 = -4.0

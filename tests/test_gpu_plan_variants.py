@@ -8,6 +8,7 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 
+import envelope_worlds as ew  # noqa: E402
 from oracle import orc  # noqa: E402
 
 
@@ -64,7 +65,7 @@ def test_parameter_sets_on_catalina(api, catalina_map, shark_grid):
         dict(freq=70.0, dist_to_end=1.0, diff_max=0.9),             # many invalid primitives, 3 chunks of 32
         dict(max_traj_time=498.0),                                  # bin 100 is re-created on every overflow insert (:149-150)
         dict(max_traj_time=123.0, bin_interval=7.0, v=1.0),
-        dict(bin_interval=0.5, max_traj_time=60.0, v=0.5),          # 120 bins: per-bin metadata stays in global memory
+        dict(bin_interval=0.4, max_traj_time=60.0, v=0.5),          # 150 bins: per-bin metadata in global memory (BS = false)
         dict(weights=(0.1, -0.7, 1.3)),
         dict(min_dist=0.0), dict(min_dist=1.5),
         dict(mode=1), dict(mode=1, freq=40.0, max_traj_time=120.0),
@@ -94,6 +95,19 @@ def test_degenerate_worlds(api, catalina_map, shark_grid):
         _compare(api, env, ow, starts, seeds, dict(max_traj_time=150.0), iters=300)
         _compare(api, env, ow, starts, seeds, dict(max_traj_time=150.0, mode=1), iters=150)
         env.close()
+
+
+@pytest.mark.parametrize("world", [w for w in ew.NAMES if w != "catalina"])
+def test_envelope_worlds(api, world):
+    """the envelope worlds (envelope_worlds.py): fp64 traces of every group size in every parent-pick mode, exact"""
+    w = ew.assert_flags(world)
+    env = api.Env(**w)
+    ow = orc.OracleWorld(**w)
+    starts = ew.free_starts(world, 2, 7)
+    I = 96 if world == "huge" else 200
+    for kw in (dict(max_traj_time=150.0), dict(max_traj_time=150.0, mode=1), dict(max_traj_time=150.0, mode=2, max_plan_time=3.0)):
+        _compare(api, env, ow, starts, [5, 6], kw, groups=(32, 16, 8, 1), iters=I)
+    env.close()
 
 
 def test_trees_that_cannot_grow(api, catalina_map, shark_grid):

@@ -73,7 +73,7 @@ EXPORTS = [
     "auvrrt_cost_point", "auvrrt_edges_dubins_dev", "auvrrt_edges_arc_dev", "auvrrt_edges_dubins",
     "auvrrt_edges_arc", "auvrrt_stream_u", "auvrrt_plan_batch", "auvrrt_plan_workspace_bytes", "auvrrt_plan_workspace_bytes_q",
     "auvrrt_plan_batch_dev", "auvrrt_materialize", "auvrrt_calibrate_fp32", "auvrrt_occupancy_dims", "auvrrt_occupancy_grid",
-    "auvrrt_gym_create", "auvrrt_gym_destroy", "auvrrt_gym_grid_shape", "auvrrt_gym_reset", "auvrrt_gym_step",
+    "auvrrt_gym_create", "auvrrt_gym_destroy", "auvrrt_gym_grid_shape", "auvrrt_gym_reset", "auvrrt_gym_reset_dev", "auvrrt_gym_step",
     "auvrrt_gym_step_dev", "auvrrt_gym_tree", "auvrrt_gym_counts", "auvrrt_gym_counts_dev", "auvrrt_gym_path",
     "auvrrt_astar_env_create", "auvrrt_astar_env_destroy", "auvrrt_astar_batch", "auvrrt_astar_workspace_bytes",
     "auvrrt_astar_batch_dev", "auvrrt_edges_arc_cost_dev", "auvrrt_edges_arc_cost", "auvrrt_env_host_blob",
@@ -151,6 +151,7 @@ def lib():
     L.auvrrt_gym_destroy.restype = None
     L.auvrrt_gym_grid_shape.argtypes = [vp, _ip, _ip]
     L.auvrrt_gym_reset.argtypes = [vp, _dp, _dp, _u64p]
+    L.auvrrt_gym_reset_dev.argtypes = [vp, vp, vp, vp, vp, vp]
     L.auvrrt_gym_step.argtypes = [vp, _i32p, C.c_int, C.c_int, vp]
     L.auvrrt_gym_step_dev.argtypes = [vp, vp, C.c_int, C.c_int, vp, vp]
     L.auvrrt_gym_tree.argtypes = [vp, C.c_int64, C.c_int32, _dp, _i32p, _i32p, _i32p, _i32p, _i32p]

@@ -100,3 +100,71 @@ def edges_arc_dev(env: Env, parents, seeds, params5, out_safe, out_counts, out_l
     check(lib().auvrrt_edges_arc_dev(env.handle, _vp(parents), _vp(seeds), parents.shape[0], p,
                                      _prec(precision), _vp(out_safe), _vp(out_counts), _vp(out_leaf),
                                      _stream_ptr(stream)))
+
+
+# ---- vectorised gym_rrt episodes (csrc/gym.cu) -----------------------------------------------------------------
+
+def _need(name, t, dtypes, shape, device):
+    if not isinstance(t, torch.Tensor):
+        raise ValueError("%s must be a torch tensor, got %s" % (name, type(t).__name__))
+    if t.device != device:
+        raise ValueError("%s must be on %s, got %s" % (name, device, t.device))
+    if t.dtype not in dtypes:
+        raise ValueError("%s must be %s, got %s" % (name, " or ".join(str(d) for d in dtypes), t.dtype))
+    if tuple(t.shape) != tuple(shape):
+        raise ValueError("%s must have shape %s, got %s" % (name, tuple(shape), tuple(t.shape)))
+    if not t.is_contiguous():
+        raise ValueError("%s must be contiguous" % name)
+
+
+def _gym_device(batch):
+    return torch.device("cuda", batch.device)
+
+
+def gym_reset_dev(batch, mask, starts, goals, seeds, stream=None):
+    """Planner_RRT.__init__ for the episodes of `batch` (a gym.GymBatch) with mask[q] != 0, in place, enqueued on
+    `stream` (default: the current stream).  mask: bool or uint8 [Q], or None for every episode (a full reset);
+    starts float64 [Q, 3]; goals float64 [Q, 2]; seeds int64 or uint64 [Q] (bit patterns of the uint64 seeds).
+    Rows of episodes outside the mask are not read.  A masked reset clears only the cells the episode's previous
+    tree occupied, and needs one full reset of the batch before it."""
+    dev, Q = _gym_device(batch), batch.Q
+    if mask is not None:
+        _need("mask", mask, (torch.bool, torch.uint8), (Q,), dev)
+    _need("starts", starts, (torch.float64,), (Q, 3), dev)
+    _need("goals", goals, (torch.float64,), (Q, 2), dev)
+    _need("seeds", seeds, (torch.int64, torch.uint64), (Q,), dev)
+    check(lib().auvrrt_gym_reset_dev(batch.handle, _vp(mask), _vp(starts), _vp(goals), _vp(seeds),
+                                     _stream_ptr(stream if stream is not None else torch.cuda.current_stream(dev))))
+
+
+def gym_step_dev(batch, actions, records, stream=None, *, full_candidates=False):
+    """One RRTEnv.step for every episode of `batch`, enqueued on `stream`: actions int32 [Q] flat sub-cell ids
+    (-1 or an empty cell: nothing happens, no draw), or None for one Planner_RRT.planning step; records uint8
+    [Q, 88] (gym.GYM_RECORD_DTYPE rows) or None."""
+    dev, Q = _gym_device(batch), batch.Q
+    if actions is not None:
+        _need("actions", actions, (torch.int32,), (Q,), dev)
+    if records is not None:
+        _need("records", records, (torch.uint8,), (Q, C.sizeof(_lib.GymRecord)), dev)
+    check(lib().auvrrt_gym_step_dev(batch.handle, _vp(actions), 1, int(bool(full_candidates)), _vp(records),
+                                    _stream_ptr(stream if stream is not None else torch.cuda.current_stream(dev))))
+
+
+class _CountsArray:
+    """the library's resident counts array as a __cuda_array_interface__ object; it holds the batch so that the
+    handle outlives every tensor built on it (until batch.close())"""
+
+    def __init__(self, batch, ptr):
+        self.batch = batch
+        self.__cuda_array_interface__ = {"shape": (batch.Q, batch.n_subcells), "typestr": "<u2",
+                                         "data": (int(ptr), False), "version": 3}
+
+
+def gym_counts_tensor(batch):
+    """Zero-copy torch.uint16 view [Q, n_subcells] of the node count of every sub-cell of every episode
+    (RRTEnv.convert_rrt_grid_to_1D_num_of_nodes_only), resident on the device.  It is the library's own array:
+    every step and reset writes it in place.  The batch must have been created with track_counts=True."""
+    ptr = batch.counts_device_ptr()
+    if not ptr:
+        raise ValueError("gym_counts_tensor: the batch was created without track_counts")
+    return torch.as_tensor(_CountsArray(batch, ptr), device=_gym_device(batch))

@@ -9,6 +9,7 @@
 // open-addressing table per episode; the goal-arc test is done by the whole warp, arc by arc.
 //
 //   k_gym_reset   Planner_RRT.__init__ (:34-74): node 0, its sub-cell, occupied list, counts
+//   k_gym_reset_masked  the same for the episodes a mask selects, clearing only the cells their last tree held
 //   k_gym_run     n_steps x generate_one_node (:198-238), cell from random.choice (planning,
 //                 :157-196) or from the agent's action (RRTEnv.step)
 //   k_gym_path    generate_final_course (:318-328): waypoints are not stored; each node keeps the
@@ -34,6 +35,7 @@ struct auvrrt_gym {
     int32_t *d_actions;
     auvrrt_gym_record_t *d_recs;
     cudaStream_t stream;
+    bool reset_once;               // a full reset has been enqueued: every episode's state is defined
 };
 
 namespace auv {
@@ -237,11 +239,11 @@ template <typename R> __device__ __forceinline__ void gym_arc_point(const R arc[
 #define OC(i) S.occ[(size_t)q * (size_t)P.cap + (size_t)(i)]
 #define HT(h) S.hash[(size_t)q * (size_t)P.hsize + (size_t)(h)]
 
+// Planner_RRT.__init__ for episode q on a clean hash table and counts row (the writes k_gym_reset and
+// k_gym_reset_masked share)
 template <typename R>
-__global__ void __launch_bounds__(128) k_gym_reset(GymP<R> P, GymS<R> S, const double *starts, const double *goals,
-                                                   const uint64_t *seeds) {
-    const long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    if (q >= P.Q) return;
+__device__ __forceinline__ void gym_init_episode(const GymP<R> &P, const GymS<R> &S, long long q, const double *starts,
+                                                 const double *goals, const uint64_t *seeds) {
     const R x = (R)starts[3 * q], y = (R)starts[3 * q + 1], th = (R)starts[3 * q + 2];
     S.gx[q] = (R)goals[2 * q]; S.gy[q] = (R)goals[2 * q + 1];
     S.key[q] = stream_key(seeds[q]);
@@ -261,6 +263,14 @@ __global__ void __launch_bounds__(128) k_gym_reset(GymP<R> P, GymS<R> S, const d
     S.status[q] = c == -2 ? AUVRRT_ST_KEY_ERROR : AUVRRT_ST_OK;
 }
 
+template <typename R>
+__global__ void __launch_bounds__(128) k_gym_reset(GymP<R> P, GymS<R> S, const double *starts, const double *goals,
+                                                   const uint64_t *seeds) {
+    const long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (q >= P.Q) return;
+    gym_init_episode<R>(P, S, q, starts, goals, seeds);
+}
+
 // occupied-cell lookup: open-addressing table per episode (key = sub-cell id + 1, 0 = empty; value = index into the
 // occupied list).  Replaces a linear scan of occupied_grid_cells_array, which streamed ~n_occ/2 rows per step.
 template <typename R>
@@ -272,6 +282,32 @@ __device__ __forceinline__ int gym_occ_find(const GymP<R> &P, const GymS<R> &S, 
         if (k == c + 1) { slot = h; return HT(h).val; }
         h = (h + 1) & (unsigned)(P.hsize - 1);
     }
+}
+
+// Planner_RRT.__init__ for the episodes with mask[q] != 0, in place: a vectorised environment resets each episode
+// when it ends instead of waiting for all Q.  Everything the previous episode wrote outside its own rows is undone
+// at the cells it occupied, so the cost is O(n_occ) and not O(ncells + hsize):
+//  - counts: only the sub-cells in the occupied list are non-zero (k_gym_run counts a node only in a cell it has
+//    put in that list), so those entries are zeroed;
+//  - hash: linear probing that never deletes means a key's probe path crosses only slots filled before it, and the
+//    occupied list is in insertion order, so clearing keys from the LAST occupied cell to the first, each found by
+//    the ordinary probe, always finds it with every earlier key still in place.  This keeps k_gym_run as it is
+//    (recording each key's slot at insertion would cost it a store per new cell).
+// Node and occupied-list rows are not cleared: n_nodes / n_occ bound every read of them.  An episode's state must
+// have been written by an earlier full reset (the host side refuses a masked call before one).
+template <typename R>
+__global__ void __launch_bounds__(128) k_gym_reset_masked(GymP<R> P, GymS<R> S, const uint8_t *mask, const double *starts,
+                                                          const double *goals, const uint64_t *seeds) {
+    const long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (q >= P.Q || !mask[q]) return;
+    for (int i = S.n_occ[q] - 1; i >= 0; i--) {
+        const int c = OC(i).cell;
+        unsigned slot;
+        gym_occ_find<R>(P, S, q, c, slot);
+        HT(slot).key = 0;
+        if (S.counts) S.counts[(size_t)q * P.ncells + c] = 0;
+    }
+    gym_init_episode<R>(P, S, q, starts, goals, seeds);
 }
 
 #ifndef AUV_GYM_MINB
@@ -529,6 +565,16 @@ static int gym_reset_t(auvrrt_gym *g, const double *d_starts, const double *d_go
 }
 
 template <typename R>
+static int gym_reset_masked_t(auvrrt_gym *g, const uint8_t *d_mask, const double *d_starts, const double *d_goals,
+                              const uint64_t *d_seeds, cudaStream_t s) {
+    const GymS<R> &S = *(const GymS<R> *)g->S;
+    k_gym_reset_masked<R><<<(unsigned)((g->Q + 127) / 128), 128, 0, s>>>(make_gymp<R>(g), S, d_mask, d_starts, d_goals, d_seeds);
+    g_launches++;
+    AUV_CUDA(cudaGetLastError());
+    return AUVRRT_OK;
+}
+
+template <typename R>
 static int gym_run_t(auvrrt_gym *g, const int32_t *d_actions, int n_steps, int full, auvrrt_gym_record_t *d_recs, cudaStream_t s) {
     const GymS<R> &S = *(const GymS<R> *)g->S;
     k_gym_run<R><<<(unsigned)((g->Q + 127) / 128), 128, sizeof(R) * 3 * (size_t)(g->K > 0 ? g->K : 1), s>>>(
@@ -594,6 +640,7 @@ extern "C" int auvrrt_gym_create(const double *circles, int K, const auvrrt_gym_
     if (!g) return set_err(AUVRRT_ERR_ARG, "gym_create: out of memory");
     g->device = device; g->precision = precision; g->Q = Q; g->p = *params; g->K = K;
     g->d_all = nullptr; g->d_circ = nullptr; g->S = nullptr; g->d_actions = nullptr; g->d_recs = nullptr; g->stream = nullptr;
+    g->reset_once = false;
     // discretize_env (:77-93): int(env_height) // int(cell_side_length)
     const long long cs = (long long)params->cell_side, hh = (long long)(params->y1 - params->y0), ww = (long long)(params->x1 - params->x0);
     if (cs <= 0 || hh < cs || ww < cs) { delete g; return set_err(AUVRRT_ERR_ARG, "gym_create: int(cell_side) must be >= 1 and the boundary at least one cell wide (ZeroDivisionError / IndexError in the reference)"); }
@@ -644,6 +691,20 @@ extern "C" int auvrrt_gym_reset(auvrrt_gym_t *g, const double *starts, const dou
     e = cudaStreamSynchronize(g->stream);
     cudaFree(d);
     if (rc == AUVRRT_OK && e != cudaSuccess) rc = set_err(AUVRRT_ERR_CUDA, "gym_reset: %s", cudaGetErrorString(e));
+    if (rc == AUVRRT_OK) g->reset_once = true;
+    return rc;
+}
+
+extern "C" int auvrrt_gym_reset_dev(auvrrt_gym_t *g, const uint8_t *d_mask, const double *d_starts, const double *d_goals,
+                                    const uint64_t *d_seeds, void *stream) {
+    if (!g || !d_starts || !d_goals || !d_seeds) return set_err(AUVRRT_ERR_ARG, "gym_reset_dev: null argument");
+    if (d_mask && !g->reset_once)
+        return set_err(AUVRRT_ERR_ARG, "gym_reset_dev: a masked reset reads each episode's previous tree, which is undefined "
+                                       "until the handle has had one full reset (d_mask = NULL or auvrrt_gym_reset)");
+    AUV_CUDA(cudaSetDevice(g->device));
+    const int rc = d_mask ? GYM_DISPATCH(g, gym_reset_masked_t, g, d_mask, d_starts, d_goals, d_seeds, (cudaStream_t)stream)
+                          : GYM_DISPATCH(g, gym_reset_t, g, d_starts, d_goals, d_seeds, (cudaStream_t)stream);
+    if (rc == AUVRRT_OK && !d_mask) g->reset_once = true;
     return rc;
 }
 

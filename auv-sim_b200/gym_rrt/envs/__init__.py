@@ -1,1 +1,1 @@
-from gym_rrt.envs.rrt_env import RRTEnv, VecRRTEnv  # noqa: F401
+from gym_rrt.envs.rrt_env import DeviceVecRRTEnv, RRTEnv, VecRRTEnv  # noqa: F401

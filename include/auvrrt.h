@@ -315,6 +315,12 @@ void auvrrt_gym_destroy(auvrrt_gym_t *g);
 int auvrrt_gym_grid_shape(const auvrrt_gym_t *g, int *rows, int *cols);
 /* Planner_RRT.__init__ for every episode: starts [Q][3] = x, y, theta; goals [Q][2]; seeds [Q] */
 int auvrrt_gym_reset(auvrrt_gym_t *g, const double *starts, const double *goals, const uint64_t *seeds);
+/* Planner_RRT.__init__ for the episodes with d_mask[q] != 0 (d_mask == NULL: all, as auvrrt_gym_reset), on device
+ * buffers d_starts [Q][3], d_goals [Q][2] (double), d_seeds [Q]; rows of episodes outside the mask are not read.
+ * Asynchronous on `stream`.  Clears only what the episode's previous tree occupied.  A masked call needs one
+ * earlier full reset of the handle (AUVRRT_ERR_ARG otherwise). */
+int auvrrt_gym_reset_dev(auvrrt_gym_t *g, const uint8_t *d_mask, const double *d_starts, const double *d_goals,
+                         const uint64_t *d_seeds, void *stream);
 /* n_steps generate_one_node calls per episode, stopping early at done.  actions == NULL: the cell
  * is drawn with random.choice(occupied_grid_cells_array) (Planner_RRT.planning, :157-196);
  * else actions[Q] flat sub-cell ids (n_steps must be 1): RRTEnv.step; an empty cell does nothing.

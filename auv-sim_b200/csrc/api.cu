@@ -811,6 +811,9 @@ extern "C" int auvrrt_plan_batch_dev(const auvrrt_env_t *env, const void *starts
                                      void *out_path, const auvrrt_plan_trace_t *trace, void *stream) {
     AUV_TRY(check_precision(precision));
     if (!env || !params) return set_err(AUVRRT_ERR_ARG, "plan_batch: NULL env or params");
+    // the in-kernel path writer walks the chain buffer: without one no path would be written
+    if (out_path && params->path_cap > 0 && !out_chain)
+        return set_err(AUVRRT_ERR_ARG, "plan_batch: out_path needs out_chain");
     cudaStream_t s = (cudaStream_t)stream;
     if (precision == AUVRRT_F32)
         return launch_plan<float>(env, (const float *)starts, seeds, Q, params, workspace, workspace_bytes, out_records, out_chain, (float *)out_path, trace, s);
@@ -940,6 +943,14 @@ extern "C" int auvrrt_materialize(const auvrrt_env_t *env, const double *starts,
     AUV_TRY(need_device(env->device));
     if (Q <= 0) return AUVRRT_OK;
     if (params->path_cap < 1) return set_err(AUVRRT_ERR_ARG, "materialize: path_cap must be >= 1");
+    if (params->group != 0 && params->group != 32 && params->group != 16 && params->group != 8 && params->group != 1)
+        return set_err(AUVRRT_ERR_ARG, "materialize: group must be 32, 16, 8 or 1");
+    // a chain holds chain_cap positions: a record of an overflowed plan (depth > chain_cap) cannot be re-created
+    if (!starts || !seeds || !chain || !depth || !out_path || !out_n_path) return set_err(AUVRRT_ERR_ARG, "materialize: NULL buffer");
+    for (int64_t q = 0; q < Q; q++)
+        if (depth[q] < 0 || depth[q] > params->chain_cap)
+            return set_err(AUVRRT_ERR_ARG, "materialize: depth[%lld] = %d outside [0, chain_cap = %d]", (long long)q, depth[q],
+                           params->chain_cap);
     return precision == AUVRRT_F32 ? materialize_host<float>(env, starts, seeds, chain, depth, Q, params, out_path, out_n_path)
                                    : materialize_host<double>(env, starts, seeds, chain, depth, Q, params, out_path, out_n_path);
 }

@@ -307,6 +307,7 @@ __device__ __forceinline__ void slowq_drain(const EnvView<R> &env, const SlowQ &
 // what one thread carries along an edge
 template <typename R> struct ArcEdge {
     R x, y, th, t, len;
+    R vt;                      // velocity_temp of the last valid primitive (the v column of a path row)
     R sin0, cos0;              // fp64 build: sin / cos of the heading the next primitive starts from
     int nwp;                   // len(new.path): appended waypoints + 1 (path[0] = parent)
     bool bad, moved, degenerate, last_is_wp;
@@ -341,7 +342,7 @@ template <typename R, bool ALLPAIRS, bool FASTENV = false, bool GRIDS = false, b
 __device__ __forceinline__ void arc_edge_begin(const EnvView<R> &env, const CircTable &ct, ArcEdge<R> &e, R px, R py, R pth,
                                                R pt, R plen, R parent_self_s2, int parent_self_hab, const SlowQ sq = SlowQ()) {
     typedef typename Policy<R>::A A;
-    e.x = px; e.y = py; e.th = pth; e.t = pt; e.len = plen;
+    e.x = px; e.y = py; e.th = pth; e.t = pt; e.len = plen; e.vt = 0;
     e.sin0 = 0; e.cos0 = 0;
     if (Policy<R>::VERIFY) A::sincos(pth, &e.sin0, &e.cos0);
     e.nwp = 1; e.moved = false; e.degenerate = false; e.last_is_wp = false;
@@ -408,6 +409,7 @@ __device__ __forceinline__ bool arc_edge_step(const EnvView<R> &env, const CircT
         e.len += movement;
     }
     e.moved = true;
+    e.vt = vt;
     e.last_is_wp = movement >= sp.min_dist;                                          // :283
     if (e.last_is_wp) {
         e.nwp++;

@@ -790,16 +790,25 @@ int launch_plan(const auvrrt_env *env, const R *starts, const uint64_t *seeds, i
     if (G == 8) return launch_plan_g<R, 8>(env, starts, seeds, Q, p, workspace, workspace_bytes, records, chain, path, trace, s, nullptr);
     return set_err(AUVRRT_ERR_ARG, "plan: group must be 32, 16, 8 or 1");
 }
+// Q <= 0: a batch of any size.  Group 0 lets launch_plan pick the kernel per batch (by its size and whether paths are
+// written), so the workspace must hold the largest one it can pick for a batch of at most Q queries.
 template <typename R>
 int64_t plan_workspace_bytes(const auvrrt_env *env, const auvrrt_plan_params_t *p, int64_t Q) {
     int64_t need = -1;
-    int G = p->group ? p->group : ((Q >= 32768 && p->mode != 3) ? 1 : 32), rc;
+    int rc;
+    const int G = p->group ? p->group : 32;
     if (G == 1) rc = launch_plan_tpt<R>(env, nullptr, nullptr, Q, p, nullptr, 0, nullptr, nullptr, nullptr, 0, &need);
     else if (G == 32) rc = launch_plan_g<R, 32>(env, nullptr, nullptr, 0, p, nullptr, 0, nullptr, nullptr, nullptr, nullptr, 0, &need);
     else if (G == 16) rc = launch_plan_g<R, 16>(env, nullptr, nullptr, 0, p, nullptr, 0, nullptr, nullptr, nullptr, nullptr, 0, &need);
     else if (G == 8) rc = launch_plan_g<R, 8>(env, nullptr, nullptr, 0, p, nullptr, 0, nullptr, nullptr, nullptr, nullptr, 0, &need);
     else { set_err(AUVRRT_ERR_ARG, "plan: group must be 32, 16, 8 or 1"); return -1; }
-    return rc ? -1 : need;
+    if (rc) return -1;
+    if (p->group == 0 && p->mode != 3 && (Q <= 0 || Q >= 32768)) {
+        int64_t tpt = -1;
+        if (launch_plan_tpt<R>(env, nullptr, nullptr, Q, p, nullptr, 0, nullptr, nullptr, nullptr, 0, &tpt)) return -1;
+        if (tpt > need) need = tpt;
+    }
+    return need;
 }
 template int launch_plan<float>(const auvrrt_env *, const float *, const uint64_t *, int64_t, const auvrrt_plan_params_t *,
                                 void *, int64_t, auvrrt_plan_record_t *, uint32_t *, float *, const auvrrt_plan_trace_t *, cudaStream_t);
@@ -816,9 +825,19 @@ int launch_materialize(const auvrrt_env *env, const R *starts, const uint64_t *s
     PlanP<R> P;
     int rc = make_planp<R>(env, p, &P);
     if (rc) return rc;
-    int64_t blocks = (Q + 3) / 4;
+    // the evaluator of the planner that made the chains: the fp32 group sizes sum an edge's primitives in their own order
+    const int G = p->group ? p->group : 32;
+    if (G == 1) {
+        if (p->mode == 3) return set_err(AUVRRT_ERR_UNSUPPORTED, "materialize: mode 3 has no thread-per-tree plans");
+        return launch_materialize_tpt<R>(env, starts, seeds, chain, depth, Q, P, path, n_path, s);
+    }
+    int64_t blocks = (Q * G + 127) / 128;
     if (blocks > AUV_SMS * 8) blocks = AUV_SMS * 8;
-    k_materialize<R, 32><<<(unsigned)blocks, 128, 0, s>>>(env_blob<R>(env).blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
+    const unsigned char *blob = env_blob<R>(env).blob;
+    if (G == 32) k_materialize<R, 32><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
+    else if (G == 16) k_materialize<R, 16><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
+    else if (G == 8) k_materialize<R, 8><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
+    else return set_err(AUVRRT_ERR_ARG, "materialize: group must be 32, 16, 8 or 1");
     AUV_LAUNCH_CHECK2();
     return AUVRRT_OK;
 }

@@ -96,5 +96,9 @@ int launch_plan_tpt(const auvrrt_env *env, const R *starts, const uint64_t *seed
                     const auvrrt_plan_params_t *p, void *workspace, int64_t workspace_bytes,
                     auvrrt_plan_record_t *records, uint32_t *chain, const auvrrt_plan_trace_t *trace,
                     cudaStream_t s, int64_t *need_bytes);
+// paths of its plans, re-created with its own edge evaluator
+template <typename R>
+int launch_materialize_tpt(const auvrrt_env *env, const R *starts, const uint64_t *seeds, const uint32_t *chain,
+                           const int32_t *depth, int64_t Q, const PlanP<R> &P, R *path, int32_t *n_path, cudaStream_t s);
 
 }  // namespace auv

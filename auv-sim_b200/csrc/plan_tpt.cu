@@ -399,6 +399,68 @@ int launch_plan_tpt(const auvrrt_env *env, const R *starts, const uint64_t *seed
     if (e != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "plan_tpt launch: %s", cudaGetErrorString(e));
     return AUVRRT_OK;
 }
+// ---- re-create paths of thread-per-tree plans from (start, seed, chain of stream positions) ----------------------
+// One thread per query, with the edge evaluator k_plan_tpt grew the tree with (arc_edge_step): in fp32 the warp
+// evaluator of plan.cu sums the same primitives in another order, so its waypoints, and from the first waypoint count
+// that differs on the whole path, would not be the plan that was scored.
+template <typename R>
+__global__ void __launch_bounds__(128)
+k_materialize_tpt(const unsigned char *blob, const R *starts, const uint64_t *seeds, const uint32_t *chain,
+                  const int32_t *depth, long long Q, PlanP<R> P, R *path_out, int32_t *n_path_out) {
+    EnvView<R> env;
+    env.bind(blob, blob);
+    env.bind_grid(blob, blob);
+    CircTable ct; ct.pair = nullptr; ct.npair = 0; ct.ox = ct.oy = ct.ccmax = 0.f; ct.rmax1 = 1.f; ct.buf2 = false;
+    ct.hpair = nullptr; ct.nhpair = 0; ct.hccmax = 0.f; ct.epair = nullptr; ct.nepair = 0; ct.escale = 0.f; ct.eoff = 0.f;
+    for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x) {
+        const uint64_t key = stream_key(seeds[q]);
+        R x = starts[5 * q], y = starts[5 * q + 1], th = starts[5 * q + 2], t = starts[5 * q + 3], len = starts[5 * q + 4];
+        R *rows = path_out + (size_t)q * P.path_cap * 6;
+        int n_path = 0;
+        const int d = depth[q];
+        auto put = [&](R vx, R vy, R vth, R vv, R vtt, R vlen) {
+            if (n_path < P.path_cap) {
+                R *w = rows + 6 * (size_t)n_path;
+                w[0] = vx; w[1] = vy; w[2] = vth; w[3] = vv; w[4] = vtt; w[5] = vlen;
+            }
+            n_path++;
+        };
+        for (int e = 0; e < d; e++) {
+            put(x, y, th, (R)0, t, len);
+            SerialStream<R> rng;
+            rng.seek(key, chain[(size_t)q * P.chain_cap + e]);           // the edge's n_expand draw comes next
+            const int n_exp = (int)Policy<R>::A::floor(uniform_ab<R>((R)0, P.sp.freq, rng.next()));
+            ArcEdge<R> ed;
+            arc_edge_begin<R, false>(env, ct, ed, x, y, th, t, len, (R)0, -1);
+            for (int k = 0; k < n_exp; k++) {
+                const int nwp = ed.nwp;
+                if (!arc_edge_step<R, false, false, false>(env, ct, P.sp, P.w3, rng, ed)) break;
+                if (ed.nwp > nwp) put(ed.x, ed.y, ed.th, ed.vt, ed.t, ed.len);
+            }
+            x = ed.x; y = ed.y; th = ed.th; t = ed.t; len = ed.len;
+        }
+        if (d >= 0) put(x, y, th, (R)0, t, len);
+        n_path_out[q] = n_path;
+    }
+}
+
+template <typename R>
+int launch_materialize_tpt(const auvrrt_env *env, const R *starts, const uint64_t *seeds, const uint32_t *chain,
+                           const int32_t *depth, int64_t Q, const PlanP<R> &P, R *path, int32_t *n_path, cudaStream_t s) {
+    int64_t blocks = (Q + 127) / 128;
+    if (blocks > AUV_SMS * 8) blocks = AUV_SMS * 8;
+    k_materialize_tpt<R><<<(unsigned)blocks, 128, 0, s>>>(env_blob<R>(env).blob, starts, seeds, chain, depth, (long long)Q, P,
+                                                          path, n_path);
+    g_launches++;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "materialize_tpt launch: %s", cudaGetErrorString(e));
+    return AUVRRT_OK;
+}
+template int launch_materialize_tpt<float>(const auvrrt_env *, const float *, const uint64_t *, const uint32_t *, const int32_t *,
+                                           int64_t, const PlanP<float> &, float *, int32_t *, cudaStream_t);
+template int launch_materialize_tpt<double>(const auvrrt_env *, const double *, const uint64_t *, const uint32_t *, const int32_t *,
+                                            int64_t, const PlanP<double> &, double *, int32_t *, cudaStream_t);
+
 template int launch_plan_tpt<float>(const auvrrt_env *, const float *, const uint64_t *, int64_t, const auvrrt_plan_params_t *,
                                     void *, int64_t, auvrrt_plan_record_t *, uint32_t *, const auvrrt_plan_trace_t *, cudaStream_t, int64_t *);
 template int launch_plan_tpt<double>(const auvrrt_env *, const double *, const uint64_t *, int64_t, const auvrrt_plan_params_t *,

@@ -229,17 +229,26 @@ typedef struct {
 /* starts[Q][5] = (x, y, theta, traj_time_stamp, length); seeds[Q];
  * out_chain[Q][chain_cap]: stream positions of the steer calls root->leaf along the optimal path
  * (enough to re-create it with auvrrt_materialize); out_path[Q][path_cap][6] =
- * (x, y, theta, v, traj_time_stamp, length) in root->leaf order, i.e. result["path"][0]. */
+ * (x, y, theta, v, traj_time_stamp, length) in root->leaf order, i.e. result["path"][0].
+ * out_chain may be NULL.  Status AUVRRT_ST_OVERFLOW is raised only where a chain buffer is passed: a plan
+ * deeper than chain_cap is OVERFLOW with a chain and OK without one.  Records of plans with
+ * depth <= chain_cap are the same either way.  Paths are written while walking the chain, so out_path
+ * needs out_chain. */
 int auvrrt_plan_batch(const auvrrt_env_t *env, const double *starts, const uint64_t *seeds,
                       int64_t Q, const auvrrt_plan_params_t *params, int precision,
                       auvrrt_plan_record_t *out_records, uint32_t *out_chain, double *out_path,
                       const auvrrt_plan_trace_t *trace);
 /* device-resident variant: starts are float[Q][5] (F32) or double[Q][5] (F64); records / chain /
  * path / trace are device pointers (path rows in the precision's floating type; trace.leaf too).
- * workspace from auvrrt_plan_workspace_bytes(); nothing is synchronised. */
+ * workspace from auvrrt_plan_workspace_bytes(); nothing is synchronised.  out_path != NULL with
+ * path_cap > 0 and out_chain == NULL is AUVRRT_ERR_ARG, and so is a workspace smaller than the
+ * launch needs; either way nothing is written.
+ * group 0 picks the kernel per call: one thread per tree for >= 32768 queries without paths
+ * (mode != 3), else one warp per tree. */
 int64_t auvrrt_plan_workspace_bytes(const auvrrt_env_t *env, const auvrrt_plan_params_t *params,
                                     int precision);
-/* same, for a batch of at most Q queries (group == 1 sizes its workspace by the batch) */
+/* same, for a batch of at most Q queries (group == 1 sizes its workspace by the batch; group 0
+ * covers every kernel a batch of at most Q queries can launch) */
 int64_t auvrrt_plan_workspace_bytes_q(const auvrrt_env_t *env, const auvrrt_plan_params_t *params,
                                       int precision, int64_t Q);
 int auvrrt_plan_batch_dev(const auvrrt_env_t *env, const void *starts, const uint64_t *seeds,
@@ -249,7 +258,12 @@ int auvrrt_plan_batch_dev(const auvrrt_env_t *env, const void *starts, const uin
                           const auvrrt_plan_trace_t *trace, void *stream);
 
 /* re-create optimal paths from (start, seed, chain) records, e.g. for the few winners after the
- * multi-GPU gather.  Same row layout as out_path. */
+ * multi-GPU gather.  Same row layout as out_path; out_n_path[q] is the full row count even when it
+ * exceeds path_cap (then only the first path_cap rows are written).  A depth of 0 gives the start
+ * row alone.  Any depth[q] < 0 or > chain_cap (an OVERFLOW record) is AUVRRT_ERR_ARG, checked before
+ * anything runs.  params->group must name the planner that made the chains, because the fp32 edge
+ * evaluators of the group sizes round differently: 32 (or 0), 16, 8, or 1 for the thread-per-tree
+ * planner -- which is also what group 0 ran for a batch of >= 32768 queries without paths. */
 int auvrrt_materialize(const auvrrt_env_t *env, const double *starts, const uint64_t *seeds,
                        const uint32_t *chain, const int32_t *depth, int64_t Q,
                        const auvrrt_plan_params_t *params, int precision, double *out_path,

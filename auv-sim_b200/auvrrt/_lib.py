@@ -77,7 +77,8 @@ EXPORTS = [
     "auvrrt_gym_step_dev", "auvrrt_gym_tree", "auvrrt_gym_counts", "auvrrt_gym_counts_dev", "auvrrt_gym_path",
     "auvrrt_astar_env_create", "auvrrt_astar_env_destroy", "auvrrt_astar_batch", "auvrrt_astar_workspace_bytes",
     "auvrrt_astar_batch_dev", "auvrrt_edges_arc_cost_dev", "auvrrt_edges_arc_cost", "auvrrt_env_host_blob",
-    "auvrrt_edges_dubins_cost_dev", "auvrrt_edges_dubins_cost",
+    "auvrrt_edges_dubins_cost_dev", "auvrrt_edges_dubins_cost", "auvrrt_occ_create", "auvrrt_occ_destroy", "auvrrt_occ_shape",
+    "auvrrt_occ_grid_dev", "auvrrt_env_set_probs", "auvrrt_env_set_probs_dev", "auvrrt_env_get_probs",
 ]
 
 _lib = None
@@ -145,6 +146,15 @@ def lib():
     L.auvrrt_occupancy_dims.argtypes = [_dp, C.c_double, C.c_double, _dp, _i64p, C.c_int, _ip, _ip, _ip]
     L.auvrrt_occupancy_grid.argtypes = [_dp, _i64p, C.c_int, _dp, C.c_double, C.c_double, C.c_double, _dp, _i64p,
                                         C.c_int, C.c_int, _dp, C.c_int64]
+    L.auvrrt_occ_create.argtypes = [_dp, _i64p, C.c_int, _dp, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
+                                    C.c_int64, C.c_int, C.POINTER(vp)]
+    L.auvrrt_occ_destroy.argtypes = [vp]
+    L.auvrrt_occ_destroy.restype = None
+    L.auvrrt_occ_shape.argtypes = [vp, _ip, _ip, _ip]
+    L.auvrrt_occ_grid_dev.argtypes = [vp, vp, vp, C.c_int, C.c_int64, vp, vp, vp, vp]
+    L.auvrrt_env_set_probs.argtypes = [vp, _dp]
+    L.auvrrt_env_set_probs_dev.argtypes = [vp, vp, vp]
+    L.auvrrt_env_get_probs.argtypes = [vp, C.c_int, _dp]
     _u16p = C.POINTER(C.c_uint16)
     L.auvrrt_gym_create.argtypes = [_dp, C.c_int, C.POINTER(GymParams), C.c_int64, C.c_int, C.c_int, C.POINTER(vp)]
     L.auvrrt_gym_destroy.argtypes = [vp]

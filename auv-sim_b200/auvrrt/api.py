@@ -58,12 +58,12 @@ class Env:
         self.bins = _f64(bins, (-1, 2))
         self.cells = _f64(cells, (-1, 4))
         T, Cn = len(self.bins), len(self.cells)
-        self.probs = _f64(probs if probs is not None else np.zeros((T, Cn)), (T, Cn))
+        probs = _f64(probs if probs is not None else np.zeros((T, Cn)), (T, Cn))
         self.device = int(device)
         self._h = C.c_void_p()
         check(lib().auvrrt_env_create(_p(self.circles), len(self.circles), _p(self.boundary),
                                       len(self.boundary), _p(self.habitats), len(self.habitats),
-                                      _p(self.bins), T, _p(self.cells), Cn, _p(self.probs), self.device,
+                                      _p(self.bins), T, _p(self.cells), Cn, _p(probs), self.device,
                                       C.byref(self._h)))
 
     @classmethod
@@ -74,6 +74,30 @@ class Env:
     @property
     def handle(self):
         return self._h
+
+    @property
+    def shape(self):
+        """(T, C) of the shark-occupancy table probs[T][C]"""
+        return len(self.bins), len(self.cells)
+
+    def set_probs(self, probs):
+        """Replace the shark-occupancy table probs[T][C] in place (both precisions' copies; the fp32 copy holds each
+        value rounded to nearest, as at creation).  Bins, cells and everything else stay.  Returns when the table is
+        written; work that reads the world on another stream must be ordered after it by the caller."""
+        T, Cn = self.shape
+        a = np.asarray(probs, dtype=np.float64)
+        if a.shape != (T, Cn):
+            raise ValueError("probs must have shape %s, got %s" % ((T, Cn), a.shape))
+        a = np.ascontiguousarray(a)
+        check(lib().auvrrt_env_set_probs(self._h, _p(a)))
+
+    def probs(self, precision="f64"):
+        """The shark-occupancy table the kernels of `precision` read, as a float64 array [T, C] (the fp32 table
+        widened).  Read on the world's internal stream: a refresh enqueued on another stream must be ordered before
+        this call by the caller."""
+        out = np.zeros(self.shape)
+        check(lib().auvrrt_env_get_probs(self._h, _prec(precision), _p(out)))
+        return out
 
     def close(self):
         if self._h:
@@ -331,14 +355,20 @@ def calibrate_fp32(device=0, iters=4096):
     return f.value, ms.value
 
 
-def occupancy_grid(cell_polys, bounds, cell_size, bin_interval, detect_range, tracks, device=0):
-    """SharkOccupancyGrid.convert: list of cell polygons (vertex arrays, cell_list order), boundary bounds,
-    and one [n,3] (x, y, traj_time_stamp) track per shark -> (grid[T, rows, cols], bins[T, 2])"""
+def flat_polys(cell_polys):
+    """list of polygons (vertex arrays) -> (offsets[C+1] int64, vertices[V, 2] float64), the C ABI's ragged layout"""
     coff = np.zeros(len(cell_polys) + 1, np.int64)
     for i, p in enumerate(cell_polys):
         coff[i + 1] = coff[i] + len(p)
     cxy = _f64(np.concatenate([np.asarray(p, dtype=np.float64).reshape(-1, 2) for p in cell_polys]), (-1, 2)) \
         if len(cell_polys) else np.zeros((0, 2))
+    return coff, cxy
+
+
+def occupancy_grid(cell_polys, bounds, cell_size, bin_interval, detect_range, tracks, device=0):
+    """SharkOccupancyGrid.convert: list of cell polygons (vertex arrays, cell_list order), boundary bounds,
+    and one [n,3] (x, y, traj_time_stamp) track per shark -> (grid[T, rows, cols], bins[T, 2])"""
+    coff, cxy = flat_polys(cell_polys)
     toff = np.zeros(len(tracks) + 1, np.int64)
     for i, t in enumerate(tracks):
         toff[i + 1] = toff[i] + len(t)

@@ -12,7 +12,7 @@ import torch
 
 from . import _lib
 from ._lib import F32, F64, PlanRecord, check, lib
-from .api import RECORD_DTYPE, Env, _prec
+from .api import RECORD_DTYPE, Env, _f64, _p, _prec, flat_polys
 
 
 def _rdtype(precision):
@@ -168,3 +168,74 @@ def gym_counts_tensor(batch):
     if not ptr:
         raise ValueError("gym_counts_tensor: the batch was created without track_counts")
     return torch.as_tensor(_CountsArray(batch, ptr), device=_gym_device(batch))
+
+
+# ---- shark-occupancy grids from device-resident tracks (csrc/occupancy.cu) ----------------------------------------
+
+def _stream_on(dev, stream):
+    return _stream_ptr(stream if stream is not None else torch.cuda.current_stream(dev))
+
+
+class SharkOccupancy:
+    """SharkOccupancyGrid.convert for fixed cells (polygons in cell_list order), boundary bounds, cell size, bin interval
+    and detection range, on tracks that live on the device.  n_bins bins (b * bin_interval, (b + 1) * bin_interval);
+    each call takes at most max_sharks tracks and max_points points.  The handle owns its cell tables, candidate-cell
+    index and workspace: a call allocates nothing and synchronises nothing (it can be captured in a CUDA graph)."""
+
+    def __init__(self, cell_polys, bounds, cell_size, bin_interval, detect_range, n_bins, max_sharks, max_points,
+                 device=0):
+        coff, cxy = flat_polys(cell_polys)
+        b = _f64(bounds, (4,))
+        self.dev = torch.device("cuda", int(device))
+        self.C, self.n_bins = len(cell_polys), int(n_bins)
+        self.max_sharks, self.max_points = int(max_sharks), int(max_points)
+        self._h = C.c_void_p()
+        check(lib().auvrrt_occ_create(_p(cxy), _p(coff, C.c_int64), self.C, _p(b), float(cell_size), float(bin_interval),
+                                      float(detect_range), self.n_bins, self.max_sharks, self.max_points, int(device),
+                                      C.byref(self._h)))
+        T, rows, cols = C.c_int(0), C.c_int(0), C.c_int(0)
+        check(lib().auvrrt_occ_shape(self._h, C.byref(T), C.byref(rows), C.byref(cols)))
+        self.rows, self.cols = rows.value, cols.value
+
+    @property
+    def grid_shape(self):
+        return self.n_bins, self.rows, self.cols
+
+    def grid_dev(self, tracks, track_off, out=None, env=None, t_occ=None, stream=None):
+        """Enqueue one conversion on `stream` (default: the current stream).  tracks float64 [n, 3] (x, y,
+        traj_time_stamp of every point, sharks in dict order), track_off int64 [S + 1]; out float64 [n_bins, rows, cols]
+        or None; env an api.Env whose probs[T][C] is replaced in place (it needs T == n_bins, the same cells and
+        createBinList's bins) or None; t_occ int32 [1] or None, set to createBinList's T for these tracks.  Bins
+        b < min(n_bins, t_occ) equal api.occupancy_grid's bit for bit.  Returns `out`."""
+        n = tracks.shape[0] if isinstance(tracks, torch.Tensor) and tracks.dim() == 2 else -1
+        _need("tracks", tracks, (torch.float64,), (n, 3), self.dev)
+        S = track_off.shape[0] - 1 if isinstance(track_off, torch.Tensor) and track_off.dim() == 1 else -1
+        _need("track_off", track_off, (torch.int64,), (S + 1,), self.dev)
+        if out is not None:
+            _need("out", out, (torch.float64,), self.grid_shape, self.dev)
+        if t_occ is not None:
+            _need("t_occ", t_occ, (torch.int32,), (1,), self.dev)
+        if env is not None and not isinstance(env, Env):
+            raise ValueError("env must be an auvrrt.api.Env, got %s" % type(env).__name__)
+        check(lib().auvrrt_occ_grid_dev(self._h, _vp(tracks), _vp(track_off), S, n, _vp(out),
+                                        env.handle if env is not None else None, _vp(t_occ), _stream_on(self.dev, stream)))
+        return out
+
+    def close(self):
+        if self._h:
+            lib().auvrrt_occ_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def env_set_probs_dev(env: Env, probs, stream=None):
+    """Replace env's shark-occupancy table with probs (float64 [T, C] on env's device), enqueued on `stream` (default:
+    the current stream) without synchronising.  Work that reads env on another stream must be ordered after it."""
+    dev = torch.device("cuda", env.device)
+    _need("probs", probs, (torch.float64,), env.shape, dev)
+    check(lib().auvrrt_env_set_probs_dev(env.handle, _vp(probs), _stream_on(dev, stream)))

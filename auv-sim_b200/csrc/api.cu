@@ -426,6 +426,9 @@ extern "C" int auvrrt_env_create(const double *circles, int K, const double *pol
     auvrrt_env *e = new auvrrt_env();
     memset(e, 0, sizeof(*e));
     e->device = device; e->K = K; e->E = E; e->H = H; e->T = T; e->C = C;
+    e->h_bins = (double *)malloc(16 * (size_t)std::max(T, 1));
+    if (!e->h_bins) { delete e; return set_err(AUVRRT_ERR_CUDA, "env_create: out of host memory"); }
+    if (T) memcpy(e->h_bins, bins, 16 * (size_t)T);
     std::vector<unsigned char> b32 = build_blob<float>(circles, K, poly, E, habitats, H, bins, T, cells, C, probs, &e->h32);
     std::vector<unsigned char> b64 = build_blob<double>(circles, K, poly, E, habitats, H, bins, T, cells, C, probs, &e->h64);
     cudaError_t er = cudaMalloc((void **)&e->blob32, b32.size());
@@ -465,7 +468,44 @@ extern "C" void auvrrt_env_destroy(auvrrt_env_t *e) {
     for (int i = 0; i < 8; i++) if (e->d_scratch[i]) cudaFree(e->d_scratch[i]);
     for (int i = 0; i < 4; i++) if (e->h_pinned[i]) cudaFreeHost(e->h_pinned[i]);
     if (e->stream) cudaStreamDestroy(e->stream);
+    free(e->h_bins);
     delete e;
+}
+
+// ------------------------------------------------------------------ shark-occupancy table of a live world
+extern "C" int auvrrt_env_set_probs_dev(auvrrt_env_t *env, const double *d_probs, void *stream) {
+    if (!env || (!d_probs && (int64_t)env->T * env->C > 0)) return set_err(AUVRRT_ERR_ARG, "env_set_probs_dev: NULL argument");
+    AUV_CUDA(cudaSetDevice(env->device));
+    return launch_probs_to_env(env, d_probs, nullptr, 0, (cudaStream_t)stream);
+}
+extern "C" int auvrrt_env_set_probs(auvrrt_env_t *env, const double *probs) {
+    if (!env || (!probs && (int64_t)env->T * env->C > 0)) return set_err(AUVRRT_ERR_ARG, "env_set_probs: NULL argument");
+    const size_t n = (size_t)env->T * env->C;
+    if (n == 0) return AUVRRT_OK;
+    AUV_CUDA(cudaSetDevice(env->device));
+    void *d = nullptr;
+    AUV_TRY(env_dev_scratch(env, 7, 8 * n, &d));
+    AUV_CUDA(cudaMemcpyAsync(d, probs, 8 * n, cudaMemcpyHostToDevice, env->stream));
+    AUV_TRY(launch_probs_to_env(env, (const double *)d, nullptr, 0, env->stream));
+    AUV_CUDA(cudaStreamSynchronize(env->stream));
+    return AUVRRT_OK;
+}
+extern "C" int auvrrt_env_get_probs(const auvrrt_env_t *env, int precision, double *out) {
+    if (!env || (!out && (int64_t)env->T * env->C > 0)) return set_err(AUVRRT_ERR_ARG, "env_get_probs: NULL argument");
+    AUV_TRY(check_precision(precision));
+    const size_t n = (size_t)env->T * env->C;
+    if (n == 0) return AUVRRT_OK;
+    AUV_CUDA(cudaSetDevice(env->device));
+    if (precision == AUVRRT_F64) {
+        AUV_CUDA(cudaMemcpyAsync(out, env->blob64 + env->h64.off_probs, 8 * n, cudaMemcpyDeviceToHost, env->stream));
+        AUV_CUDA(cudaStreamSynchronize(env->stream));
+        return AUVRRT_OK;
+    }
+    std::vector<float> f(n);
+    AUV_CUDA(cudaMemcpyAsync(f.data(), env->blob32 + env->h32.off_probs, 4 * n, cudaMemcpyDeviceToHost, env->stream));
+    AUV_CUDA(cudaStreamSynchronize(env->stream));
+    for (size_t i = 0; i < n; i++) out[i] = (double)f[i];
+    return AUVRRT_OK;
 }
 
 // ------------------------------------------------------------------ nearest node

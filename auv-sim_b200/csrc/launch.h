@@ -11,6 +11,7 @@ struct auvrrt_env {
     auv::EnvHeader h32, h64;
     unsigned char *blob32, *blob64;   // device
     int K, E, H, T, C;
+    double *h_bins;                   // host copy of bins[T][2] (owned, malloc)
     // host-call scratch (grown on demand, reused across calls)
     void *d_scratch[8];
     size_t d_scratch_bytes[8];
@@ -68,6 +69,10 @@ int64_t nn_scratch_bytes(int nq);
 int launch_calibrate_fp32(int iters, double *flops, double *ms);
 template <typename R> void launch_convert(const double *src, R *dst, int64_t n, cudaStream_t s);
 template <typename R> void launch_convert_back(const R *src, double *dst, int64_t n, cudaStream_t s);
+
+// ---- occupancy.cu: the one writer of both blobs' probs[T][C]: grid[b][cell_sq[c]] of a [T][RC] grid, or src[b][c]
+// when cell_sq is NULL
+int launch_probs_to_env(auvrrt_env *env, const double *src, const int *cell_sq, int RC, cudaStream_t s);
 
 // ---- plan.cu
 template <typename R>

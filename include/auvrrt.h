@@ -285,6 +285,47 @@ int auvrrt_occupancy_grid(const double *cell_xy, const int64_t *cell_off, int C,
                           double detect_range, const double *tracks, const int64_t *track_off,
                           int S, int device, double *out_grid, int64_t out_cap);
 
+/* ---- the same grids from device-resident tracks, and a live world's shark-occupancy table ------
+ * An auvrrt_occ_t is one SharkOccupancyGrid for fixed cells / bounds / cell_size / bin_interval /
+ * detect_range (arguments as for auvrrt_occupancy_grid), with n_bins bins (b * bin_interval,
+ * (b + 1) * bin_interval), at most max_sharks tracks and max_points points per call.  It owns the
+ * cell tables, a candidate-cell index (built once, on the host) and its workspace, so a call
+ * allocates nothing and synchronises nothing.
+ *
+ * auvrrt_occ_grid_dev: d_tracks [n_points][3] (x, y, traj_time_stamp) fp64 and d_track_off [S+1]
+ * int64 on the device, S sharks in dict order (points in no [track_off[s], track_off[s+1]) are
+ * skipped).  Writes d_grid [n_bins][rows][cols] fp64 if non-NULL; if env is non-NULL, replaces its
+ * probs[T][C] (both precisions' tables) in place with probs[b][c] = grid[b][row_c][col_c], where
+ * cell c of the world is polygon c of this handle, in cell_list order, as createSharkGrid lays
+ * them out; if d_t_occ is non-NULL, writes createBinList's T for these tracks there (int32, as
+ * auvrrt_occupancy_dims).  Bins b < min(n_bins, T) are bit-identical to bin b of
+ * auvrrt_occupancy_grid for the same tracks; the caller reads *d_t_occ to know whether all are
+ * covered.  Asynchronous on `stream`: memsets, then 4 kernels (3 when n_points == 0) plus 1 when
+ * env is given.
+ * Writing to env needs env's C == C, T == n_bins and bins exactly (b * bin_interval,
+ * (b + 1) * bin_interval) in double, as createBinList builds them.  A mismatch, S < 1,
+ * S > max_sharks or n_points > max_points is AUVRRT_ERR_ARG, checked before anything is enqueued,
+ * so the world is left unchanged.
+ * Ordering: work that reads the world on another stream -- including every host-buffer entry, which
+ * runs on the world's internal stream -- must be ordered after the refresh by the caller (e.g. by
+ * synchronising `stream`). */
+typedef struct auvrrt_occ auvrrt_occ_t;
+int auvrrt_occ_create(const double *cell_xy, const int64_t *cell_off, int C, const double bounds[4],
+                      double cell_size, double bin_interval, double detect_range, int n_bins,
+                      int max_sharks, int64_t max_points, int device, auvrrt_occ_t **out);
+void auvrrt_occ_destroy(auvrrt_occ_t *o);
+int auvrrt_occ_shape(const auvrrt_occ_t *o, int *T, int *rows, int *cols);
+int auvrrt_occ_grid_dev(auvrrt_occ_t *o, const double *d_tracks, const int64_t *d_track_off, int S,
+                        int64_t n_points, double *d_grid, auvrrt_env_t *env, int32_t *d_t_occ,
+                        void *stream);
+/* Replace a world's probs[T][C] (host table; device table, asynchronous on `stream`) or read it
+ * back (precision AUVRRT_F64: the fp64 table; AUVRRT_F32: the fp32 table, widened).  The fp32
+ * table holds each value rounded to nearest, as auvrrt_env_create stores it.  The same ordering
+ * rule as above applies to auvrrt_env_set_probs_dev. */
+int auvrrt_env_set_probs(auvrrt_env_t *env, const double *probs);
+int auvrrt_env_set_probs_dev(auvrrt_env_t *env, const double *d_probs, void *stream);
+int auvrrt_env_get_probs(const auvrrt_env_t *env, int precision, double *out);
+
 /* ---- gym_rrt Planner_RRT: the goal-directed tree RRTEnv.step grows one node at a time ---------
  * (gym_rrt/envs/rrt_dubins.py:30-503, driven by gym_rrt/envs/rrt_env.py:182-247).  SURVEY.md 8(f) N1.
  * One handle holds Q independent episodes ("vectorised environments") resident in HBM: the tree

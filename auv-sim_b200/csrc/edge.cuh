@@ -75,8 +75,9 @@ __device__ __forceinline__ float sinc_small(float h) {
 // FLAT = true : an explicit recorded stream (e.g. a CPython Mersenne-Twister sequence) consumed back to back,
 //   2 or 3 uniforms per primitive: the per-position step goes to shared memory and log2(G) rounds of pointer
 //   doubling give each lane the offset of its primitive.
-// ONE_CHUNK: the caller guarantees n_expand <= G (freq <= G, checked on the host): the chunk loop runs at most once
-//   and its loop-carried state disappears.
+// ONE_CHUNK: the caller guarantees n_expand <= G - 1 (freq <= G, checked on the host): the chunk runs exactly once (no
+//   loop-carried state), and lane G - 1, which never holds a primitive, tests the parent point (path[0]) with the same
+//   code as the waypoint lanes.
 // GRIDS: plane 0 of the classification grid is staged in shared memory (env.grid0s)
 template <typename R, int G, bool DO_COLLIDE, bool DO_COST, bool WRITE_WP, bool FLAT = false, bool ONE_CHUNK = false, bool GRIDS = false>
 __device__ __forceinline__ void eval_edge(const Grp<G> &g, GroupScratch<R, G, FLAT> &sc, const EnvView<R> &env,
@@ -106,8 +107,11 @@ __device__ __forceinline__ void eval_edge(const Grp<G> &g, GroupScratch<R, G, FL
     if (DO_COLLIDE) {
         // path[0] = the parent node object: tested like any other path point (rrt_dubins.py:537,544)
         // (testing it behind the draws and the steer arithmetic of the first chunk, to run those under the planner's
-        // load of the parent row, was measured slower: 9.16 vs 8.75 ms per step on config 2)
+        // load of the parent row, was measured slower: 9.16 vs 8.75 ms per step on config 2; ONE_CHUNK tests it in
+        // lane G - 1 of the chunk instead)
         if (g.gl == 0) { sc.wx[G] = px; sc.wy[G] = py; }
+    }
+    if (DO_COLLIDE && !ONE_CHUNK) {
         const Cls pcl = env.template classify<GRIDS>(px, py);
         parent_clear = (pcl.code & 4u) != 0u;
         parent_many = (pcl.code & AUV_GRID_CIRC_MANY) != 0u;
@@ -117,8 +121,8 @@ __device__ __forceinline__ void eval_edge(const Grp<G> &g, GroupScratch<R, G, FL
         } else outside = point_unsafe_one<R>(env, pcl.code, px, py);     // (either flag makes the edge unsafe)
     }
 
-    for (int base = 0; base < n_exp; base += G) {
-        const int nact = min(G, n_exp - base);          // active primitives in this chunk
+    for (int base = 0; ONE_CHUNK ? base == 0 : base < n_exp; base += G) {
+        const int nact = ONE_CHUNK ? max(min(G, n_exp), 0) : min(G, n_exp - base);     // active primitives in this chunk
         const bool act = g.gl < nact;
         R dist = 0, diff = 0, vt = 1;
         bool valid = false;
@@ -254,31 +258,35 @@ __device__ __forceinline__ void eval_edge(const Grp<G> &g, GroupScratch<R, G, FL
                 }
             }
         }
+        // ONE_CHUNK: lane G - 1 holds no primitive (n_expand <= G - 1) and tests the parent point
+        const bool pl = ONE_CHUNK && DO_COLLIDE && g.gl == G - 1;
+        const R tx = pl ? px : x, ty = pl ? py : y;          // the point this lane tests
         // one classification-grid load per waypoint replaces most of the exact tests below
         Cls cl; cl.code = AUV_GRID_ALL_AMBIG | 4u; cl.idx = -1;
-        if ((DO_COLLIDE || DO_COST) && (is_wp || g.gl == last_valid)) cl = env.template classify<GRIDS>(x, y);
+        if ((DO_COLLIDE || DO_COST) && (is_wp || g.gl == last_valid || pl)) cl = env.template classify<GRIDS>(tx, ty);
         if (DO_COLLIDE) {
             // lane = waypoint: polygon and the cell's candidate circles
             bool in = true, h1 = false;
-            if (is_wp) {
+            if (is_wp || pl) {
                 if (VERIFY || !AUV_EDGE_ONE) {
-                    in = point_within_c<R>(env, cl, x, y);
-                    if (!(cl.code & AUV_GRID_CIRC_MANY)) h1 = point_hits_circles_c<R>(env, cl, x, y);
+                    in = point_within_c<R>(env, cl, tx, ty);
+                    if (!(cl.code & AUV_GRID_CIRC_MANY)) h1 = point_hits_circles_c<R>(env, cl, tx, ty);
                 } else {
                     // decided cells and single-candidate boundary cells in straight-line code; `in` carries the verdict
-                    in = !point_unsafe_one<R>(env, cl.code, x, y);
+                    in = !point_unsafe_one<R>(env, cl.code, tx, ty);
                     if (__builtin_expect((cl.code & AUV_GRID_SLOW) != 0u, 0)) {
-                        in = point_within_c<R>(env, cl, x, y);
-                        if (!(cl.code & AUV_GRID_CIRC_MANY)) h1 = point_hits_circles_c<R>(env, cl, x, y);
+                        in = point_within_c<R>(env, cl, tx, ty);
+                        if (!(cl.code & AUV_GRID_CIRC_MANY)) h1 = point_hits_circles_c<R>(env, cl, tx, ty);
                     }
                 }
             }
             if (g.ballot(!in)) outside = true;
             if (g.ballot(h1)) hit = true;
             // cells with more than 3 candidate circles (or points outside the grid): lane = circle over
-            // all circles, waypoints broadcast through shared memory
-            const bool circles_needed = g.ballot(is_wp && !(cl.code & 4u) && (cl.code & AUV_GRID_CIRC_MANY)) != 0u ||
-                                        (base == 0 && !parent_clear && parent_many);
+            // all circles, waypoints broadcast through shared memory; the parent joins them in the first chunk (the
+            // chunked form tests a parent in such a cell after the loop when n_expand == 0, and not at all when < 0)
+            const bool circles_needed = g.ballot((is_wp || (pl && n_exp >= 0)) && !(cl.code & 4u) && (cl.code & AUV_GRID_CIRC_MANY)) != 0u ||
+                                        (!ONE_CHUNK && base == 0 && !parent_clear && parent_many);
             // (an edge that already left the polygon is unsafe whatever the circles say)
             if (env.K > 0 && circles_needed && !outside) {
                 if (is_wp) { int slot = __popc(wpm & ((1u << g.gl) - 1u)); sc.wx[slot] = x; sc.wy[slot] = y; }
@@ -348,7 +356,7 @@ __device__ __forceinline__ void eval_edge(const Grp<G> &g, GroupScratch<R, G, FL
         }
         if (ONE_CHUNK) break;
     }
-    if (DO_COLLIDE && n_exp == 0 && env.K > 0 && !parent_clear && parent_many) {
+    if (!ONE_CHUNK && DO_COLLIDE && n_exp == 0 && env.K > 0 && !parent_clear && parent_many) {
         // the path is [parent] alone: test it against the circles
         bool h = false;
 #pragma unroll 1

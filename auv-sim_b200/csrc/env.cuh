@@ -126,24 +126,39 @@ template <typename R> struct EnvView {
     const int *cell;
     const R *probs;
 
-    __device__ __forceinline__ void bind(const unsigned char *hot, const unsigned char *probs_base) {
-        const EnvHeader *h = (const EnvHeader *)hot;
-        K = h->K; E = h->E; H = h->H; T = h->T; C = h->C; NB = h->NB; NP = h->NP; convex = h->convex;
+    // every field but bin_lo / bin_hi (they are read from the bound arrays) from a header and the addresses of the staged
+    // image and of the probability table; usable on the host
+    __host__ __device__ __forceinline__ void bind_header(const EnvHeader &h, const unsigned char *hot, const unsigned char *probs_base) {
+        K = h.K; E = h.E; H = h.H; T = h.T; C = h.C; NB = h.NB; NP = h.NP; convex = h.convex;
         shared_self = nullptr;
-        minx = (R)h->bbox[0]; miny = (R)h->bbox[1]; maxx = (R)h->bbox[2]; maxy = (R)h->bbox[3];
-        cx = (const R *)(hot + h->off_cx); cy = (const R *)(hot + h->off_cy);
-        cr = (const R *)(hot + h->off_cr); creff = (const R *)(hot + h->off_creff);
-        creff2 = (const R *)(hot + h->off_creff2);
-        px = (const R *)(hot + h->off_px); py = (const R *)(hot + h->off_py);
-        hx = (const R *)(hot + h->off_hx); hy = (const R *)(hot + h->off_hy);
-        hr = (const R *)(hot + h->off_hr); hr2 = (const R *)(hot + h->off_hr2);
-        b0 = (const R *)(hot + h->off_b0); b1 = (const R *)(hot + h->off_b1);
-        brk = (const R *)(hot + h->off_brk); piece = (const int *)(hot + h->off_piece);
-        c1 = (const R *)(hot + h->off_c1); cell = (const int *)(hot + h->off_cell);
-        probs = (const R *)(probs_base + h->off_probs);
-        pfirst = (const PFirst<R> *)(hot + h->off_pfirst);
-        cone = (const One<R> *)(hot + h->off_one); pone = cone + (K + 1); hone = pone + (E > 0 ? E : 1);
+        minx = (R)h.bbox[0]; miny = (R)h.bbox[1]; maxx = (R)h.bbox[2]; maxy = (R)h.bbox[3];
+        cx = (const R *)(hot + h.off_cx); cy = (const R *)(hot + h.off_cy);
+        cr = (const R *)(hot + h.off_cr); creff = (const R *)(hot + h.off_creff);
+        creff2 = (const R *)(hot + h.off_creff2);
+        px = (const R *)(hot + h.off_px); py = (const R *)(hot + h.off_py);
+        hx = (const R *)(hot + h.off_hx); hy = (const R *)(hot + h.off_hy);
+        hr = (const R *)(hot + h.off_hr); hr2 = (const R *)(hot + h.off_hr2);
+        b0 = (const R *)(hot + h.off_b0); b1 = (const R *)(hot + h.off_b1);
+        brk = (const R *)(hot + h.off_brk); piece = (const int *)(hot + h.off_piece);
+        c1 = (const R *)(hot + h.off_c1); cell = (const int *)(hot + h.off_cell);
+        probs = (const R *)(probs_base + h.off_probs);
+        pfirst = (const PFirst<R> *)(hot + h.off_pfirst);
+        cone = (const One<R> *)(hot + h.off_one); pone = cone + (K + 1); hone = pone + (E > 0 ? E : 1);
+    }
+    __device__ __forceinline__ void bind(const unsigned char *hot, const unsigned char *probs_base) {
+        bind_header(*(const EnvHeader *)hot, hot, probs_base);
         bin_lo = T > 0 ? b0[0] : (R)1; bin_hi = T > 0 ? b1[T - 1] : (R)0;      // [first b0, last b1]; empty when T == 0
+    }
+    // A view the host bound to the blob in HBM, moved to a copy of the staged image (probability table included) at
+    // `to`.  The kernel receives the view as a parameter: its scalars and array offsets then come from the constant
+    // bank instead of registers loaded from the staged header, and every array is `to` plus a uniform offset.
+    __device__ __forceinline__ void move_staged(const unsigned char *from, const unsigned char *to) {
+#define AUV_MOVE(p) p = (decltype(p))(to + ((const unsigned char *)(p) - from))
+        AUV_MOVE(cx); AUV_MOVE(cy); AUV_MOVE(cr); AUV_MOVE(creff); AUV_MOVE(creff2); AUV_MOVE(px); AUV_MOVE(py);
+        AUV_MOVE(hx); AUV_MOVE(hy); AUV_MOVE(hr); AUV_MOVE(hr2); AUV_MOVE(b0); AUV_MOVE(b1);
+        AUV_MOVE(brk); AUV_MOVE(piece); AUV_MOVE(c1); AUV_MOVE(cell); AUV_MOVE(probs); AUV_MOVE(pfirst);
+        AUV_MOVE(cone); AUV_MOVE(pone); AUV_MOVE(hone); AUV_MOVE(xb);
+#undef AUV_MOVE
     }
     // Tell the compiler that the staged arrays live in shared memory (the pointers are computed from offsets read
     // at run time, so address-space inference cannot see it): loads become LDS with 32-bit addresses instead of
@@ -160,16 +175,18 @@ template <typename R> struct EnvView {
         if (probs_too) __builtin_assume(__isShared(probs));
     }
     // the grid stays in global memory: bind it from the blob in HBM
-    __device__ __forceinline__ void bind_grid(const unsigned char *blob_global, const unsigned char *hot) {
-        const EnvHeader *h = (const EnvHeader *)hot;
-        gnx = h->gnx; gny = h->gny; bins_uniform = h->bins_uniform; nxb = h->nxb;
-        xb0 = (R)h->xb0; xbinv = (R)(1.0 / h->xbw); xbo = (R)(-h->xb0 / h->xbw); xb = (const unsigned short *)(hot + h->off_xb);
-        gx0 = (R)h->gx0; gy0 = (R)h->gy0; ginv = (R)(1.0 / h->gs);
-        gxo = (R)(-h->gx0 / h->gs); gyo = (R)(-h->gy0 / h->gs);
-        bin_s0 = (R)h->bin_s0; bin_w = (R)h->bin_w; bin_winv = (R)(1.0 / h->bin_w); bin_off = (R)(-h->bin_s0 / h->bin_w);
-        grid = (const unsigned *)(blob_global + h->off_grid);
+    __host__ __device__ __forceinline__ void bind_grid_header(const EnvHeader &h, const unsigned char *blob_global, const unsigned char *hot) {
+        gnx = h.gnx; gny = h.gny; bins_uniform = h.bins_uniform; nxb = h.nxb;
+        xb0 = (R)h.xb0; xbinv = (R)(1.0 / h.xbw); xbo = (R)(-h.xb0 / h.xbw); xb = (const unsigned short *)(hot + h.off_xb);
+        gx0 = (R)h.gx0; gy0 = (R)h.gy0; ginv = (R)(1.0 / h.gs);
+        gxo = (R)(-h.gx0 / h.gs); gyo = (R)(-h.gy0 / h.gs);
+        bin_s0 = (R)h.bin_s0; bin_w = (R)h.bin_w; bin_winv = (R)(1.0 / h.bin_w); bin_off = (R)(-h.bin_s0 / h.bin_w);
+        grid = (const unsigned *)(blob_global + h.off_grid);
         grid0s = nullptr;
         ncell = gnx * gny;
+    }
+    __device__ __forceinline__ void bind_grid(const unsigned char *blob_global, const unsigned char *hot) {
+        bind_grid_header(*(const EnvHeader *)hot, blob_global, hot);
     }
     // classification of the cell containing (x, y); off the grid: outside the polygon, everything else ambiguous
     // GRIDS: plane 0 is read from its shared-memory copy (grid0s)

@@ -76,16 +76,20 @@ template <typename R> static WsLayout make_layout(int cap, int nb, int nchunks) 
     return L;
 }
 
+// The group's tree: one slot base; every array is the base plus its WsLayout offset, which are kernel parameters (one
+// 64-bit register for the tree instead of eight pointers)
 template <typename R> struct Tree {
-    NodeRow<R> *row;
-    R *nx, *ny;            // coalesced x[] / y[] for RRT.get_closest_mps (mode 1)
-    int *pool, *next, *head, *tail, *count;
-    __device__ __forceinline__ void bind(unsigned char *b, const WsLayout &L, int cap) {
-        row = (NodeRow<R> *)(b + L.rows);
-        nx = (R *)(b + L.xy); ny = nx + cap;
-        pool = (int *)(b + L.pool); next = (int *)(b + L.next);
-        head = (int *)(b + L.head); tail = (int *)(b + L.tail); count = (int *)(b + L.count);
-    }
+    unsigned char *b;
+    const WsLayout &L;
+    int cap;
+    __device__ __forceinline__ NodeRow<R> *row() const { return (NodeRow<R> *)(b + L.rows); }
+    __device__ __forceinline__ R *nx() const { return (R *)(b + L.xy); }         // coalesced x[] / y[] for RRT.get_closest_mps (mode 1)
+    __device__ __forceinline__ R *ny() const { return nx() + cap; }
+    __device__ __forceinline__ int *pool() const { return (int *)(b + L.pool); }
+    __device__ __forceinline__ int *next() const { return (int *)(b + L.next); }
+    __device__ __forceinline__ int *head() const { return (int *)(b + L.head); }
+    __device__ __forceinline__ int *tail() const { return (int *)(b + L.tail); }
+    __device__ __forceinline__ int *count() const { return (int *)(b + L.count); }
 };
 
 // BS: keep the per-bin metadata (count / head chunk / tail chunk) of the group's tree in shared
@@ -154,26 +158,33 @@ __device__ __forceinline__ void dubins_sample_at(const EnvView<R> &env, const St
 
 #define AUV_BINS_SMEM 128
 template <typename R> struct BestPlan { R c0, c1, c2, len, t; int node, iter; };
+// a group's shared state, reached from one shared address: edge scratch, the best plan so far and, with BS, the bin
+// metadata (count / head chunk / tail chunk)
+template <typename R, int G, bool BS> struct GroupSmem {
+    GroupScratch<R, G, false> sc;
+    BestPlan<R> best;
+    unsigned short bins[3][BS ? AUV_BINS_SMEM : 1];
+};
 // MODE >= 0 compiles the kernel for that parent-pick mode alone (the other modes' code -- about 1000 instructions that
 // the compiler otherwise places inside the hot loop -- disappears); MODE < 0 reads P.mode at run time.
 // ONE: freq <= G, every edge is a single chunk of primitives (eval_edge ONE_CHUNK)
 template <typename R, int G, bool BS, int MODE, bool ONE>
 __global__ void __launch_bounds__(PlanCta<R, G>::T, sizeof(R) == 4 ? PlanCta<R, G>::MINB : (PlanCta<R, G>::MINB + 1) / 2)
-k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode, const R *starts,
-       const uint64_t *seeds, long long Q, PlanP<R> P, WsLayout L, unsigned char *ws, unsigned long long *qcounter,
-       auvrrt_plan_record_t *records, uint32_t *chain_out, R *path_out, auvrrt_plan_trace_t tr) {
+k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode, const __grid_constant__ EnvView<R> envp,
+       const R *starts, const uint64_t *seeds, long long Q, PlanP<R> P, const __grid_constant__ WsLayout L,
+       unsigned char *ws, unsigned long long *qcounter, auvrrt_plan_record_t *records, uint32_t *chain_out, R *path_out,
+       auvrrt_plan_trace_t tr) {
     typedef typename Policy<R>::A A;
     const bool VERIFY = Policy<R>::VERIFY;
     const int pick_mode = MODE >= 0 ? MODE : P.mode;
     extern __shared__ __align__(16) unsigned char smem[];
     const int PLAN_THREADS = PlanCta<R, G>::T;
-    __shared__ GroupScratch<R, G, false> scratch[PlanCta<R, G>::T / G];
-    __shared__ BestPlan<R> best_s[PlanCta<R, G>::T / G];
-    __shared__ unsigned short binmeta[BS ? PlanCta<R, G>::T / G : 1][3][BS ? AUV_BINS_SMEM : 1];
+    __shared__ GroupSmem<R, G, BS> groups[PlanCta<R, G>::T / G];
     EnvView<R> env;
     {
-        if (stage_mode == 0) { env.bind(blob, blob); env.bind_grid(blob, blob); }
-        else if (stage_mode == 3) {
+        // (the single-chunk variant in its one-CTA-per-SM shape always stages this way, plan_geometry: the other modes'
+        // views would make the compiler keep every field in registers)
+        if ((ONE && PlanCta<R, G>::T >= 896) || stage_mode == 3) {
             // one CTA per SM: the world model, the probability table and plane 0 of the classification grid (two regions,
             // one barrier) -- every lookup of the edge evaluation is then an LDS
             uint64_t *bar = (uint64_t *)smem;
@@ -188,10 +199,16 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                 for (int o = 0; o < plane; o += 65536) tma_bulk_g2s(smem + 16 + total_bytes + o, gsrc + o, (uint32_t)(plane - o < 65536 ? plane - o : 65536), bar);
             }
             mbar_wait(bar, 0);
-            env.bind(smem + 16, smem + 16);
-            env.bind_grid(blob, smem + 16);
-            env.grid0s = (const unsigned *)(smem + 16 + total_bytes);
-            __builtin_assume(__isShared(env.grid0s));
+            // (the copy's shared address through volatile asm: the compiler would otherwise rebuild it from SR_CgaCtaId at
+            // every lookup inside the loop)
+            uint32_t staged = smem_u32(smem + 16);
+            asm volatile("" : "+r"(staged));
+            const unsigned char *sp = (const unsigned char *)__cvta_shared_to_generic(staged);
+            env = envp;
+            env.move_staged(blob, sp);
+            env.grid0s = (const unsigned *)(sp + total_bytes);
+        } else if (stage_mode == 0) {
+            env.bind(blob, blob); env.bind_grid(blob, blob);
         } else {
             uint64_t *bar = (uint64_t *)smem;
             stage_env_tma(smem + 16, blob, stage_mode == 2 ? total_bytes : hot_bytes, bar);
@@ -202,18 +219,21 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
         if (ONE) env.assume_hot_shared(PlanCta<R, G>::T >= 896);     // (896-thread shape: stage mode 3, the probability table is staged too)
     }
     Grp<G> g;
-    GroupScratch<R, G, false> &sc = scratch[threadIdx.x / G];
-    const int slot = blockIdx.x * (PLAN_THREADS / G) + threadIdx.x / G;
-    Tree<R> T;
-    T.bind(ws + (size_t)slot * L.slot_bytes, L, P.cap);
-    unsigned short *s_count = binmeta[BS ? threadIdx.x / G : 0][0], *s_head = binmeta[BS ? threadIdx.x / G : 0][1],
-                   *s_tail = binmeta[BS ? threadIdx.x / G : 0][2];
-#define BIN_COUNT(b) (BS ? (int)s_count[b] : T.count[b])
-#define BIN_HEAD(b) (BS ? (int)s_head[b] : T.head[b])
-#define BIN_TAIL(b) (BS ? (int)s_tail[b] : T.tail[b])
-#define SET_BIN_COUNT(b, v) do { if (BS) s_count[b] = (unsigned short)(v); else T.count[b] = (v); } while (0)
-#define SET_BIN_HEAD(b, v) do { if (BS) s_head[b] = (unsigned short)(v); else T.head[b] = (v); } while (0)
-#define SET_BIN_TAIL(b, v) do { if (BS) s_tail[b] = (unsigned short)(v); else T.tail[b] = (v); } while (0)
+    // The group's shared state and its tree slot, each one address computed once.  (Through volatile asm: the compiler
+    // would otherwise rebuild them from SR_TID.X, SR_CTAID.X and SR_CgaCtaId at every use inside the loop.)
+    uint32_t gsa = smem_u32(&groups[threadIdx.x / G]);
+    asm volatile("" : "+r"(gsa));
+    GroupSmem<R, G, BS> &gs = *(GroupSmem<R, G, BS> *)__cvta_shared_to_generic(gsa);
+    GroupScratch<R, G, false> &sc = gs.sc;
+    unsigned char *slot_base = ws + (size_t)(blockIdx.x * (PLAN_THREADS / G) + threadIdx.x / G) * L.slot_bytes;
+    asm volatile("" : "+l"(slot_base));
+    const Tree<R> T{slot_base, L, P.cap};
+#define BIN_COUNT(b) (BS ? (int)gs.bins[0][b] : T.count()[b])
+#define BIN_HEAD(b) (BS ? (int)gs.bins[1][b] : T.head()[b])
+#define BIN_TAIL(b) (BS ? (int)gs.bins[2][b] : T.tail()[b])
+#define SET_BIN_COUNT(b, v) do { if (BS) gs.bins[0][b] = (unsigned short)(v); else T.count()[b] = (v); } while (0)
+#define SET_BIN_HEAD(b, v) do { if (BS) gs.bins[1][b] = (unsigned short)(v); else T.head()[b] = (v); } while (0)
+#define SET_BIN_TAIL(b, v) do { if (BS) gs.bins[2][b] = (unsigned short)(v); else T.tail()[b] = (v); } while (0)
 
     for (;;) {
         long long q = 0;
@@ -221,8 +241,6 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
         q = g.bcast(q, 0);
         if (q >= Q) break;
 
-        Stream<R> rng;
-        rng.key = stream_key(seeds[q]); rng.ext = nullptr; rng.n_ext = 0;
         const R sx = starts[5 * q], sy = starts[5 * q + 1], sth = starts[5 * q + 2], st = starts[5 * q + 3],
                 slen = starts[5 * q + 4];
         // ---- init: mps_list = [initial]; time_bin[bin_interval] = [initial]        rrt_dubins.py:105-114
@@ -234,12 +252,14 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
             Contrib c = point_contrib<R>(env, sx, sy, st, 0xffffffffu, env.H, env.classify(sx, sy));
             r0.self_s2 = (c.bin >= 0 && c.cell >= 0) ? A::mul(P.w3, env.probs[(size_t)c.bin * env.C + c.cell]) : (R)0;
             r0.self_hab = c.bin >= 0 ? c.hab : -1;
-            T.row[0] = r0;
-            if (pick_mode == 1 || pick_mode == 3) { T.nx[0] = sx; T.ny[0] = sy; }
+            T.row()[0] = r0;
+            if (pick_mode == 1 || pick_mode == 3) { T.nx()[0] = sx; T.ny()[0] = sy; }
         }
         g.sync();
-        if (g.gl == 0) { SET_BIN_HEAD(1, 0); SET_BIN_TAIL(1, 0); SET_BIN_COUNT(1, 1); T.pool[0] = 0; T.next[0] = -1; }
+        if (g.gl == 0) { SET_BIN_HEAD(1, 0); SET_BIN_TAIL(1, 0); SET_BIN_COUNT(1, 1); T.pool()[0] = 0; T.next()[0] = -1; }
         g.sync();
+        Stream<R> rng;                 // (after the root's cost: the key is not live across it)
+        rng.key = stream_key(seeds[q]); rng.ext = nullptr; rng.n_ext = 0;
         int n_nodes = 1, n_chunks = 1;
         uint32_t ctr = 0, upos_mark = 0;
         int status = AUVRRT_ST_OK;
@@ -248,7 +268,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
         // the best plan so far: only its total is compared every iteration; the rest lives in shared memory
         // (written by lane 0 on the rare improvement), which frees registers for the edge evaluation
         R best_total = A::inf();
-        if (g.gl == 0) { BestPlan<R> b0; b0.c0 = b0.c1 = b0.c2 = b0.len = b0.t = (R)0; b0.node = -1; b0.iter = -1; best_s[threadIdx.x / G] = b0; }
+        if (g.gl == 0) { BestPlan<R> b0; b0.c0 = b0.c1 = b0.c2 = b0.len = b0.t = (R)0; b0.node = -1; b0.iter = -1; gs.best = b0; }
         int it = 0;
         int guard = 0;
         const int guard_max = (int)min(64LL * P.I + 1024, 2147483647LL);
@@ -271,7 +291,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                     const int i = i0 + g.gl;
                     bool in = false;
                     if (i < n_nodes) {
-                        const R qq = A::sq2(A::sub(smx, T.nx[i]), A::sub(smy, T.ny[i]));
+                        const R qq = A::sq2(A::sub(smx, T.nx()[i]), A::sub(smy, T.ny()[i]));
                         if (qq < bq) {
                             if (VERIFY) { R sd = A::sqrt(qq); if (sd < bs) { bs = sd; bi = i; } }
                             else { bs = qq; bi = i; }
@@ -295,7 +315,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                 }
                 const int nearest = bi;
                 g.sync();
-                if (T.row[nearest].t > P.max_traj) { upos_mark = ctr; continue; }          // :138-139
+                if (T.row()[nearest].t > P.max_traj) { upos_mark = ctr; continue; }          // :138-139
                 // candidates: [nearest] + the list without it, G at most
                 int pn = nlist;                                    // position of the nearest node in the list, if any
                 for (int j = g.gl; j < nlist; j += G) if (near[j] == nearest) pn = j;
@@ -312,7 +332,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                 NodeRow<R> pr;
                 pr.s2 = 0; pr.self_s2 = 0; pr.cnt = 0; pr.mask = 0ull; pr.self_hab = -1; pr.t = 0;
                 if (pidx >= 0) {
-                    pr = T.row[pidx];
+                    pr = T.row()[pidx];
                     if (!(pr.t > P.max_traj))
                         dubins_edge_eval<R>(env, P, pr.x, pr.y, pr.th, pr.t, pr.len, smx, smy, smth, true, nullptr, 0, de);
                 }
@@ -359,8 +379,8 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                         nr.x = de.x; nr.y = de.y; nr.th = de.th; nr.t = de.t; nr.len = de.len; nr.parent = bp; nr.ctr = ctr0;
                         nr.s2 = pre_s2; nr.cnt = pre_cnt; nr.mask = pre_mask; nr.self_s2 = de.self_s2; nr.self_hab = de.self_hab;
                         nr.born = it;
-                        T.row[id] = nr;
-                        T.nx[id] = de.x; T.ny[id] = de.y;
+                        T.row()[id] = nr;
+                        T.nx()[id] = de.x; T.ny()[id] = de.y;
                     }
                     if (nt_ >= P.horizon) {                                                  // :158-171
                         n_cost_evals++;
@@ -368,7 +388,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                             best_total = bt;
                             if (g.gl == bl) {
                                 BestPlan<R> b; b.c0 = c0; b.c1 = c1; b.c2 = c2; b.len = de.len; b.t = de.t; b.node = id; b.iter = it;
-                                best_s[threadIdx.x / G] = b;
+                                gs.best = b;
                             }
                         }
                     }
@@ -404,14 +424,14 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                 if (idx >= bincnt) { status = AUVRRT_ST_KEY_ERROR; break; }
                 int ch = BIN_HEAD(ran_bin);
 #pragma unroll 1
-                for (int hop = idx >> 5; hop > 0; hop--) ch = T.next[ch];
-                parent = T.pool[ch * 32 + (idx & 31)];
+                for (int hop = idx >> 5; hop > 0; hop--) ch = T.next()[ch];
+                parent = T.pool()[ch * 32 + (idx & 31)];
             } else if (pick_mode == 2) {
                 // ---- wall-clock pick on the simulated clock (:129-132): every lane walks the same bisection
                 const R ran_time = uniform_ab<R>((R)0, P.ran_time_max, rng.u(ctr));
                 ctr += 1;
-                parent = closest_mps_time<R>(T.row, n_nodes, ran_time, P.plan_dt);
-                if (T.row[parent].t > P.max_traj) continue;                               // :131-132
+                parent = closest_mps_time<R>(T.row(), n_nodes, ran_time, P.plan_dt);
+                if (T.row()[parent].t > P.max_traj) continue;                               // :131-132
             } else {
                 // ---- get_random_mps (:333-343) + get_closest_mps (:505-513)
                 R rx = uniform_ab<R>(env.minx, env.maxx, rng.u(ctr));
@@ -420,7 +440,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                 R bq = A::inf(), bs = A::inf();
                 int bi = 0x7fffffff;
                 for (int i = g.gl; i < n_nodes; i += G) {
-                    R qq = A::sq2(A::sub(rx, T.nx[i]), A::sub(ry, T.ny[i]));
+                    R qq = A::sq2(A::sub(rx, T.nx()[i]), A::sub(ry, T.ny()[i]));
                     if (qq < bq) {
                         if (VERIFY) { R s = A::sqrt(qq); if (s < bs) { bs = s; bi = i; } }
                         else { bs = qq; bi = i; }
@@ -434,11 +454,13 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                     if (os < bs || (os == bs && oi < bi)) { bs = os; bi = oi; }
                 }
                 parent = bi;
-                if (T.row[parent].t > P.max_traj) continue;                               // :138-139
+                if (T.row()[parent].t > P.max_traj) continue;                               // :138-139
             }
             // ---- steer + check_collision + per-waypoint cost                              :141-143
-            const NodeRow<R> pr = T.row[parent];           // every lane reads the same row: broadcast
-            const R ppx = pr.x, ppy = pr.y, ppth = pr.th, ppt = pr.t, pplen = pr.len;
+            // every lane reads the same row (a broadcast): the state now, the cost prefix after the edge and only if it is
+            // safe (the line is then in L1), so that the prefix is not live across the edge evaluation
+            const NodeRow<R> *prow = T.row() + parent;
+            const R ppx = prow->x, ppy = prow->y, ppth = prow->th, ppt = prow->t, pplen = prow->len;
             const uint32_t ctr0 = ctr;
 #if AUV_PLAN_PREFETCH
             // Look ahead.  Slot addressing makes the next iteration's stream position known now (this edge owns
@@ -451,13 +473,13 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                 const int n_exp_now = (int)A::floor(uniform_ab<R>((R)0, P.sp.freq, rng.u(ctr)));
                 const uint32_t cn0 = ctr + 1u + 3u * (uint32_t)(n_exp_now > 0 ? n_exp_now : 0);
                 const int rb = (int)uniform_ab<R>((R)1, (R)(P.nb + 1), rng.u(cn0 + (uint32_t)g.gl));
-                const int cn = (rb >= 1 && rb <= P.nb) ? (int)s_count[rb] : 0;
+                const int cn = (rb >= 1 && rb <= P.nb) ? (int)gs.bins[0][rb] : 0;
                 const unsigned m = g.ballot(cn > 0);
                 if (m) {
                     const int f = __ffs(m) - 1;
                     const int sb = g.bcast(rb, f), sc_ = g.bcast(cn, f);
                     const int idx = (int)uniform_ab<R>((R)0, (R)sc_, rng.u(cn0 + (uint32_t)f + 1u));
-                    if (idx < 32 && idx < sc_) spec_parent = T.pool[(int)s_head[sb] * 32 + idx];
+                    if (idx < 32 && idx < sc_) spec_parent = T.pool()[(int)gs.bins[1][sb] * 32 + idx];
                 }
             }
 #endif
@@ -466,7 +488,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                                                            nullptr, 0, o);
 #if AUV_PLAN_PREFETCH
             if (ONE && BS && pick_mode == 0 && spec_parent >= 0 && g.gl < 2)
-                asm volatile("prefetch.global.L1 [%0];" ::"l"((const char *)&T.row[spec_parent] + 32 * g.gl));
+                asm volatile("prefetch.global.L1 [%0];" ::"l"((const char *)&T.row()[spec_parent] + 32 * g.gl));
 #endif
             ctr = o.ctr;
             n_waypoints += o.nwp; n_prims += o.n_exp;
@@ -479,21 +501,23 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
             if (o.status != 0) { status = o.status; break; }
             if (o.safe) {
                 const int id = n_nodes++;                                                  // :144-145
-                R pre_s2 = 0, self_s2n = 0;
-                uint32_t pre_cnt = 0; unsigned long long pre_mask = 0; int self_habn = -1;
+                // (every lane computes the new node's cost prefix: the leaf cost below needs no broadcast)
+                const R pr_s2 = prow->s2, pr_self_s2 = prow->self_s2;
+                const uint32_t pr_cnt = prow->cnt;
+                const int ph = prow->self_hab;
+                const unsigned long long pr_mask = prow->mask;
+                const R pre_s2 = A::add(A::add(pr_s2, pr_self_s2), o.s2);
+                const uint32_t pre_cnt = pr_cnt + (ph >= 0 ? 1u : 0u) + o.cnt;
+                const unsigned long long pre_mask = pr_mask | (ph >= 0 ? (1ull << ph) : 0ull) | o.mask;
+                const R self_s2n = o.leaf_moved ? o.self_s2 : pr_self_s2;
+                const int self_habn = o.leaf_moved ? o.self_hab : ph;
                 if (g.gl == 0) {
-                    const int ph = pr.self_hab;
-                    pre_s2 = A::add(A::add(pr.s2, pr.self_s2), o.s2);
-                    pre_cnt = pr.cnt + (ph >= 0 ? 1u : 0u) + o.cnt;
-                    pre_mask = pr.mask | (ph >= 0 ? (1ull << ph) : 0ull) | o.mask;
-                    self_s2n = o.leaf_moved ? o.self_s2 : pr.self_s2;
-                    self_habn = o.leaf_moved ? o.self_hab : ph;
                     NodeRow<R> nr;
                     nr.x = o.x; nr.y = o.y; nr.th = o.th; nr.t = o.t; nr.len = o.len; nr.parent = parent; nr.ctr = ctr0;
                     nr.s2 = pre_s2; nr.cnt = pre_cnt; nr.mask = pre_mask; nr.self_s2 = self_s2n; nr.self_hab = self_habn;
                     nr.born = it;
-                    T.row[id] = nr;
-                    if (pick_mode == 1 || pick_mode == 3) { T.nx[id] = o.x; T.ny[id] = o.y; }
+                    T.row()[id] = nr;
+                    if (pick_mode == 1 || pick_mode == 3) { T.nx()[id] = o.x; T.ny()[id] = o.y; }
                 }
                 // ---- time-bin insert (decision is group-uniform, lane 0 writes)            :147-151
                 if (pick_mode != 2) {                   // `if traj_time_stamp:` -- mode 2 keeps no bins
@@ -519,38 +543,31 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                         if (g.gl == 0) {
                             int tl = reuse_head ? BIN_HEAD(bidx) : BIN_TAIL(bidx);
                             if (alloc) {
-                                T.next[nc] = -1;
-                                if (c == 0) SET_BIN_HEAD(bidx, nc); else T.next[tl] = nc;
+                                T.next()[nc] = -1;
+                                if (c == 0) SET_BIN_HEAD(bidx, nc); else T.next()[tl] = nc;
                                 tl = nc;
                             }
                             SET_BIN_TAIL(bidx, tl);
-                            T.pool[tl * 32 + (c & 31)] = id;
+                            T.pool()[tl * 32 + (c & 31)] = id;
                             SET_BIN_COUNT(bidx, c + 1);
                         }
                     }
                 }
-                status = g.bcast(status, 0);
-                if (status != AUVRRT_ST_OK) break;
+                if (status != AUVRRT_ST_OK) break;              // (status is group-uniform)
                 // ---- candidate leaf: cost of the path root -> new node                    :158-171
                 if (o.t >= P.horizon) {
-                    R tot_s2 = 0, c0 = 0, c1 = 0, c2 = 0, total = 0;
-                    if (g.gl == 0) {
-                        uint32_t cnt = pre_cnt + (self_habn >= 0 ? 1u : 0u);
-                        unsigned long long mk = pre_mask | (self_habn >= 0 ? (1ull << self_habn) : 0ull);
-                        tot_s2 = A::add(pre_s2, self_s2n);
-                        c1 = A::mul(P.w2, (R)cnt);
-                        c2 = tot_s2;
-                        if (o.t > (R)0) { c1 = A::div(c1, o.t); c2 = A::div(c2, o.t); }        // cost.py:194-196
-                        if (env.H != 0) c0 = A::div(A::mul(P.w1, (R)__popcll(mk)), (R)env.H);  // cost.py:204-205
-                        total = py_sum3p<R>(c0, c1, c2);
-                    }
-                    total = g.bcast(total, 0);
+                    const uint32_t cnt = pre_cnt + (self_habn >= 0 ? 1u : 0u);
+                    const unsigned long long mk = pre_mask | (self_habn >= 0 ? (1ull << self_habn) : 0ull);
+                    R c0 = 0, c1 = A::mul(P.w2, (R)cnt), c2 = A::add(pre_s2, self_s2n);
+                    if (o.t > (R)0) { c1 = A::div(c1, o.t); c2 = A::div(c2, o.t); }            // cost.py:194-196
+                    if (env.H != 0) c0 = A::div(A::mul(P.w1, (R)__popcll(mk)), (R)env.H);      // cost.py:204-205
+                    const R total = py_sum3p<R>(c0, c1, c2);
                     n_cost_evals++;
                     if (total < best_total) {                                              // :169 strict <
                         best_total = total;
                         if (g.gl == 0) {
                             BestPlan<R> b; b.c0 = c0; b.c1 = c1; b.c2 = c2; b.len = o.len; b.t = o.t; b.node = id; b.iter = it;
-                            best_s[threadIdx.x / G] = b;
+                            gs.best = b;
                         }
                     }
                 }
@@ -560,7 +577,8 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
             upos_mark = ctr;
         }
         g.sync();
-        const BestPlan<R> best = best_s[threadIdx.x / G];
+        rng.key = stream_key(seeds[q]);   // (derived again for the path: the part the loop does not use is not kept across it)
+        const BestPlan<R> best = gs.best;
         const int best_node = best.node, best_iter = best.iter;
         const R best_c[4] = {best_total, best.c0, best.c1, best.c2}, best_len = best.len, best_t = best.t;
         if (status == AUVRRT_ST_OK && best_node < 0) status = AUVRRT_ST_NO_PATH;
@@ -569,19 +587,19 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
         if (best_node < 0 && chain_out)
             for (int k = g.gl; k < P.chain_cap; k += G) chain_out[(size_t)q * P.chain_cap + k] = 0u;
         if (best_node >= 0) {
-            for (int n = best_node; T.row[n].parent >= 0; n = T.row[n].parent) depth++;
+            for (int n = best_node; T.row()[n].parent >= 0; n = T.row()[n].parent) depth++;
             uint32_t *chain = chain_out ? chain_out + (size_t)q * P.chain_cap : nullptr;
             if (depth > P.chain_cap && chain) { if (status == AUVRRT_ST_OK) status = AUVRRT_ST_OVERFLOW; }
             if (chain && g.gl == 0) {
                 int n = best_node;
-                for (int k = depth - 1; k >= 0; k--) { if (k < P.chain_cap) chain[k] = (uint32_t)n; n = T.row[n].parent; }
+                for (int k = depth - 1; k >= 0; k--) { if (k < P.chain_cap) chain[k] = (uint32_t)n; n = T.row()[n].parent; }
             }
             g.sync();
             if (path_out && P.path_cap > 0 && chain && depth <= P.chain_cap) {
                 R *rows = path_out + (size_t)q * P.path_cap * 6;
                 for (int e = 0; e < depth; e++) {
                     const int id = (int)chain[e];
-                    const NodeRow<R> pn = T.row[T.row[id].parent];
+                    const NodeRow<R> pn = T.row()[T.row()[id].parent];
                     if (g.gl == 0 && n_path < P.path_cap) {
                         R *w = rows + 6 * (size_t)n_path;
                         w[0] = pn.x; w[1] = pn.y; w[2] = pn.th; w[3] = (pick_mode == 3 && pn.parent >= 0) ? P.vel : (R)0;
@@ -592,7 +610,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                     if (pick_mode == 3) {
                         if (g.gl == 0) {
                             R smx, smy, smth;
-                            dubins_sample_at<R>(env, rng, T.row[id].ctr, smx, smy, smth);
+                            dubins_sample_at<R>(env, rng, T.row()[id].ctr, smx, smy, smth);
                             DubinsEdge<R> de;
                             dubins_edge_eval<R>(env, P, pn.x, pn.y, pn.th, pn.t, pn.len, smx, smy, smth, false,
                                                 rows + 6 * (size_t)(n_path < P.path_cap ? n_path : 0), room, de);
@@ -601,14 +619,14 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                         continue;
                     }
                     EdgeOut<R> o;
-                    eval_edge<R, G, false, false, true>(g, sc, env, rng, T.row[id].ctr, P.sp, pn.x, pn.y, pn.th,
+                    eval_edge<R, G, false, false, true>(g, sc, env, rng, T.row()[id].ctr, P.sp, pn.x, pn.y, pn.th,
                                                         pn.t, pn.len, (R)0, 0,
                                                         rows + 6 * (size_t)(n_path < P.path_cap ? n_path : 0), room, o);
                     n_path += o.nwp - 1;
                 }
                 if (g.gl == 0 && n_path < P.path_cap) {
                     R *w = rows + 6 * (size_t)n_path;
-                    const NodeRow<R> bn = T.row[best_node];
+                    const NodeRow<R> bn = T.row()[best_node];
                     w[0] = bn.x; w[1] = bn.y; w[2] = bn.th; w[3] = (pick_mode == 3 && bn.parent >= 0) ? P.vel : (R)0;
                     w[4] = bn.t; w[5] = bn.len;
                 }
@@ -617,7 +635,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
             }
             g.sync();
             if (chain && g.gl == 0)
-                for (int k = 0; k < depth && k < P.chain_cap; k++) chain[k] = T.row[chain[k]].ctr;
+                for (int k = 0; k < depth && k < P.chain_cap; k++) chain[k] = T.row()[chain[k]].ctr;
             if (chain) for (int k = depth + g.gl; k < P.chain_cap; k += G) chain[k] = 0u;
         }
         if (g.gl == 0) {
@@ -740,7 +758,13 @@ static int launch_plan_gb(const auvrrt_env *env, const R *starts, const uint64_t
     auvrrt_plan_trace_t tr;
     if (trace) tr = *trace; else { tr.parent = nullptr; tr.safe = nullptr; tr.nwp = nullptr; tr.leaf = nullptr; tr.upos = nullptr; }
     EnvBlob<R> b = env_blob<R>(env);
-    k_plan<R, G, BS, MODE, ONE><<<grid, PlanCta<R, G>::T, smem, s>>>(b.blob, b.hot_bytes, b.total_bytes, mode, starts, seeds, (long long)Q, P, L,
+    // the world-model view bound to the blob in HBM (stage mode 3 moves its arrays to the shared-memory copy)
+    const EnvHeader &hd = sizeof(R) == 4 ? env->h32 : env->h64;
+    EnvView<R> ev;
+    ev.bind_header(hd, b.blob, b.blob);
+    ev.bind_grid_header(hd, b.blob, b.blob);
+    ev.bin_lo = hd.T > 0 ? (R)env->h_bins[0] : (R)1; ev.bin_hi = hd.T > 0 ? (R)env->h_bins[2 * hd.T - 1] : (R)0;
+    k_plan<R, G, BS, MODE, ONE><<<grid, PlanCta<R, G>::T, smem, s>>>(b.blob, b.hot_bytes, b.total_bytes, mode, ev, starts, seeds, (long long)Q, P, L,
                                                   (unsigned char *)workspace + 256, (unsigned long long *)workspace,
                                                   records, chain, path, tr);
     AUV_LAUNCH_CHECK2();
@@ -763,7 +787,12 @@ static int launch_plan_g(const auvrrt_env *env, const R *starts, const uint64_t 
             const bool fits = PlanCta<R, G>::T >= 896
                                   ? (env->h32.gnx > 0 && env->h32.total_bytes + 16 + env->h32.gnx * env->h32.gny * 4 + 16 <= 180 * 1024)
                                   : env->h32.hot_bytes + 16 <= 24 * 1024;
-            if (p->freq <= (double)G && bs && fits && !getenv("AUVRRT_PLAN_STAGE_KB"))
+            // n_expand = floor(uniform_ab<float>(0, freq, d)) = floor(fmaf(freq, d, -freq)) with d in [1, 2 - 2^-23]: at
+            // most G - 1 for freq <= G, which leaves lane G - 1 of the single chunk to the parent point (eval_edge).
+            // The form is monotone in d, so the largest draw bounds it.
+            const float fq = (float)p->freq;
+            const bool one_chunk = p->freq <= (double)G && floorf(fmaf(fq, 2.0f - 0x1p-23f, -fq)) <= (float)(G - 1);
+            if (one_chunk && bs && fits && !getenv("AUVRRT_PLAN_STAGE_KB"))
                 return launch_plan_gb<R, G, true, 0, true>(AUV_PLAN_ARGS);
             return bs ? launch_plan_gb<R, G, true, 0, false>(AUV_PLAN_ARGS) : launch_plan_gb<R, G, false, 0, false>(AUV_PLAN_ARGS);
         }

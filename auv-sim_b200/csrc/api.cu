@@ -1,6 +1,7 @@
 // api.cu -- the C ABI (include/auvrrt.h): world-model flattening and host-buffer entry points.
 // No CPU fallback anywhere: every compute entry runs the CUDA kernels or fails with AUVRRT_ERR_CUDA.
 #include <algorithm>
+#include <deque>
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -19,6 +20,14 @@ extern "C" int64_t auvrrt_launch_count(void) { return g_launches; }
 extern "C" double auvrrt_stream_u(uint64_t seed, int64_t k, int f32) {
     uint64_t z = stream_bits(stream_key(seed), (uint32_t)k);
     return f32 ? (double)(z >> 41) * 0x1.0p-23 : (double)(z >> 11) * 0x1.0p-53;
+}
+
+int auv::need_device(int device) {
+    int n = auvrrt_device_count();
+    if (n <= 0) return set_err(AUVRRT_ERR_CUDA, "no CUDA device: libauvrrt has no CPU fallback");
+    if (device < 0 || device >= n) return set_err(AUVRRT_ERR_ARG, "device %d out of range (%d devices)", device, n);
+    AUV_CUDA(cudaSetDevice(device));
+    return AUVRRT_OK;
 }
 
 // ------------------------------------------------------------------ env blob builder (host)
@@ -329,85 +338,101 @@ std::vector<unsigned char> build_blob(const double *circles, int K, const double
     return blob;
 }
 
-// RAII device buffer
-struct DBuf {
-    void *p = nullptr;
-    size_t bytes = 0;
-    int alloc(size_t n) {
-        bytes = n ? n : 16;
-        cudaError_t e = cudaMalloc(&p, bytes);
-        if (e != cudaSuccess) { p = nullptr; return set_err(AUVRRT_ERR_CUDA, "cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e)); }
-        return AUVRRT_OK;
-    }
-    template <typename T> T *as() { return (T *)p; }
-    ~DBuf() { if (p) cudaFree(p); }
-};
-#define AUV_TRY(x) do { int rc_ = (x); if (rc_) return rc_; } while (0)
-
-// upload host doubles as R
-template <typename R> int upload_real(DBuf &dst, const double *src, int64_t n, cudaStream_t s, DBuf &tmp) {
-    AUV_TRY(dst.alloc(sizeof(R) * (size_t)std::max<int64_t>(n, 1)));
-    if (n <= 0) return AUVRRT_OK;
-    if (sizeof(R) == 8) { AUV_CUDA(cudaMemcpyAsync(dst.p, src, 8 * (size_t)n, cudaMemcpyHostToDevice, s)); return AUVRRT_OK; }
-    AUV_TRY(tmp.alloc(8 * (size_t)n));
-    AUV_CUDA(cudaMemcpyAsync(tmp.p, src, 8 * (size_t)n, cudaMemcpyHostToDevice, s));
-    launch_convert<R>(tmp.as<double>(), dst.as<R>(), n, s);
-    return AUVRRT_OK;
-}
-template <typename R> int download_real(double *dst, DBuf &src, int64_t n, cudaStream_t s, DBuf &tmp) {
-    if (n <= 0 || !dst) return AUVRRT_OK;
-    if (sizeof(R) == 8) { AUV_CUDA(cudaMemcpyAsync(dst, src.p, 8 * (size_t)n, cudaMemcpyDeviceToHost, s)); return AUVRRT_OK; }
-    AUV_TRY(tmp.alloc(8 * (size_t)n));
-    launch_convert_back<R>(src.as<R>(), tmp.as<double>(), n, s);
-    AUV_CUDA(cudaMemcpyAsync(dst, tmp.p, 8 * (size_t)n, cudaMemcpyDeviceToHost, s));
-    return AUVRRT_OK;
-}
-template <typename T> int upload_raw(DBuf &dst, const T *src, int64_t n, cudaStream_t s) {
-    AUV_TRY(dst.alloc(sizeof(T) * (size_t)std::max<int64_t>(n, 1)));
-    if (n > 0) AUV_CUDA(cudaMemcpyAsync(dst.p, src, sizeof(T) * (size_t)n, cudaMemcpyHostToDevice, s));
-    return AUVRRT_OK;
-}
-template <typename T> int download_raw(T *dst, DBuf &src, int64_t n, cudaStream_t s) {
-    if (n > 0 && dst) AUV_CUDA(cudaMemcpyAsync(dst, src.p, sizeof(T) * (size_t)n, cudaMemcpyDeviceToHost, s));
-    return AUVRRT_OK;
-}
-
-int need_device(int device) {
-    int n = auvrrt_device_count();
-    if (n <= 0) return set_err(AUVRRT_ERR_CUDA, "no CUDA device: libauvrrt has no CPU fallback");
-    if (device < 0 || device >= n) return set_err(AUVRRT_ERR_ARG, "device %d out of range (%d devices)", device, n);
-    AUV_CUDA(cudaSetDevice(device));
-    return AUVRRT_OK;
-}
 int check_precision(int precision) {
     if (precision != AUVRRT_F32 && precision != AUVRRT_F64) return set_err(AUVRRT_ERR_ARG, "precision must be AUVRRT_F32 or AUVRRT_F64");
     return AUVRRT_OK;
 }
 
-// env-owned reusable buffers for the host plan path
-int env_dev_scratch(auvrrt_env *e, int slot, size_t bytes, void **out) {
-    if (e->d_scratch_bytes[slot] < bytes) {
-        if (e->d_scratch[slot]) cudaFree(e->d_scratch[slot]);
-        e->d_scratch[slot] = nullptr; e->d_scratch_bytes[slot] = 0;
-        size_t want = bytes + bytes / 4 + 256;
-        cudaError_t er = cudaMalloc(&e->d_scratch[slot], want);
-        if (er != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "cudaMalloc(%zu): %s", want, cudaGetErrorString(er));
-        e->d_scratch_bytes[slot] = want;
+// One host-buffer call on the legacy default stream.  in() copies a host array to the device when it is declared;
+// out() allocates a device output that finish(), after the launch, copies back where the host pointer is non-null.
+// Real arrays (in_real, out_real) are double on the host and R on the device: for R = float they pass through an fp64
+// buffer and k_convert / k_convert_back.  Zero-length arrays get 16 bytes.  Every buffer lives as long as the object.
+// The first error sticks in rc: later steps do nothing and hand out NULL, so a caller checks rc once, before its launch.
+class Staging {
+  public:
+    int rc = AUVRRT_OK;
+
+    template <typename T> const T *in(const T *h, int64_t n) {
+        T *d = (T *)alloc(sizeof(T), n, false);
+        if (d && n > 0) copy(d, h, sizeof(T) * (size_t)n, cudaMemcpyHostToDevice);
+        return d;
     }
-    *out = e->d_scratch[slot];
+    template <typename R> const R *in_real(const double *h, int64_t n) {
+        if (sizeof(R) == 8) return (const R *)in(h, n);
+        R *d = (R *)alloc(sizeof(R), n, false);
+        if (d && n > 0) {
+            const double *t = in(h, n);
+            if (t) keep(launch_convert<R>(t, d, n, 0));
+        }
+        return d;
+    }
+    template <typename T> T *out(T *h, int64_t n, bool zero = false) {
+        T *d = (T *)alloc(sizeof(T), n, zero);
+        if (d && h && n > 0) outs.push_back(Out{h, d, n, false, sizeof(T) * (size_t)n});
+        return d;
+    }
+    template <typename R> R *out_real(double *h, int64_t n, bool zero = false) {
+        if (sizeof(R) == 8) return (R *)out(h, n, zero);
+        R *d = (R *)alloc(sizeof(R), n, zero);
+        if (d && h && n > 0) outs.push_back(Out{h, d, n, true, 8 * (size_t)n});
+        return d;
+    }
+    // every conversion and copy back, then one synchronisation
+    int finish() {
+        for (const Out &o : outs) {
+            const void *src = o.dev;
+            if (o.widen) {
+                double *t = (double *)alloc(8, o.n, false);
+                if (t) keep(launch_convert_back<float>((const float *)o.dev, t, o.n, 0));
+                src = t;
+            }
+            copy(o.host, src, o.bytes, cudaMemcpyDeviceToHost);
+        }
+        if (!rc) keep_cuda(cudaStreamSynchronize(0), "cudaStreamSynchronize");
+        return rc;
+    }
+
+  private:
+    struct Out { void *host; const void *dev; int64_t n; bool widen; size_t bytes; };   // bytes: on the host
+    std::deque<DBuf> bufs;
+    std::vector<Out> outs;
+
+    void *alloc(size_t size, int64_t n, bool zero) {
+        if (rc) return nullptr;
+        bufs.emplace_back();
+        DBuf &b = bufs.back();
+        if ((rc = b.alloc(n > 0 ? size * (size_t)n : 0))) return nullptr;
+        if (zero) keep_cuda(cudaMemsetAsync(b.p, 0, b.bytes, 0), "cudaMemsetAsync");
+        return rc ? nullptr : b.p;
+    }
+    void copy(void *dst, const void *src, size_t bytes, cudaMemcpyKind kind) {
+        if (!rc) keep_cuda(cudaMemcpyAsync(dst, src, bytes, kind, 0), "cudaMemcpyAsync");
+    }
+    void keep(int r) { if (!rc) rc = r; }
+    void keep_cuda(cudaError_t e, const char *what) {
+        if (e != cudaSuccess) keep(set_err(AUVRRT_ERR_CUDA, "%s: %s", what, cudaGetErrorString(e)));
+    }
+};
+
+// env-owned buffers of the host plan path, grown on demand and reused across calls: device scratch or pinned host staging
+int env_grow(void *&p, size_t &have, size_t bytes, bool pinned, void **out) {
+    if (have < bytes) {
+        if (p) { if (pinned) cudaFreeHost(p); else cudaFree(p); }
+        p = nullptr; have = 0;
+        const size_t want = bytes + bytes / 4 + 256;
+        cudaError_t er = pinned ? cudaMallocHost(&p, want) : cudaMalloc(&p, want);
+        if (er != cudaSuccess)
+            return set_err(AUVRRT_ERR_CUDA, "%s(%zu): %s", pinned ? "cudaMallocHost" : "cudaMalloc", want, cudaGetErrorString(er));
+        have = want;
+    }
+    *out = p;
     return AUVRRT_OK;
 }
+int env_dev_scratch(auvrrt_env *e, int slot, size_t bytes, void **out) {
+    return env_grow(e->d_scratch[slot], e->d_scratch_bytes[slot], bytes, false, out);
+}
 int env_pinned(auvrrt_env *e, int slot, size_t bytes, void **out) {
-    if (e->h_pinned_bytes[slot] < bytes) {
-        if (e->h_pinned[slot]) cudaFreeHost(e->h_pinned[slot]);
-        e->h_pinned[slot] = nullptr; e->h_pinned_bytes[slot] = 0;
-        size_t want = bytes + bytes / 4 + 256;
-        cudaError_t er = cudaMallocHost(&e->h_pinned[slot], want);
-        if (er != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "cudaMallocHost(%zu): %s", want, cudaGetErrorString(er));
-        e->h_pinned_bytes[slot] = want;
-    }
-    *out = e->h_pinned[slot];
-    return AUVRRT_OK;
+    return env_grow(e->h_pinned[slot], e->h_pinned_bytes[slot], bytes, true, out);
 }
 
 }  // namespace
@@ -454,9 +479,7 @@ extern "C" int64_t auvrrt_env_host_blob(const double *circles, int K, const doub
         return -1;
     }
     EnvHeader h;
-    std::vector<unsigned char> b = precision == AUVRRT_F32
-        ? build_blob<float>(circles, K, poly, E, habitats, H, bins, T, cells, C, probs, &h)
-        : build_blob<double>(circles, K, poly, E, habitats, H, bins, T, cells, C, probs, &h);
+    std::vector<unsigned char> b = AUV_DISPATCH(precision, build_blob, circles, K, poly, E, habitats, H, bins, T, cells, C, probs, &h);
     if (out && cap >= (int64_t)b.size()) memcpy(out, b.data(), b.size());
     return (int64_t)b.size();
 }
@@ -520,15 +543,14 @@ extern "C" int auvrrt_nn_dev(const void *tx, const void *ty, int64_t n, const vo
 }
 template <typename R>
 static int nn_host(const double *tx, const double *ty, int64_t n, const double *qx, const double *qy, int nq, int32_t *out) {
-    cudaStream_t s = 0;
-    DBuf dtx, dty, dqx, dqy, t0, t1, t2, t3, scr, di;
-    AUV_TRY(upload_real<R>(dtx, tx, n, s, t0)); AUV_TRY(upload_real<R>(dty, ty, n, s, t1));
-    AUV_TRY(upload_real<R>(dqx, qx, nq, s, t2)); AUV_TRY(upload_real<R>(dqy, qy, nq, s, t3));
-    AUV_TRY(scr.alloc((size_t)nn_scratch_bytes(nq))); AUV_TRY(di.alloc(4 * (size_t)std::max(nq, 1)));
-    AUV_TRY(launch_nn<R>(dtx.as<R>(), dty.as<R>(), n, dqx.as<R>(), dqy.as<R>(), nq, scr.p, (int64_t)scr.bytes, di.as<int32_t>(), s));
-    AUV_TRY(download_raw<int32_t>(out, di, nq, s));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *dtx = st.in_real<R>(tx, n), *dty = st.in_real<R>(ty, n), *dqx = st.in_real<R>(qx, nq), *dqy = st.in_real<R>(qy, nq);
+    const int64_t scratch_bytes = nn_scratch_bytes(nq);
+    unsigned char *scratch = st.out<unsigned char>(nullptr, scratch_bytes);
+    int32_t *didx = st.out(out, nq);
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_nn<R>(dtx, dty, n, dqx, dqy, nq, scratch, scratch_bytes, didx, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_nn(const double *tx, const double *ty, int64_t n, const double *qx, const double *qy, int nq,
                          int precision, int device, int32_t *out_idx) {
@@ -536,31 +558,25 @@ extern "C" int auvrrt_nn(const double *tx, const double *ty, int64_t n, const do
     AUV_TRY(need_device(device));
     if (nq <= 0) return AUVRRT_OK;
     if (n <= 0) return set_err(AUVRRT_ERR_ARG, "nn: empty tree");
-    return precision == AUVRRT_F32 ? nn_host<float>(tx, ty, n, qx, qy, nq, out_idx) : nn_host<double>(tx, ty, n, qx, qy, nq, out_idx);
+    return AUV_DISPATCH(precision, nn_host, tx, ty, n, qx, qy, nq, out_idx);
 }
 
 // ------------------------------------------------------------------ steer (arc)
 template <typename R>
 static int steer_arc_host(const double *parents, int64_t n, const double *u, const int64_t *uoff, const double params[5],
                           double *leaf, int32_t *counts, double *wp, int wp_cap, int32_t *used, int32_t *status) {
-    cudaStream_t s = 0;
-    DBuf dp, tp, du, doff, dleaf, dcnt, dwp, dused, dst, t1, t2;
-    AUV_TRY(upload_real<R>(dp, parents, 5 * n, s, tp));
-    AUV_TRY(upload_raw<double>(du, u, uoff[n], s));
-    AUV_TRY(upload_raw<int64_t>(doff, uoff, n + 1, s));
-    AUV_TRY(dleaf.alloc(sizeof(R) * 5 * (size_t)n)); AUV_TRY(dcnt.alloc(4 * (size_t)n));
-    AUV_TRY(dwp.alloc(sizeof(R) * 6 * (size_t)n * std::max(wp_cap, 1)));
-    AUV_TRY(dused.alloc(4 * (size_t)n)); AUV_TRY(dst.alloc(4 * (size_t)n));
-    AUV_CUDA(cudaMemsetAsync(dwp.p, 0, dwp.bytes, s));
-    AUV_TRY(launch_steer_arc<R>(dp.as<R>(), n, du.as<double>(), doff.as<int64_t>(), params, dleaf.as<R>(), dcnt.as<int32_t>(),
-                                dwp.as<R>(), wp_cap, dused.as<int32_t>(), dst.as<int32_t>(), s));
-    AUV_TRY(download_real<R>(leaf, dleaf, 5 * n, s, t1));
-    AUV_TRY(download_real<R>(wp, dwp, 6 * n * wp_cap, s, t2));
-    AUV_TRY(download_raw<int32_t>(counts, dcnt, n, s));
-    AUV_TRY(download_raw<int32_t>(used, dused, n, s));
-    AUV_TRY(download_raw<int32_t>(status, dst, n, s));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *dp = st.in_real<R>(parents, 5 * n);
+    const double *du = st.in(u, uoff[n]);
+    const int64_t *doff = st.in(uoff, n + 1);
+    R *dleaf = st.out_real<R>(leaf, 5 * n);
+    int32_t *dcnt = st.out(counts, n);
+    // wp_cap 0: one zeroed row per edge on the device, nothing to copy back
+    R *dwp = st.out_real<R>(wp_cap > 0 ? wp : nullptr, 6 * n * std::max(wp_cap, 1), true);
+    int32_t *dused = st.out(used, n), *dst = st.out(status, n);
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_steer_arc<R>(dp, n, du, doff, params, dleaf, dcnt, dwp, wp_cap, dused, dst, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_steer_arc(const double *parents, int64_t n, const double *u, const int64_t *uoff,
                                 const double params[5], int precision, int device, double *leaf, int32_t *counts,
@@ -569,28 +585,21 @@ extern "C" int auvrrt_steer_arc(const double *parents, int64_t n, const double *
     AUV_TRY(need_device(device));
     if (n <= 0) return AUVRRT_OK;
     if (!parents || !u || !uoff || !params) return set_err(AUVRRT_ERR_ARG, "steer_arc: NULL input");
-    return precision == AUVRRT_F32
-               ? steer_arc_host<float>(parents, n, u, uoff, params, leaf, counts, waypoints, wp_cap, used, status)
-               : steer_arc_host<double>(parents, n, u, uoff, params, leaf, counts, waypoints, wp_cap, used, status);
+    return AUV_DISPATCH(precision, steer_arc_host, parents, n, u, uoff, params, leaf, counts, waypoints, wp_cap, used, status);
 }
 
 // ------------------------------------------------------------------ steer (Dubins)
 template <typename R>
 static int steer_dubins_host(const double *from, const double *to, int64_t n, double rho, int W, uint8_t *word,
                              double *seg, double *length, double *wp) {
-    cudaStream_t s = 0;
-    DBuf df, dt, t0, t1, dword, dseg, dlen, dwp, t2, t3, t4;
-    AUV_TRY(upload_real<R>(df, from, 3 * n, s, t0)); AUV_TRY(upload_real<R>(dt, to, 3 * n, s, t1));
-    AUV_TRY(dword.alloc((size_t)n)); AUV_TRY(dseg.alloc(sizeof(R) * 3 * (size_t)n)); AUV_TRY(dlen.alloc(sizeof(R) * (size_t)n));
-    if (wp) { AUV_TRY(dwp.alloc(sizeof(R) * 3 * (size_t)n * W)); AUV_CUDA(cudaMemsetAsync(dwp.p, 0, dwp.bytes, s)); }
-    AUV_TRY(launch_steer_dubins<R>(df.as<R>(), dt.as<R>(), n, rho, W, dword.as<uint8_t>(), dseg.as<R>(), dlen.as<R>(),
-                                   wp ? dwp.as<R>() : nullptr, s));
-    AUV_TRY(download_raw<uint8_t>(word, dword, n, s));
-    AUV_TRY(download_real<R>(seg, dseg, 3 * n, s, t2));
-    AUV_TRY(download_real<R>(length, dlen, n, s, t3));
-    if (wp) AUV_TRY(download_real<R>(wp, dwp, 3 * n * W, s, t4));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *df = st.in_real<R>(from, 3 * n), *dt = st.in_real<R>(to, 3 * n);
+    uint8_t *dword = st.out(word, n);
+    R *dseg = st.out_real<R>(seg, 3 * n), *dlen = st.out_real<R>(length, n);
+    R *dwp = wp ? st.out_real<R>(wp, 3 * n * W, true) : nullptr;
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_steer_dubins<R>(df, dt, n, rho, W, dword, dseg, dlen, dwp, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_steer_dubins(const double *from, const double *to, int64_t n, double rho, int W, int precision,
                                    int device, uint8_t *word, double *seg, double *length, double *waypoints) {
@@ -599,22 +608,19 @@ extern "C" int auvrrt_steer_dubins(const double *from, const double *to, int64_t
     if (n <= 0) return AUVRRT_OK;
     if (!(rho > 0)) return set_err(AUVRRT_ERR_ARG, "steer_dubins: rho must be > 0");
     if (waypoints && W < 2) return set_err(AUVRRT_ERR_ARG, "steer_dubins: W must be >= 2");
-    return precision == AUVRRT_F32 ? steer_dubins_host<float>(from, to, n, rho, W, word, seg, length, waypoints)
-                                   : steer_dubins_host<double>(from, to, n, rho, W, word, seg, length, waypoints);
+    return AUV_DISPATCH(precision, steer_dubins_host, from, to, n, rho, W, word, seg, length, waypoints);
 }
 
 // ------------------------------------------------------------------ collide
 template <typename R>
 static int collide_host(const auvrrt_env *env, const double *points, const int64_t *off, int64_t n, uint8_t *out) {
-    cudaStream_t s = 0;
-    DBuf dp, t0, doff, dout;
-    AUV_TRY(upload_real<R>(dp, points, 2 * off[n], s, t0));
-    AUV_TRY(upload_raw<int64_t>(doff, off, n + 1, s));
-    AUV_TRY(dout.alloc((size_t)n));
-    AUV_TRY(launch_collide<R>(env, dp.as<R>(), doff.as<int64_t>(), n, dout.as<uint8_t>(), s));
-    AUV_TRY(download_raw<uint8_t>(out, dout, n, s));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *dp = st.in_real<R>(points, 2 * off[n]);
+    const int64_t *doff = st.in(off, n + 1);
+    uint8_t *dout = st.out(out, n);
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_collide<R>(env, dp, doff, n, dout, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_collide(const auvrrt_env_t *env, const double *points, const int64_t *off, int64_t n,
                               int precision, uint8_t *out_safe) {
@@ -622,41 +628,37 @@ extern "C" int auvrrt_collide(const auvrrt_env_t *env, const double *points, con
     if (!env) return set_err(AUVRRT_ERR_ARG, "collide: env is NULL");
     AUV_TRY(need_device(env->device));
     if (n <= 0) return AUVRRT_OK;
-    return precision == AUVRRT_F32 ? collide_host<float>(env, points, off, n, out_safe) : collide_host<double>(env, points, off, n, out_safe);
+    return AUV_DISPATCH(precision, collide_host, env, points, off, n, out_safe);
 }
 template <typename R>
 static int collide_points_host(const auvrrt_env *env, const double *points, int64_t n, uint8_t *out) {
-    cudaStream_t s = 0;
-    DBuf dp, t0, dout;
-    AUV_TRY(upload_real<R>(dp, points, 2 * n, s, t0));
-    AUV_TRY(dout.alloc((size_t)n));
-    AUV_TRY(launch_collide_points<R>(env, dp.as<R>(), n, dout.as<uint8_t>(), s));
-    AUV_TRY(download_raw<uint8_t>(out, dout, n, s));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *dp = st.in_real<R>(points, 2 * n);
+    uint8_t *dout = st.out(out, n);
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_collide_points<R>(env, dp, n, dout, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_collide_points(const auvrrt_env_t *env, const double *points, int64_t n, int precision, uint8_t *out_safe) {
     AUV_TRY(check_precision(precision));
     if (!env) return set_err(AUVRRT_ERR_ARG, "collide_points: env is NULL");
     AUV_TRY(need_device(env->device));
     if (n <= 0) return AUVRRT_OK;
-    return precision == AUVRRT_F32 ? collide_points_host<float>(env, points, n, out_safe) : collide_points_host<double>(env, points, n, out_safe);
+    return AUV_DISPATCH(precision, collide_points_host, env, points, n, out_safe);
 }
 
 // ------------------------------------------------------------------ cost
 template <typename R>
 static int cost_host(const auvrrt_env *env, const double *points, const int64_t *off, int64_t n, const double *t_total,
                      const double weights[3], unsigned mask, int n_hab, double *out) {
-    cudaStream_t s = 0;
-    DBuf dp, t0, doff, dt, t1, dout, t2;
-    AUV_TRY(upload_real<R>(dp, points, 3 * off[n], s, t0));
-    AUV_TRY(upload_raw<int64_t>(doff, off, n + 1, s));
-    AUV_TRY(upload_real<R>(dt, t_total, n, s, t1));
-    AUV_TRY(dout.alloc(sizeof(R) * 4 * (size_t)n));
-    AUV_TRY(launch_cost<R>(env, dp.as<R>(), doff.as<int64_t>(), n, dt.as<R>(), weights, mask, n_hab, dout.as<R>(), s));
-    AUV_TRY(download_real<R>(out, dout, 4 * n, s, t2));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *dp = st.in_real<R>(points, 3 * off[n]);
+    const int64_t *doff = st.in(off, n + 1);
+    const R *dt = st.in_real<R>(t_total, n);
+    R *dout = st.out_real<R>(out, 4 * n);
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_cost<R>(env, dp, doff, n, dt, weights, mask, n_hab, dout, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_cost(const auvrrt_env_t *env, const double *points, const int64_t *off, int64_t n,
                            const double *t_total, const double weights[3], const uint8_t *bin_mask, int n_habitats,
@@ -672,20 +674,17 @@ extern "C" int auvrrt_cost(const auvrrt_env_t *env, const double *points, const 
         for (int b = 0; b < env->T; b++) if (bin_mask[b]) mask |= 1u << b;
     }
     int nh = n_habitats < 0 ? env->H : std::min(n_habitats, env->H);
-    return precision == AUVRRT_F32 ? cost_host<float>(env, points, off, n, t_total, weights, mask, nh, out)
-                                   : cost_host<double>(env, points, off, n, t_total, weights, mask, nh, out);
+    return AUV_DISPATCH(precision, cost_host, env, points, off, n, t_total, weights, mask, nh, out);
 }
 template <typename R>
 static int cost_point_host(const auvrrt_env *env, const double *points, int64_t n, unsigned long long visited, int tb,
                            const double weights[3], double *out) {
-    cudaStream_t s = 0;
-    DBuf dp, t0, dout, t1;
-    AUV_TRY(upload_real<R>(dp, points, 2 * n, s, t0));
-    AUV_TRY(dout.alloc(sizeof(R) * (size_t)n));
-    AUV_TRY(launch_cost_point<R>(env, dp.as<R>(), n, visited, tb, weights, dout.as<R>(), s));
-    AUV_TRY(download_real<R>(out, dout, n, s, t1));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *dp = st.in_real<R>(points, 2 * n);
+    R *dout = st.out_real<R>(out, n);
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_cost_point<R>(env, dp, n, visited, tb, weights, dout, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_cost_point(const auvrrt_env_t *env, const double *points, int64_t n, const uint8_t *visited,
                                  int tb, const double weights[3], int precision, double *out_sum) {
@@ -695,8 +694,7 @@ extern "C" int auvrrt_cost_point(const auvrrt_env_t *env, const double *points, 
     if (n <= 0) return AUVRRT_OK;
     unsigned long long vm = 0;
     if (visited) for (int h = 0; h < env->H; h++) if (visited[h]) vm |= 1ull << h;
-    return precision == AUVRRT_F32 ? cost_point_host<float>(env, points, n, vm, tb, weights, out_sum)
-                                   : cost_point_host<double>(env, points, n, vm, tb, weights, out_sum);
+    return AUV_DISPATCH(precision, cost_point_host, env, points, n, vm, tb, weights, out_sum);
 }
 
 // ------------------------------------------------------------------ fused edges
@@ -723,18 +721,14 @@ extern "C" int auvrrt_edges_arc_dev(const auvrrt_env_t *env, const void *parents
 template <typename R>
 static int edges_dubins_host(const auvrrt_env *env, const double *from, const double *to, int64_t n, double rho, int W,
                              uint8_t *safe, uint8_t *word, double *length, double vel = 1.0, double w3 = 0.0, double *cost = nullptr) {
-    cudaStream_t s = 0;
-    DBuf df, dt, t0, t1, dsafe, dword, dlen, t2, dcost, t3;
-    AUV_TRY(upload_real<R>(df, from, 3 * n, s, t0)); AUV_TRY(upload_real<R>(dt, to, 3 * n, s, t1));
-    AUV_TRY(dsafe.alloc((size_t)n)); AUV_TRY(dword.alloc((size_t)n)); AUV_TRY(dlen.alloc(sizeof(R) * (size_t)n));
-    if (cost) AUV_TRY(dcost.alloc(sizeof(R) * 3 * (size_t)n));
-    AUV_TRY(launch_edges_dubins<R>(env, df.as<R>(), dt.as<R>(), n, rho, W, dsafe.as<uint8_t>(), dword.as<uint8_t>(), dlen.as<R>(), s,
-                                   vel, w3, cost ? dcost.as<R>() : nullptr));
-    AUV_TRY(download_raw<uint8_t>(safe, dsafe, n, s)); AUV_TRY(download_raw<uint8_t>(word, dword, n, s));
-    AUV_TRY(download_real<R>(length, dlen, n, s, t2));
-    if (cost) AUV_TRY(download_real<R>(cost, dcost, 3 * n, s, t3));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *df = st.in_real<R>(from, 3 * n), *dt = st.in_real<R>(to, 3 * n);
+    uint8_t *dsafe = st.out(safe, n), *dword = st.out(word, n);
+    R *dlen = st.out_real<R>(length, n);
+    R *dcost = cost ? st.out_real<R>(cost, 3 * n) : nullptr;
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_edges_dubins<R>(env, df, dt, n, rho, W, dsafe, dword, dlen, 0, vel, w3, dcost));
+    return st.finish();
 }
 extern "C" int auvrrt_edges_dubins(const auvrrt_env_t *env, const double *from, const double *to, int64_t n, double rho,
                                    int W, int precision, uint8_t *out_safe, uint8_t *out_word, double *out_length) {
@@ -742,8 +736,7 @@ extern "C" int auvrrt_edges_dubins(const auvrrt_env_t *env, const double *from, 
     if (!env) return set_err(AUVRRT_ERR_ARG, "edges_dubins: env is NULL");
     AUV_TRY(need_device(env->device));
     if (n <= 0) return AUVRRT_OK;
-    return precision == AUVRRT_F32 ? edges_dubins_host<float>(env, from, to, n, rho, W, out_safe, out_word, out_length)
-                                   : edges_dubins_host<double>(env, from, to, n, rho, W, out_safe, out_word, out_length);
+    return AUV_DISPATCH(precision, edges_dubins_host, env, from, to, n, rho, W, out_safe, out_word, out_length);
 }
 extern "C" int auvrrt_edges_dubins_cost_dev(const auvrrt_env_t *env, const void *from, const void *to, int64_t n, double rho,
                                             int W, double velocity, double w3, int precision, uint8_t *out_safe,
@@ -766,22 +759,22 @@ extern "C" int auvrrt_edges_dubins_cost(const auvrrt_env_t *env, const double *f
     if (!out_cost) return set_err(AUVRRT_ERR_ARG, "edges_dubins_cost: out_cost is NULL");
     AUV_TRY(need_device(env->device));
     if (n <= 0) return AUVRRT_OK;
-    return precision == AUVRRT_F32 ? edges_dubins_host<float>(env, from, to, n, rho, W, out_safe, out_word, out_length, velocity, w3, out_cost)
-                                   : edges_dubins_host<double>(env, from, to, n, rho, W, out_safe, out_word, out_length, velocity, w3, out_cost);
+    return AUV_DISPATCH(precision, edges_dubins_host, env, from, to, n, rho, W, out_safe, out_word, out_length, velocity, w3, out_cost);
 }
 template <typename R>
 static int edges_arc_host(const auvrrt_env *env, const double *parents, const uint64_t *seeds, int64_t n,
-                          const double params[5], uint8_t *safe, int32_t *counts, double *leaf) {
-    cudaStream_t s = 0;
-    DBuf dp, t0, dseed, dsafe, dcnt, dleaf, t1;
-    AUV_TRY(upload_real<R>(dp, parents, 5 * n, s, t0));
-    AUV_TRY(upload_raw<uint64_t>(dseed, seeds, n, s));
-    AUV_TRY(dsafe.alloc((size_t)n)); AUV_TRY(dcnt.alloc(4 * (size_t)n)); AUV_TRY(dleaf.alloc(sizeof(R) * 5 * (size_t)n));
-    AUV_TRY(launch_edges_arc<R>(env, dp.as<R>(), dseed.as<uint64_t>(), n, params, dsafe.as<uint8_t>(), dcnt.as<int32_t>(), dleaf.as<R>(), s));
-    AUV_TRY(download_raw<uint8_t>(safe, dsafe, n, s)); AUV_TRY(download_raw<int32_t>(counts, dcnt, n, s));
-    AUV_TRY(download_real<R>(leaf, dleaf, 5 * n, s, t1));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+                          const double params[5], uint8_t *safe, int32_t *counts, double *leaf, double w3 = 0.0,
+                          double *cost = nullptr) {
+    Staging st;
+    const R *dp = st.in_real<R>(parents, 5 * n);
+    const uint64_t *dseed = st.in(seeds, n);
+    uint8_t *dsafe = st.out(safe, n);
+    int32_t *dcnt = st.out(counts, n);
+    R *dleaf = st.out_real<R>(leaf, 5 * n);
+    R *dcost = cost ? st.out_real<R>(cost, 3 * n) : nullptr;
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_edges_arc<R>(env, dp, dseed, n, params, dsafe, dcnt, dleaf, 0, w3, dcost));
+    return st.finish();
 }
 extern "C" int auvrrt_edges_arc(const auvrrt_env_t *env, const double *parents, const uint64_t *seeds, int64_t n,
                                 const double params[5], int precision, uint8_t *out_safe, int32_t *out_counts,
@@ -790,8 +783,7 @@ extern "C" int auvrrt_edges_arc(const auvrrt_env_t *env, const double *parents, 
     if (!env) return set_err(AUVRRT_ERR_ARG, "edges_arc: env is NULL");
     AUV_TRY(need_device(env->device));
     if (n <= 0) return AUVRRT_OK;
-    return precision == AUVRRT_F32 ? edges_arc_host<float>(env, parents, seeds, n, params, out_safe, out_counts, out_leaf)
-                                   : edges_arc_host<double>(env, parents, seeds, n, params, out_safe, out_counts, out_leaf);
+    return AUV_DISPATCH(precision, edges_arc_host, env, parents, seeds, n, params, out_safe, out_counts, out_leaf);
 }
 
 extern "C" int auvrrt_edges_arc_cost_dev(const auvrrt_env_t *env, const void *parents, const uint64_t *seeds, int64_t n,
@@ -806,23 +798,6 @@ extern "C" int auvrrt_edges_arc_cost_dev(const auvrrt_env_t *env, const void *pa
     return launch_edges_arc<double>(env, (const double *)parents, seeds, n, params, out_safe, out_counts, (double *)out_leaf, s, w3,
                                     (double *)out_cost);
 }
-template <typename R>
-static int edges_arc_cost_host(const auvrrt_env *env, const double *parents, const uint64_t *seeds, int64_t n,
-                               const double params[5], double w3, uint8_t *safe, int32_t *counts, double *leaf, double *cost) {
-    cudaStream_t s = 0;
-    DBuf dp, t0, dseed, dsafe, dcnt, dleaf, dcost, t1, t2;
-    AUV_TRY(upload_real<R>(dp, parents, 5 * n, s, t0));
-    AUV_TRY(upload_raw<uint64_t>(dseed, seeds, n, s));
-    AUV_TRY(dsafe.alloc((size_t)n)); AUV_TRY(dcnt.alloc(4 * (size_t)n)); AUV_TRY(dleaf.alloc(sizeof(R) * 5 * (size_t)n));
-    AUV_TRY(dcost.alloc(sizeof(R) * 3 * (size_t)n));
-    AUV_TRY(launch_edges_arc<R>(env, dp.as<R>(), dseed.as<uint64_t>(), n, params, dsafe.as<uint8_t>(), dcnt.as<int32_t>(), dleaf.as<R>(), s,
-                                w3, dcost.as<R>()));
-    AUV_TRY(download_raw<uint8_t>(safe, dsafe, n, s)); AUV_TRY(download_raw<int32_t>(counts, dcnt, n, s));
-    AUV_TRY(download_real<R>(leaf, dleaf, 5 * n, s, t1));
-    AUV_TRY(download_real<R>(cost, dcost, 3 * n, s, t2));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
-}
 extern "C" int auvrrt_edges_arc_cost(const auvrrt_env_t *env, const double *parents, const uint64_t *seeds, int64_t n,
                                      const double params[5], double w3, int precision, uint8_t *out_safe,
                                      int32_t *out_counts, double *out_leaf, double *out_cost) {
@@ -830,20 +805,19 @@ extern "C" int auvrrt_edges_arc_cost(const auvrrt_env_t *env, const double *pare
     if (!env || !out_cost || !out_safe || !out_counts || !out_leaf) return set_err(AUVRRT_ERR_ARG, "edges_arc_cost: NULL argument");
     AUV_TRY(need_device(env->device));
     if (n <= 0) return AUVRRT_OK;
-    return precision == AUVRRT_F32 ? edges_arc_cost_host<float>(env, parents, seeds, n, params, w3, out_safe, out_counts, out_leaf, out_cost)
-                                   : edges_arc_cost_host<double>(env, parents, seeds, n, params, w3, out_safe, out_counts, out_leaf, out_cost);
+    return AUV_DISPATCH(precision, edges_arc_host, env, parents, seeds, n, params, out_safe, out_counts, out_leaf, w3, out_cost);
 }
 
 // ------------------------------------------------------------------ planner
 extern "C" int64_t auvrrt_plan_workspace_bytes(const auvrrt_env_t *env, const auvrrt_plan_params_t *params, int precision) {
     if (!env || !params || check_precision(precision)) return -1;
     if (need_device(env->device)) return -1;
-    return precision == AUVRRT_F32 ? plan_workspace_bytes<float>(env, params, 0) : plan_workspace_bytes<double>(env, params, 0);
+    return AUV_DISPATCH(precision, plan_workspace_bytes, env, params, 0);
 }
 extern "C" int64_t auvrrt_plan_workspace_bytes_q(const auvrrt_env_t *env, const auvrrt_plan_params_t *params, int precision, int64_t Q) {
     if (!env || !params || check_precision(precision)) return -1;
     if (need_device(env->device)) return -1;
-    return precision == AUVRRT_F32 ? plan_workspace_bytes<float>(env, params, Q) : plan_workspace_bytes<double>(env, params, Q);
+    return AUV_DISPATCH(precision, plan_workspace_bytes, env, params, Q);
 }
 extern "C" int auvrrt_plan_batch_dev(const auvrrt_env_t *env, const void *starts, const uint64_t *seeds, int64_t Q,
                                      const auvrrt_plan_params_t *params, int precision, void *workspace,
@@ -950,29 +924,23 @@ extern "C" int auvrrt_plan_batch(const auvrrt_env_t *env, const double *starts, 
     if (Q <= 0) return AUVRRT_OK;
     if (!starts || !seeds) return set_err(AUVRRT_ERR_ARG, "plan_batch: NULL starts or seeds");
     auvrrt_env *e = const_cast<auvrrt_env *>(env);
-    return precision == AUVRRT_F32 ? plan_host<float>(e, starts, seeds, Q, params, out_records, out_chain, out_path, trace)
-                                   : plan_host<double>(e, starts, seeds, Q, params, out_records, out_chain, out_path, trace);
+    return AUV_DISPATCH(precision, plan_host, e, starts, seeds, Q, params, out_records, out_chain, out_path, trace);
 }
 
 template <typename R>
 static int materialize_host(const auvrrt_env *env, const double *starts, const uint64_t *seeds, const uint32_t *chain,
                             const int32_t *depth, int64_t Q, const auvrrt_plan_params_t *p, double *path, int32_t *n_path) {
-    cudaStream_t s = 0;
     const int ccap = p->chain_cap > 0 ? p->chain_cap : 1;
-    DBuf ds, t0, dseed, dchain, ddepth, dpath, dn, t1;
-    AUV_TRY(upload_real<R>(ds, starts, 5 * Q, s, t0));
-    AUV_TRY(upload_raw<uint64_t>(dseed, seeds, Q, s));
-    AUV_TRY(upload_raw<uint32_t>(dchain, chain, Q * ccap, s));
-    AUV_TRY(upload_raw<int32_t>(ddepth, depth, Q, s));
-    AUV_TRY(dpath.alloc(sizeof(R) * 6 * (size_t)Q * p->path_cap));
-    AUV_CUDA(cudaMemsetAsync(dpath.p, 0, dpath.bytes, s));
-    AUV_TRY(dn.alloc(4 * (size_t)Q));
-    AUV_TRY(launch_materialize<R>(env, ds.as<R>(), dseed.as<uint64_t>(), dchain.as<uint32_t>(), ddepth.as<int32_t>(), Q, p,
-                                  dpath.as<R>(), dn.as<int32_t>(), s));
-    AUV_TRY(download_real<R>(path, dpath, 6 * Q * p->path_cap, s, t1));
-    AUV_TRY(download_raw<int32_t>(n_path, dn, Q, s));
-    AUV_CUDA(cudaStreamSynchronize(s));
-    return AUVRRT_OK;
+    Staging st;
+    const R *ds = st.in_real<R>(starts, 5 * Q);
+    const uint64_t *dseed = st.in(seeds, Q);
+    const uint32_t *dchain = st.in(chain, Q * ccap);
+    const int32_t *ddepth = st.in(depth, Q);
+    R *dpath = st.out_real<R>(path, 6 * Q * p->path_cap, true);
+    int32_t *dn = st.out(n_path, Q);
+    AUV_TRY(st.rc);
+    AUV_TRY(launch_materialize<R>(env, ds, dseed, dchain, ddepth, Q, p, dpath, dn, 0));
+    return st.finish();
 }
 extern "C" int auvrrt_materialize(const auvrrt_env_t *env, const double *starts, const uint64_t *seeds,
                                   const uint32_t *chain, const int32_t *depth, int64_t Q,
@@ -991,8 +959,7 @@ extern "C" int auvrrt_materialize(const auvrrt_env_t *env, const double *starts,
         if (depth[q] < 0 || depth[q] > params->chain_cap)
             return set_err(AUVRRT_ERR_ARG, "materialize: depth[%lld] = %d outside [0, chain_cap = %d]", (long long)q, depth[q],
                            params->chain_cap);
-    return precision == AUVRRT_F32 ? materialize_host<float>(env, starts, seeds, chain, depth, Q, params, out_path, out_n_path)
-                                   : materialize_host<double>(env, starts, seeds, chain, depth, Q, params, out_path, out_n_path);
+    return AUV_DISPATCH(precision, materialize_host, env, starts, seeds, chain, depth, Q, params, out_path, out_n_path);
 }
 
 extern "C" int auvrrt_calibrate_fp32(int device, int iters, double *out_flops, double *out_ms) {

@@ -312,9 +312,7 @@ extern "C" int auvrrt_astar_env_create(const double *circles, int K, const doubl
     if (!out || K < 0 || E < 3 || H < 0 || T < 0 || C < 0 || !boundary || !centroid || (K && !circles) || (H && !habitats) ||
         (T && !bins) || (C && !cells_rounded) || (T && C && !probs))
         return set_err(AUVRRT_ERR_ARG, "astar_env_create: bad arguments (the boundary needs at least 3 corners)");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return set_err(AUVRRT_ERR_CUDA, "astar_env_create: no CUDA device (no CPU fallback)"); }
-    AUV_CUDA(cudaSetDevice(device));
+    AUV_TRY(need_device(device));
     auvrrt_astar_env *e = new (std::nothrow) auvrrt_astar_env();
     if (!e) return set_err(AUVRRT_ERR_ARG, "astar_env_create: out of memory");
     e->device = device; e->K = K; e->E = E; e->H = H; e->T = T; e->C = C; e->cx = centroid[0]; e->cy = centroid[1];
@@ -413,8 +411,7 @@ extern "C" int auvrrt_astar_batch_dev(auvrrt_astar_env_t *env, const auvrrt_asta
     k_astar<<<(unsigned)((Q + ASTAR_WARPS - 1) / ASTAR_WARPS), 32 * ASTAR_WARPS, 0, (cudaStream_t)stream>>>(
         astar_dev(env), d_queries, (long long)Q, node_cap, path_cap, (unsigned char *)d_workspace, d_records, d_paths, d_keep,
         d_expand_order, d_node_xy);
-    g_launches++;
-    AUV_CUDA(cudaGetLastError());
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 
@@ -429,13 +426,14 @@ extern "C" int auvrrt_astar_batch(auvrrt_astar_env_t *env, const auvrrt_astar_qu
         AUV_CUDA(cudaMalloc(&env->d_ws, need));
         env->ws_bytes = need;
     }
-    struct Buf { void *p = nullptr; ~Buf() { if (p) cudaFree(p); } } dq, dr, dp, dk, de, dn;
+    DBuf dq, dr, dp, dk, de, dn;
     const size_t q = (size_t)Q;
-    AUV_CUDA(cudaMalloc(&dq.p, sizeof(auvrrt_astar_query_t) * q));
-    AUV_CUDA(cudaMalloc(&dr.p, sizeof(auvrrt_astar_record_t) * q));
-    if (paths) { AUV_CUDA(cudaMalloc(&dp.p, 48 * q * (size_t)path_cap)); AUV_CUDA(cudaMalloc(&dk.p, q * (size_t)path_cap)); }
-    if (expand_order) AUV_CUDA(cudaMalloc(&de.p, 4 * q * (size_t)node_cap));
-    if (node_xy) AUV_CUDA(cudaMalloc(&dn.p, 16 * q * (size_t)node_cap));
+    AUV_TRY(dq.alloc(sizeof(auvrrt_astar_query_t) * q));
+    AUV_TRY(dr.alloc(sizeof(auvrrt_astar_record_t) * q));
+    // path_cap 0 leaves the device path buffers NULL: the batch then writes records only
+    if (paths && path_cap != 0) { AUV_TRY(dp.alloc(48 * q * (size_t)path_cap)); AUV_TRY(dk.alloc(q * (size_t)path_cap)); }
+    if (expand_order) AUV_TRY(de.alloc(4 * q * (size_t)node_cap));
+    if (node_xy) AUV_TRY(dn.alloc(16 * q * (size_t)node_cap));
     AUV_CUDA(cudaMemcpyAsync(dq.p, queries, sizeof(auvrrt_astar_query_t) * q, cudaMemcpyHostToDevice, env->stream));
     if (paths) {     // rows past a query's path read as zeros
         AUV_CUDA(cudaMemsetAsync(dk.p, 0, q * (size_t)path_cap, env->stream));

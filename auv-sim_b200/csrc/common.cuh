@@ -266,4 +266,14 @@ int set_err(int code, const char *fmt, ...);
                                 cudaGetErrorString(e_));                                       \
     } while (0)
 
+// After every kernel launch: count it (auvrrt_launch_count) and report a failed launch as AUVRRT_ERR_CUDA.
+#define AUV_LAUNCH_CHECK()                                                                     \
+    do {                                                                                       \
+        auv::g_launches++;                                                                     \
+        cudaError_t e_ = cudaGetLastError();                                                   \
+        if (e_ != cudaSuccess)                                                                 \
+            return auv::set_err(AUVRRT_ERR_CUDA, "%s:%d launch: %s", __FILE__, __LINE__,       \
+                                cudaGetErrorString(e_));                                       \
+    } while (0)
+
 }  // namespace auv

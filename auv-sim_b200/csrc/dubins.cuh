@@ -59,7 +59,7 @@ __device__ __forceinline__ DubinsPath<R> dubins_shortest(R x0, R y0, R th0, R x1
     (void)sab;
     const R d2 = A::mul(d, d), two = (R)2;
     R bestc = A::inf();
-#define AUV_TRY(W, T_, P_, Q_)                                                    \
+#define AUV_DUBINS_WORD(W, T_, P_, Q_)                                            \
     {                                                                              \
         R tt = (T_), pp = (P_), qq = (Q_);                                         \
         R c = A::add(A::add(tt, pp), qq);                                          \
@@ -69,7 +69,7 @@ __device__ __forceinline__ DubinsPath<R> dubins_shortest(R x0, R y0, R th0, R x1
         R p2 = A::add(A::sub(A::add(two, d2), A::mul(two, cab)), A::mul(A::mul(two, d), A::sub(sa, sb)));
         if (p2 >= (R)0) {
             R t0 = M::atan2(A::sub(cb, ca), A::sub(A::add(d, sa), sb));
-            AUV_TRY(0, mod2pi<R>(A::sub(t0, alpha)), A::sqrt(p2), mod2pi<R>(A::sub(beta, t0)))
+            AUV_DUBINS_WORD(0, mod2pi<R>(A::sub(t0, alpha)), A::sqrt(p2), mod2pi<R>(A::sub(beta, t0)))
         }
     }
     {   // LSR
@@ -77,7 +77,7 @@ __device__ __forceinline__ DubinsPath<R> dubins_shortest(R x0, R y0, R th0, R x1
         if (p2 >= (R)0) {
             R p = A::sqrt(p2);
             R t0 = A::sub(M::atan2(A::sub(-ca, cb), A::add(A::add(d, sa), sb)), M::atan2(-two, p));
-            AUV_TRY(1, mod2pi<R>(A::sub(t0, alpha)), p, mod2pi<R>(A::sub(t0, mod2pi<R>(beta))))
+            AUV_DUBINS_WORD(1, mod2pi<R>(A::sub(t0, alpha)), p, mod2pi<R>(A::sub(t0, mod2pi<R>(beta))))
         }
     }
     {   // RSL
@@ -85,14 +85,14 @@ __device__ __forceinline__ DubinsPath<R> dubins_shortest(R x0, R y0, R th0, R x1
         if (p2 >= (R)0) {
             R p = A::sqrt(p2);
             R t0 = A::sub(M::atan2(A::add(ca, cb), A::sub(A::sub(d, sa), sb)), M::atan2(two, p));
-            AUV_TRY(2, mod2pi<R>(A::sub(alpha, t0)), p, mod2pi<R>(A::sub(beta, t0)))
+            AUV_DUBINS_WORD(2, mod2pi<R>(A::sub(alpha, t0)), p, mod2pi<R>(A::sub(beta, t0)))
         }
     }
     {   // RSR
         R p2 = A::add(A::sub(A::add(two, d2), A::mul(two, cab)), A::mul(A::mul(two, d), A::sub(sb, sa)));
         if (p2 >= (R)0) {
             R t0 = M::atan2(A::sub(ca, cb), A::add(A::sub(d, sa), sb));
-            AUV_TRY(3, mod2pi<R>(A::sub(alpha, t0)), A::sqrt(p2), mod2pi<R>(A::sub(t0, beta)))
+            AUV_DUBINS_WORD(3, mod2pi<R>(A::sub(alpha, t0)), A::sqrt(p2), mod2pi<R>(A::sub(t0, beta)))
         }
     }
     {   // RLR
@@ -101,7 +101,7 @@ __device__ __forceinline__ DubinsPath<R> dubins_shortest(R x0, R y0, R th0, R x1
             R ph = M::atan2(A::sub(ca, cb), A::add(A::sub(d, sa), sb));
             R p = mod2pi<R>(A::sub(M::two_pi(), M::acos(w)));
             R t = mod2pi<R>(A::add(A::sub(alpha, ph), mod2pi<R>(A::div(p, two))));
-            AUV_TRY(4, t, p, mod2pi<R>(A::add(A::sub(A::sub(alpha, beta), t), mod2pi<R>(p))))
+            AUV_DUBINS_WORD(4, t, p, mod2pi<R>(A::add(A::sub(A::sub(alpha, beta), t), mod2pi<R>(p))))
         }
     }
     {   // LRL
@@ -110,10 +110,10 @@ __device__ __forceinline__ DubinsPath<R> dubins_shortest(R x0, R y0, R th0, R x1
             R ph = M::atan2(A::sub(ca, cb), A::sub(A::add(d, sa), sb));
             R p = mod2pi<R>(A::sub(M::two_pi(), M::acos(w)));
             R t = mod2pi<R>(A::add(A::sub(-alpha, ph), A::div(p, two)));
-            AUV_TRY(5, t, p, mod2pi<R>(A::add(A::sub(A::sub(mod2pi<R>(beta), alpha), t), mod2pi<R>(p))))
+            AUV_DUBINS_WORD(5, t, p, mod2pi<R>(A::add(A::sub(A::sub(mod2pi<R>(beta), alpha), t), mod2pi<R>(p))))
         }
     }
-#undef AUV_TRY
+#undef AUV_DUBINS_WORD
     if (best.word >= 0) best.length = A::mul(bestc, rho);
     return best;
 }

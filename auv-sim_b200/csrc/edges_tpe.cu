@@ -306,9 +306,7 @@ static int launch_tpe_t(const auvrrt_env *env, const R *parents, const uint64_t 
     if (blocks > (int64_t)nsm * per_sm) blocks = (int64_t)nsm * per_sm;
     kern<<<(unsigned)blocks, nt, sm, s>>>(b.blob, b.hot_bytes, b.total_bytes, parents, seeds, (long long)n,
                                           make_steer_params<R>(params), (R)w3, safe, counts, leaf, cost_out);
-    g_launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "edges_arc (thread per edge) launch: %s", cudaGetErrorString(e));
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 

@@ -559,8 +559,7 @@ static int gym_reset_t(auvrrt_gym *g, const double *d_starts, const double *d_go
     if (S.counts) AUV_CUDA(cudaMemsetAsync(S.counts, 0, 2 * (size_t)g->Q * g->ncells, s));
     AUV_CUDA(cudaMemsetAsync(S.hash, 0, sizeof(GymHash) * (size_t)gym_hash_size(g->p.node_cap) * (size_t)g->Q, s));
     k_gym_reset<R><<<(unsigned)((g->Q + 127) / 128), 128, 0, s>>>(make_gymp<R>(g), S, d_starts, d_goals, d_seeds);
-    g_launches++;
-    AUV_CUDA(cudaGetLastError());
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 
@@ -569,8 +568,7 @@ static int gym_reset_masked_t(auvrrt_gym *g, const uint8_t *d_mask, const double
                               const uint64_t *d_seeds, cudaStream_t s) {
     const GymS<R> &S = *(const GymS<R> *)g->S;
     k_gym_reset_masked<R><<<(unsigned)((g->Q + 127) / 128), 128, 0, s>>>(make_gymp<R>(g), S, d_mask, d_starts, d_goals, d_seeds);
-    g_launches++;
-    AUV_CUDA(cudaGetLastError());
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 
@@ -579,8 +577,7 @@ static int gym_run_t(auvrrt_gym *g, const int32_t *d_actions, int n_steps, int f
     const GymS<R> &S = *(const GymS<R> *)g->S;
     k_gym_run<R><<<(unsigned)((g->Q + 127) / 128), 128, sizeof(R) * 3 * (size_t)(g->K > 0 ? g->K : 1), s>>>(
         make_gymp<R>(g), S, (const R *)g->d_circ, d_actions, n_steps, full, d_recs);
-    g_launches++;
-    AUV_CUDA(cudaGetLastError());
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 
@@ -588,8 +585,7 @@ template <typename R>
 static int gym_path_t(const auvrrt_gym *g, int64_t q, int cap, double *d_path, int *d_n, cudaStream_t s) {
     const GymS<R> &S = *(const GymS<R> *)g->S;
     k_gym_path<R><<<1, 32, 0, s>>>(make_gymp<R>(g), S, (const R *)g->d_circ, (long long)q, cap, d_path, d_n);
-    g_launches++;
-    AUV_CUDA(cudaGetLastError());
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 
@@ -624,8 +620,6 @@ static int gym_tree_t(const auvrrt_gym *g, int64_t q, int32_t cap, double *nodes
 
 using namespace auv;
 
-#define GYM_DISPATCH(g, fn, ...) ((g)->precision == AUVRRT_F64 ? fn<double>(__VA_ARGS__) : fn<float>(__VA_ARGS__))
-
 extern "C" int auvrrt_gym_create(const double *circles, int K, const auvrrt_gym_params_t *params, int64_t Q, int precision,
                                  int device, auvrrt_gym_t **out) {
     if (!params || !out || Q <= 0 || K < 0 || (K > 0 && !circles)) return set_err(AUVRRT_ERR_ARG, "gym_create: bad arguments");
@@ -633,9 +627,7 @@ extern "C" int auvrrt_gym_create(const double *circles, int K, const auvrrt_gym_
     if (params->subsections <= 0 || params->node_cap < 2 || !(params->cell_side > 0) || !(params->exp_rate > 0))
         return set_err(AUVRRT_ERR_ARG, "gym_create: subsections, node_cap >= 2, cell_side and exp_rate must be positive");
     if (K > 2048) return set_err(AUVRRT_ERR_UNSUPPORTED, "gym_create: at most 2048 obstacles");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return set_err(AUVRRT_ERR_CUDA, "gym_create: no CUDA device (no CPU fallback)"); }
-    AUV_CUDA(cudaSetDevice(device));
+    AUV_TRY(need_device(device));
     auvrrt_gym *g = new (std::nothrow) auvrrt_gym();
     if (!g) return set_err(AUVRRT_ERR_ARG, "gym_create: out of memory");
     g->device = device; g->precision = precision; g->Q = Q; g->p = *params; g->K = K;
@@ -647,7 +639,7 @@ extern "C" int auvrrt_gym_create(const double *circles, int K, const auvrrt_gym_
     g->rows = (int)(hh / cs); g->cols = (int)(ww / cs);
     g->ncells = g->rows * g->cols * params->subsections;
     if (params->track_counts && (size_t)2 * Q * g->ncells > ((size_t)64 << 30)) { delete g; return set_err(AUVRRT_ERR_ARG, "gym_create: dense counts would need more than 64 GiB"); }
-    int rc = GYM_DISPATCH(g, gym_create_t, g, circles);
+    int rc = AUV_DISPATCH(g->precision, gym_create_t, g, circles);
     if (rc == AUVRRT_OK) {
         cudaError_t e = cudaMalloc((void **)&g->d_actions, 4 * (size_t)Q);
         if (e == cudaSuccess) e = cudaMalloc((void **)&g->d_recs, sizeof(auvrrt_gym_record_t) * (size_t)Q);
@@ -679,20 +671,17 @@ extern "C" int auvrrt_gym_reset(auvrrt_gym_t *g, const double *starts, const dou
     if (!g || !starts || !goals || !seeds) return set_err(AUVRRT_ERR_ARG, "gym_reset: null argument");
     AUV_CUDA(cudaSetDevice(g->device));
     const size_t Q = (size_t)g->Q;
-    double *d = nullptr;
-    AUV_CUDA(cudaMalloc((void **)&d, 8 * Q * 6));
-    double *d_starts = d, *d_goals = d + 3 * Q;
-    uint64_t *d_seeds = (uint64_t *)(d + 5 * Q);
-    cudaError_t e = cudaMemcpyAsync(d_starts, starts, 24 * Q, cudaMemcpyHostToDevice, g->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_goals, goals, 16 * Q, cudaMemcpyHostToDevice, g->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_seeds, seeds, 8 * Q, cudaMemcpyHostToDevice, g->stream);
-    int rc = e == cudaSuccess ? GYM_DISPATCH(g, gym_reset_t, g, d_starts, d_goals, d_seeds, g->stream)
-                              : set_err(AUVRRT_ERR_CUDA, "gym_reset: %s", cudaGetErrorString(e));
-    e = cudaStreamSynchronize(g->stream);
-    cudaFree(d);
-    if (rc == AUVRRT_OK && e != cudaSuccess) rc = set_err(AUVRRT_ERR_CUDA, "gym_reset: %s", cudaGetErrorString(e));
-    if (rc == AUVRRT_OK) g->reset_once = true;
-    return rc;
+    DBuf d;
+    AUV_TRY(d.alloc(8 * Q * 6));
+    double *d_starts = d.as<double>(), *d_goals = d_starts + 3 * Q;
+    uint64_t *d_seeds = (uint64_t *)(d_starts + 5 * Q);
+    AUV_CUDA(cudaMemcpyAsync(d_starts, starts, 24 * Q, cudaMemcpyHostToDevice, g->stream));
+    AUV_CUDA(cudaMemcpyAsync(d_goals, goals, 16 * Q, cudaMemcpyHostToDevice, g->stream));
+    AUV_CUDA(cudaMemcpyAsync(d_seeds, seeds, 8 * Q, cudaMemcpyHostToDevice, g->stream));
+    AUV_TRY(AUV_DISPATCH(g->precision, gym_reset_t, g, d_starts, d_goals, d_seeds, g->stream));
+    AUV_CUDA(cudaStreamSynchronize(g->stream));
+    g->reset_once = true;
+    return AUVRRT_OK;
 }
 
 extern "C" int auvrrt_gym_reset_dev(auvrrt_gym_t *g, const uint8_t *d_mask, const double *d_starts, const double *d_goals,
@@ -702,8 +691,8 @@ extern "C" int auvrrt_gym_reset_dev(auvrrt_gym_t *g, const uint8_t *d_mask, cons
         return set_err(AUVRRT_ERR_ARG, "gym_reset_dev: a masked reset reads each episode's previous tree, which is undefined "
                                        "until the handle has had one full reset (d_mask = NULL or auvrrt_gym_reset)");
     AUV_CUDA(cudaSetDevice(g->device));
-    const int rc = d_mask ? GYM_DISPATCH(g, gym_reset_masked_t, g, d_mask, d_starts, d_goals, d_seeds, (cudaStream_t)stream)
-                          : GYM_DISPATCH(g, gym_reset_t, g, d_starts, d_goals, d_seeds, (cudaStream_t)stream);
+    const int rc = d_mask ? AUV_DISPATCH(g->precision, gym_reset_masked_t, g, d_mask, d_starts, d_goals, d_seeds, (cudaStream_t)stream)
+                          : AUV_DISPATCH(g->precision, gym_reset_t, g, d_starts, d_goals, d_seeds, (cudaStream_t)stream);
     if (rc == AUVRRT_OK && !d_mask) g->reset_once = true;
     return rc;
 }
@@ -713,7 +702,7 @@ extern "C" int auvrrt_gym_step_dev(auvrrt_gym_t *g, const int32_t *d_actions, in
     if (!g || n_steps < 0) return set_err(AUVRRT_ERR_ARG, "gym_step: bad arguments");
     if (d_actions && n_steps != 1) return set_err(AUVRRT_ERR_ARG, "gym_step: n_steps must be 1 when actions are given");
     AUV_CUDA(cudaSetDevice(g->device));
-    return GYM_DISPATCH(g, gym_run_t, g, d_actions, n_steps, full_candidates, d_records, (cudaStream_t)stream);
+    return AUV_DISPATCH(g->precision, gym_run_t, g, d_actions, n_steps, full_candidates, d_records, (cudaStream_t)stream);
 }
 
 extern "C" int auvrrt_gym_step(auvrrt_gym_t *g, const int32_t *actions, int n_steps, int full_candidates,
@@ -734,7 +723,7 @@ extern "C" int auvrrt_gym_tree(const auvrrt_gym_t *g, int64_t q, int32_t cap, do
     if (!g || q < 0 || q >= g->Q) return set_err(AUVRRT_ERR_ARG, "gym_tree: bad episode index");
     AUV_CUDA(cudaSetDevice(g->device));
     AUV_CUDA(cudaStreamSynchronize(g->stream));
-    return GYM_DISPATCH(g, gym_tree_t, g, q, cap, nodes, parents, cells, occupied, n_nodes, n_occupied);
+    return AUV_DISPATCH(g->precision, gym_tree_t, g, q, cap, nodes, parents, cells, occupied, n_nodes, n_occupied);
 }
 
 extern "C" const uint16_t *auvrrt_gym_counts_dev(const auvrrt_gym_t *g) {
@@ -755,18 +744,15 @@ extern "C" int auvrrt_gym_counts(const auvrrt_gym_t *g, int64_t q0, int64_t nq, 
 extern "C" int auvrrt_gym_path(const auvrrt_gym_t *g, int64_t q, int32_t cap, double *path, int32_t *n_path) {
     if (!g || q < 0 || q >= g->Q || cap < 0 || !n_path || (cap > 0 && !path)) return set_err(AUVRRT_ERR_ARG, "gym_path: bad arguments");
     AUV_CUDA(cudaSetDevice(g->device));
-    double *d_path = nullptr;
-    int *d_n = nullptr;
-    AUV_CUDA(cudaMalloc((void **)&d_path, 24 * (size_t)(cap > 0 ? cap : 1) + 16));
-    d_n = (int *)(d_path + 3 * (size_t)(cap > 0 ? cap : 1));
-    int rc = GYM_DISPATCH(g, gym_path_t, g, q, cap, d_path, d_n, g->stream);
-    cudaError_t e = cudaStreamSynchronize(g->stream);
+    DBuf d;
+    AUV_TRY(d.alloc(24 * (size_t)(cap > 0 ? cap : 1) + 16));
+    double *d_path = d.as<double>();
+    int *d_n = (int *)(d_path + 3 * (size_t)(cap > 0 ? cap : 1));
+    AUV_TRY(AUV_DISPATCH(g->precision, gym_path_t, g, q, cap, d_path, d_n, g->stream));
+    AUV_CUDA(cudaStreamSynchronize(g->stream));
     int n = 0;
-    if (rc == AUVRRT_OK && e == cudaSuccess) e = cudaMemcpy(&n, d_n, 4, cudaMemcpyDeviceToHost);
-    if (rc == AUVRRT_OK && e == cudaSuccess && n <= cap && n > 0) e = cudaMemcpy(path, d_path, 24 * (size_t)n, cudaMemcpyDeviceToHost);
-    cudaFree(d_path);
-    if (rc != AUVRRT_OK) return rc;
-    if (e != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "gym_path: %s", cudaGetErrorString(e));
+    AUV_CUDA(cudaMemcpy(&n, d_n, 4, cudaMemcpyDeviceToHost));
+    if (n <= cap && n > 0) AUV_CUDA(cudaMemcpy(path, d_path, 24 * (size_t)n, cudaMemcpyDeviceToHost));
     *n_path = n;
     if (n > cap) return set_err(AUVRRT_ERR_ARG, "gym_path: cap %d < path length %d", cap, n);
     return AUVRRT_OK;

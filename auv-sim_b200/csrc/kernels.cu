@@ -20,15 +20,6 @@ int set_err(int code, const char *fmt, ...) {
     return code;
 }
 
-#define AUV_LAUNCH_CHECK()                                                                  \
-    do {                                                                                    \
-        g_launches++;                                                                       \
-        cudaError_t e_ = cudaGetLastError();                                                \
-        if (e_ != cudaSuccess)                                                              \
-            return set_err(AUVRRT_ERR_CUDA, "%s:%d launch: %s", __FILE__, __LINE__,         \
-                           cudaGetErrorString(e_));                                         \
-    } while (0)
-
 template <> SteerParams<float> make_steer_params<float>(const double p[5]) {
     SteerParams<float> s;
     s.d2e = (float)p[0]; s.dmax = (float)p[1]; s.neg_dmax = (float)(-p[1]); s.freq = (float)p[2];
@@ -74,20 +65,22 @@ template <typename R> __global__ void k_convert_back(const R *src, double *dst, 
     int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i < n) dst[i] = (double)src[i];
 }
-template <typename R> void launch_convert(const double *src, R *dst, int64_t n, cudaStream_t s) {
-    if (n <= 0) return;
+template <typename R> int launch_convert(const double *src, R *dst, int64_t n, cudaStream_t s) {
+    if (n <= 0) return AUVRRT_OK;
     k_convert<R><<<(unsigned)((n + 255) / 256), 256, 0, s>>>(src, dst, n);
-    g_launches++;
+    AUV_LAUNCH_CHECK();
+    return AUVRRT_OK;
 }
-template <typename R> void launch_convert_back(const R *src, double *dst, int64_t n, cudaStream_t s) {
-    if (n <= 0) return;
+template <typename R> int launch_convert_back(const R *src, double *dst, int64_t n, cudaStream_t s) {
+    if (n <= 0) return AUVRRT_OK;
     k_convert_back<R><<<(unsigned)((n + 255) / 256), 256, 0, s>>>(src, dst, n);
-    g_launches++;
+    AUV_LAUNCH_CHECK();
+    return AUVRRT_OK;
 }
-template void launch_convert<float>(const double *, float *, int64_t, cudaStream_t);
-template void launch_convert<double>(const double *, double *, int64_t, cudaStream_t);
-template void launch_convert_back<float>(const float *, double *, int64_t, cudaStream_t);
-template void launch_convert_back<double>(const double *, double *, int64_t, cudaStream_t);
+template int launch_convert<float>(const double *, float *, int64_t, cudaStream_t);
+template int launch_convert<double>(const double *, double *, int64_t, cudaStream_t);
+template int launch_convert_back<float>(const float *, double *, int64_t, cudaStream_t);
+template int launch_convert_back<double>(const double *, double *, int64_t, cudaStream_t);
 
 // ------------------------------------------------------------------ RRT.steer on explicit streams
 template <typename R, int G>
@@ -850,24 +843,24 @@ __global__ void __launch_bounds__(256) k_ffma(float *out, int iters, float a, fl
     if (r == 123.456f) out[0] = r;
 }
 int launch_calibrate_fp32(int iters, double *flops, double *ms_out) {
-    float *d;
-    AUV_CUDA(cudaMalloc(&d, 4));
+    DBuf d;
+    AUV_TRY(d.alloc(4));
     cudaEvent_t e0, e1;
     AUV_CUDA(cudaEventCreate(&e0));
     AUV_CUDA(cudaEventCreate(&e1));
     const int blocks = AUV_SMS * 8;
-    k_ffma<<<blocks, 256>>>(d, 64, 0.999f, 0.001f);   // warm-up
-    g_launches++;
+    k_ffma<<<blocks, 256>>>(d.as<float>(), 64, 0.999f, 0.001f);   // warm-up
+    AUV_LAUNCH_CHECK();
     AUV_CUDA(cudaEventRecord(e0));
-    k_ffma<<<blocks, 256>>>(d, iters, 0.999f, 0.001f);
-    g_launches++;
+    k_ffma<<<blocks, 256>>>(d.as<float>(), iters, 0.999f, 0.001f);
+    AUV_LAUNCH_CHECK();
     AUV_CUDA(cudaEventRecord(e1));
     AUV_CUDA(cudaEventSynchronize(e1));
     float ms;
     AUV_CUDA(cudaEventElapsedTime(&ms, e0, e1));
     *ms_out = ms;
     *flops = (double)blocks * 256.0 * (double)iters * 16.0 * 8.0 * 2.0 / (ms * 1e-3);
-    cudaEventDestroy(e0); cudaEventDestroy(e1); cudaFree(d);
+    cudaEventDestroy(e0); cudaEventDestroy(e1);
     return AUVRRT_OK;
 }
 

@@ -22,6 +22,31 @@ struct auvrrt_env {
 
 namespace auv {
 
+#define AUV_TRY(x) do { int rc_ = (x); if (rc_) return rc_; } while (0)
+
+// fn<double>(args...) for AUVRRT_F64, fn<float>(args...) for AUVRRT_F32 (the caller has checked the precision)
+#define AUV_DISPATCH(precision, fn, ...) ((precision) == AUVRRT_F64 ? fn<double>(__VA_ARGS__) : fn<float>(__VA_ARGS__))
+
+// AUVRRT_OK with `device` current; "no CUDA device" (AUVRRT_ERR_CUDA) without one, AUVRRT_ERR_ARG out of range
+int need_device(int device);
+
+// A device allocation owned by one scope.  Zero bytes allocate 16, so every buffer has a valid address.
+struct DBuf {
+    void *p = nullptr;
+    size_t bytes = 0;
+    DBuf() = default;
+    DBuf(const DBuf &) = delete;
+    DBuf &operator=(const DBuf &) = delete;
+    int alloc(size_t n) {
+        bytes = n ? n : 16;
+        cudaError_t e = cudaMalloc(&p, bytes);
+        if (e != cudaSuccess) { p = nullptr; return set_err(AUVRRT_ERR_CUDA, "cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e)); }
+        return AUVRRT_OK;
+    }
+    template <typename T> T *as() { return (T *)p; }
+    ~DBuf() { if (p) cudaFree(p); }
+};
+
 template <typename R> struct EnvBlob { const unsigned char *blob; int hot_bytes; int total_bytes; int off_probs; };
 template <typename R> inline EnvBlob<R> env_blob(const auvrrt_env *e);
 template <> inline EnvBlob<float> env_blob<float>(const auvrrt_env *e) {
@@ -67,8 +92,8 @@ int launch_nn(const R *tx, const R *ty, int64_t n, const R *qx, const R *qy, int
               int64_t scratch_bytes, int32_t *out_idx, cudaStream_t s);
 int64_t nn_scratch_bytes(int nq);
 int launch_calibrate_fp32(int iters, double *flops, double *ms);
-template <typename R> void launch_convert(const double *src, R *dst, int64_t n, cudaStream_t s);
-template <typename R> void launch_convert_back(const R *src, double *dst, int64_t n, cudaStream_t s);
+template <typename R> int launch_convert(const double *src, R *dst, int64_t n, cudaStream_t s);
+template <typename R> int launch_convert_back(const R *src, double *dst, int64_t n, cudaStream_t s);
 
 // ---- occupancy.cu: the one writer of both blobs' probs[T][C]: grid[b][cell_sq[c]] of a [T][RC] grid, or src[b][c]
 // when cell_sq is NULL

@@ -18,6 +18,7 @@
 #include <string.h>
 #include <algorithm>
 #include <cmath>
+#include <memory>
 #include <vector>
 #include "launch.h"
 
@@ -151,8 +152,7 @@ int launch_probs_to_env(auvrrt_env *env, const double *src, const int *cell_sq, 
     k_occ_to_env<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(src, cell_sq, env->T, env->C, RC,
                                                              (double *)(env->blob64 + env->h64.off_probs),
                                                              (float *)(env->blob32 + env->h32.off_probs));
-    g_launches++;
-    AUV_CUDA(cudaGetLastError());
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 
@@ -275,10 +275,7 @@ extern "C" int auvrrt_occ_create(const double *cell_xy, const int64_t *cell_off,
         for (int b = 0; b <= NBK; b++) boff[b] = (int)cnt[b];
     }
     if (bcell.empty()) bcell.push_back(0);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { cudaGetLastError(); return set_err(AUVRRT_ERR_CUDA, "no CUDA device: libauvrrt has no CPU fallback"); }
-    if (device < 0 || device >= ndev) return set_err(AUVRRT_ERR_ARG, "device %d out of range (%d devices)", device, ndev);
-    AUV_CUDA(cudaSetDevice(device));
+    AUV_TRY(need_device(device));
     // one allocation: the tables (uploaded once), then the workspace
     const size_t nv = C > 0 ? (size_t)cell_off[C] : 0, ws = (size_t)n_bins * max_sharks * RC;
     size_t o = 0;
@@ -356,13 +353,14 @@ extern "C" int auvrrt_occ_grid_dev(auvrrt_occ_t *o, const double *d_tracks, cons
         k_occ_hist<<<(unsigned)((n_points + 255) / 256), 256, 0, s>>>(o->d_xy, o->d_off, o->d_bb, o->d_csq, o->d_boff, o->d_bcell, o->ix,
                                                                       d_tracks, (const long long *)d_track_off, n_points, T, S, RC,
                                                                       o->bin_interval, o->d_cnt, o->d_np, d_t_occ);
-        g_launches++;
+        AUV_LAUNCH_CHECK();
     }
     k_occ_norm<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(o->d_cnt, o->d_np, o->d_isc, T, S, RC, o->C, o->d_occ);
+    AUV_LAUNCH_CHECK();
     k_occ_auv<<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(o->d_occ, o->d_sqo, T, S, o->rows, o->cols, o->count, o->d_auv);
+    AUV_LAUNCH_CHECK();
     k_occ_avg<<<(unsigned)(((long long)T * RC + 255) / 256), 256, 0, s>>>(o->d_auv, T, S, RC, grid);
-    g_launches += 3;
-    AUV_CUDA(cudaGetLastError());
+    AUV_LAUNCH_CHECK();
     if (env) return launch_probs_to_env(env, grid, o->d_csq, RC, s);
     return AUVRRT_OK;
 }
@@ -378,17 +376,16 @@ extern "C" int auvrrt_occupancy_grid(const double *cell_xy, const int64_t *cell_
     const int RC = rows * cols;
     if ((int64_t)T * RC > out_cap) return set_err(AUVRRT_ERR_ARG, "occupancy_grid: output holds %lld values, %lld needed", (long long)out_cap, (long long)T * RC);
     if (T == 0) return AUVRRT_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { cudaGetLastError(); return set_err(AUVRRT_ERR_CUDA, "no CUDA device: libauvrrt has no CPU fallback"); }
-    AUV_CUDA(cudaSetDevice(device));
+    AUV_TRY(need_device(device));
     const int64_t n = track_off[S];
     auvrrt_occ_t *o = nullptr;
     if ((rc = auvrrt_occ_create(cell_xy, cell_off, C, bounds, cell_size, bin_interval, detect_range, T, S, n, device, &o))) return rc;
-    struct Owned { auvrrt_occ_t *o; void *p = nullptr; ~Owned() { if (p) cudaFree(p); auvrrt_occ_destroy(o); } } own{o};
+    std::unique_ptr<auvrrt_occ_t, void (*)(auvrrt_occ_t *)> own(o, auvrrt_occ_destroy);
     const size_t trk_bytes = (24 * (size_t)n + 255) & ~(size_t)255;
-    AUV_CUDA(cudaMalloc(&own.p, trk_bytes + 8 * (size_t)(S + 1)));
-    double *d_trk = (double *)own.p;
-    int64_t *d_toff = (int64_t *)((unsigned char *)own.p + trk_bytes);
+    DBuf trk;
+    AUV_TRY(trk.alloc(trk_bytes + 8 * (size_t)(S + 1)));
+    double *d_trk = trk.as<double>();
+    int64_t *d_toff = (int64_t *)((unsigned char *)trk.p + trk_bytes);
     if (n > 0) AUV_CUDA(cudaMemcpy(d_trk, tracks, 24 * (size_t)n, cudaMemcpyHostToDevice));
     AUV_CUDA(cudaMemcpy(d_toff, track_off, 8 * (size_t)(S + 1), cudaMemcpyHostToDevice));
     if ((rc = auvrrt_occ_grid_dev(o, d_trk, d_toff, S, n, nullptr, nullptr, nullptr, 0))) return rc;

@@ -32,15 +32,6 @@
 
 namespace auv {
 
-#define AUV_LAUNCH_CHECK2()                                                                 \
-    do {                                                                                    \
-        g_launches++;                                                                       \
-        cudaError_t e_ = cudaGetLastError();                                                \
-        if (e_ != cudaSuccess)                                                              \
-            return set_err(AUVRRT_ERR_CUDA, "%s:%d launch: %s", __FILE__, __LINE__,         \
-                           cudaGetErrorString(e_));                                         \
-    } while (0)
-
 // CTA shape of k_plan.  Config 2's 4096 trees (one warp each) need 28 resident warps per SM to run in one wave
 // (4096 / 148 = 27.7) and get 72 registers per thread.  Every CTA stages its own copy of the world model's hot part
 // (11 KB), so fewer, larger CTAs leave more of the SM to the L1 that serves the trees, the classification grid and the
@@ -767,7 +758,7 @@ static int launch_plan_gb(const auvrrt_env *env, const R *starts, const uint64_t
     k_plan<R, G, BS, MODE, ONE><<<grid, PlanCta<R, G>::T, smem, s>>>(b.blob, b.hot_bytes, b.total_bytes, mode, ev, starts, seeds, (long long)Q, P, L,
                                                   (unsigned char *)workspace + 256, (unsigned long long *)workspace,
                                                   records, chain, path, tr);
-    AUV_LAUNCH_CHECK2();
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 
@@ -867,7 +858,7 @@ int launch_materialize(const auvrrt_env *env, const R *starts, const uint64_t *s
     else if (G == 16) k_materialize<R, 16><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
     else if (G == 8) k_materialize<R, 8><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
     else return set_err(AUVRRT_ERR_ARG, "materialize: group must be 32, 16, 8 or 1");
-    AUV_LAUNCH_CHECK2();
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 template int launch_materialize<float>(const auvrrt_env *, const float *, const uint64_t *, const uint32_t *, const int32_t *,

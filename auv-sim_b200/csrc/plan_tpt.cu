@@ -394,9 +394,7 @@ int launch_plan_tpt(const auvrrt_env *env, const R *starts, const uint64_t *seed
     kern<<<grid, TPT_THREADS, sm, s>>>(b.blob, b.hot_bytes, b.total_bytes, mode, starts, seeds, (long long)Q, P, L,
                                                 (unsigned char *)workspace + 256, (unsigned long long *)workspace, records,
                                                 chain, tr);
-    g_launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "plan_tpt launch: %s", cudaGetErrorString(e));
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 // ---- re-create paths of thread-per-tree plans from (start, seed, chain of stream positions) ----------------------
@@ -451,9 +449,7 @@ int launch_materialize_tpt(const auvrrt_env *env, const R *starts, const uint64_
     if (blocks > AUV_SMS * 8) blocks = AUV_SMS * 8;
     k_materialize_tpt<R><<<(unsigned)blocks, 128, 0, s>>>(env_blob<R>(env).blob, starts, seeds, chain, depth, (long long)Q, P,
                                                           path, n_path);
-    g_launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return set_err(AUVRRT_ERR_CUDA, "materialize_tpt launch: %s", cudaGetErrorString(e));
+    AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
 template int launch_materialize_tpt<float>(const auvrrt_env *, const float *, const uint64_t *, const uint32_t *, const int32_t *,

@@ -43,6 +43,15 @@ def test_no_cpu_fallback(auvrrt):
         auvrrt.Env([[0, 0, 1]], [[0, 0], [1, 0], [0, 1]])
     with pytest.raises(auvrrt.AuvrrtError, match="no CUDA device"):
         auvrrt.api.nn([[0, 0]], [[1, 1]])
+    with pytest.raises(auvrrt.AuvrrtError, match="no CUDA device"):
+        auvrrt.api.steer_arc([[0, 0, 0, 0, 0]], [0.5] * 4, [0, 4], [2.0, 0.5, 30.0, 0.5, 2.0])
+    with pytest.raises(auvrrt.AuvrrtError, match="no CUDA device"):
+        auvrrt.api.steer_dubins([[0, 0, 0]], [[5, 5, 1]], W=4)
+    with pytest.raises(auvrrt.AuvrrtError, match="no CUDA device"):
+        auvrrt.api.calibrate_fp32()
+    from auvrrt import device
+    with pytest.raises(auvrrt.AuvrrtError, match="no CUDA device"):
+        device.SharkOccupancy([[[0, 0], [1, 0], [1, 1], [0, 1]]], [0, 0, 4, 4], 1.0, 5.0, 2.0, 2, 1, 16)
 
 
 def test_product_never_imports_oracle():

@@ -22,14 +22,6 @@
 #include "plan_common.cuh"
 #include "dubins.cuh"
 
-// Rehearse the next iteration's parent pick and prefetch its row (k_plan, default parent pick).  Measured on B200,
-// config 2: 9.77 ms per step with it, 8.89 ms without -- the parent-row load is 17 % of the stall samples, but the
-// rehearsal costs ~50 instructions per iteration in a kernel whose issue slots are 68 % busy, and the prefetched line
-// competes with the tree's own lines in a 28-warp L1.  Off.
-#ifndef AUV_PLAN_PREFETCH
-#define AUV_PLAN_PREFETCH 0
-#endif
-
 namespace auv {
 
 // CTA shape of k_plan.  Config 2's 4096 trees (one warp each) need 28 resident warps per SM to run in one wave
@@ -52,7 +44,7 @@ template <typename R, int G> struct PlanCta {
 
 struct WsLayout {
     size_t slot_bytes;
-    size_t rows, xy, pool, next, head, tail, count;
+    size_t rows, xy, pool, pose, next, head, tail, count;
 };
 
 template <typename R> static WsLayout make_layout(int cap, int nb, int nchunks) {
@@ -61,7 +53,9 @@ template <typename R> static WsLayout make_layout(int cap, int nb, int nchunks) 
     auto take = [&](size_t bytes) { size_t r = o; o += (bytes + 127) & ~(size_t)127; return r; };
     L.rows = take(sizeof(NodeRow<R>) * (size_t)cap);
     L.xy = take(2 * sizeof(R) * (size_t)cap);                 // SoA copy of (x, y) for the nearest-node scan
-    L.pool = take(4 * 32 * (size_t)nchunks); L.next = take(4 * (size_t)nchunks);
+    L.pool = take(4 * 32 * (size_t)nchunks);
+    L.pose = take(16 * 32 * (size_t)nchunks);                 // (x, y, theta, t) of every pool entry, same index
+    L.next = take(4 * (size_t)nchunks);
     L.head = take(4 * (size_t)(nb + 2)); L.tail = take(4 * (size_t)(nb + 2)); L.count = take(4 * (size_t)(nb + 2));
     L.slot_bytes = o;
     return L;
@@ -77,6 +71,7 @@ template <typename R> struct Tree {
     __device__ __forceinline__ R *nx() const { return (R *)(b + L.xy); }         // coalesced x[] / y[] for RRT.get_closest_mps (mode 1)
     __device__ __forceinline__ R *ny() const { return nx() + cap; }
     __device__ __forceinline__ int *pool() const { return (int *)(b + L.pool); }
+    __device__ __forceinline__ float4 *pose() const { return (float4 *)(b + L.pose); }
     __device__ __forceinline__ int *next() const { return (int *)(b + L.next); }
     __device__ __forceinline__ int *head() const { return (int *)(b + L.head); }
     __device__ __forceinline__ int *tail() const { return (int *)(b + L.tail); }
@@ -149,11 +144,12 @@ __device__ __forceinline__ void dubins_sample_at(const EnvView<R> &env, const St
 
 #define AUV_BINS_SMEM 128
 template <typename R> struct BestPlan { R c0, c1, c2, len, t; int node, iter; };
-// a group's shared state, reached from one shared address: edge scratch, the best plan so far and, with BS, the bin
-// metadata (count / head chunk / tail chunk)
+// a group's shared state, reached from one shared address: edge scratch, the best plan so far, the picked parent's row
+// (single-chunk time-bin kernel: copied in behind the edge) and, with BS, the bin metadata (count / head chunk / tail chunk)
 template <typename R, int G, bool BS> struct GroupSmem {
     GroupScratch<R, G, false> sc;
     BestPlan<R> best;
+    NodeRow<R> prow;
     unsigned short bins[3][BS ? AUV_BINS_SMEM : 1];
 };
 // MODE >= 0 compiles the kernel for that parent-pick mode alone (the other modes' code -- about 1000 instructions that
@@ -168,6 +164,10 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
     typedef typename Policy<R>::A A;
     const bool VERIFY = Policy<R>::VERIFY;
     const int pick_mode = MODE >= 0 ? MODE : P.mode;
+    // Pose-carrying pool (the single-chunk time-bin kernel): every pool entry also holds its node's (x, y, theta, t), so
+    // the parent pick ends in one global load of the state the edge starts from.  The rest of the parent's row is copied
+    // to shared memory behind the edge.  Rows of every node are still written: everything after the loop reads them.
+    const bool POSE = ONE && BS && MODE == 0 && sizeof(R) == 4;
     extern __shared__ __align__(16) unsigned char smem[];
     const int PLAN_THREADS = PlanCta<R, G>::T;
     __shared__ GroupSmem<R, G, BS> groups[PlanCta<R, G>::T / G];
@@ -247,7 +247,10 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
             if (pick_mode == 1 || pick_mode == 3) { T.nx()[0] = sx; T.ny()[0] = sy; }
         }
         g.sync();
-        if (g.gl == 0) { SET_BIN_HEAD(1, 0); SET_BIN_TAIL(1, 0); SET_BIN_COUNT(1, 1); T.pool()[0] = 0; T.next()[0] = -1; }
+        if (g.gl == 0) {
+            SET_BIN_HEAD(1, 0); SET_BIN_TAIL(1, 0); SET_BIN_COUNT(1, 1); T.pool()[0] = 0; T.next()[0] = -1;
+            if (POSE) T.pose()[0] = make_float4((float)sx, (float)sy, (float)sth, (float)st);
+        }
         g.sync();
         Stream<R> rng;                 // (after the root's cost: the key is not live across it)
         rng.key = stream_key(seeds[q]); rng.ext = nullptr; rng.n_ext = 0;
@@ -266,6 +269,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
 
         while (it < P.I && guard++ < guard_max) {
             int parent;
+            float4 ppose;                 // POSE: the parent's (x, y, theta, t) from its pool entry
             if (pick_mode == 3) {
                 // ================= mode 3: Dubins-RRT with best-parent selection =================
                 // lane = candidate parent: each lane evaluates ONE candidate edge (steer + collide + cost), a warp
@@ -416,7 +420,9 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                 int ch = BIN_HEAD(ran_bin);
 #pragma unroll 1
                 for (int hop = idx >> 5; hop > 0; hop--) ch = T.next()[ch];
-                parent = T.pool()[ch * 32 + (idx & 31)];
+                const int e = ch * 32 + (idx & 31);
+                if (POSE) ppose = T.pose()[e];          // (independent of the node id: both loads are in flight at once)
+                parent = T.pool()[e];
             } else if (pick_mode == 2) {
                 // ---- wall-clock pick on the simulated clock (:129-132): every lane walks the same bisection
                 const R ran_time = uniform_ab<R>((R)0, P.ran_time_max, rng.u(ctr));
@@ -451,36 +457,30 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
             // every lane reads the same row (a broadcast): the state now, the cost prefix after the edge and only if it is
             // safe (the line is then in L1), so that the prefix is not live across the edge evaluation
             const NodeRow<R> *prow = T.row() + parent;
-            const R ppx = prow->x, ppy = prow->y, ppth = prow->th, ppt = prow->t, pplen = prow->len;
-            const uint32_t ctr0 = ctr;
-#if AUV_PLAN_PREFETCH
-            // Look ahead.  Slot addressing makes the next iteration's stream position known now (this edge owns
-            // 1 + 3 n_expand positions), so its parent pick can be rehearsed on the bins as they stand: the pool entry is
-            // requested here and the parent's row prefetched behind the edge, while this edge is being evaluated.  The
-            // real pick of the next iteration runs unchanged (an append into a rehearsed bin changes it) and finds both
-            // lines in cache.
-            int spec_parent = -1;
-            if (ONE && BS && pick_mode == 0) {
-                const int n_exp_now = (int)A::floor(uniform_ab<R>((R)0, P.sp.freq, rng.u(ctr)));
-                const uint32_t cn0 = ctr + 1u + 3u * (uint32_t)(n_exp_now > 0 ? n_exp_now : 0);
-                const int rb = (int)uniform_ab<R>((R)1, (R)(P.nb + 1), rng.u(cn0 + (uint32_t)g.gl));
-                const int cn = (rb >= 1 && rb <= P.nb) ? (int)gs.bins[0][rb] : 0;
-                const unsigned m = g.ballot(cn > 0);
-                if (m) {
-                    const int f = __ffs(m) - 1;
-                    const int sb = g.bcast(rb, f), sc_ = g.bcast(cn, f);
-                    const int idx = (int)uniform_ab<R>((R)0, (R)sc_, rng.u(cn0 + (uint32_t)f + 1u));
-                    if (idx < 32 && idx < sc_) spec_parent = T.pool()[(int)gs.bins[1][sb] * 32 + idx];
-                }
+            R ppx, ppy, ppth, ppt, pplen;
+            if (POSE) {
+                // the row's copy into shared memory (4 lanes x 16 bytes) runs under the edge; the edge starts from the
+                // pool's pose and from length 0, the parent's length is added to the leaf's after the edge
+                if (g.gl < 4)
+                    asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(smem_u32(&gs.prow) + 16u * g.gl),
+                                 "l"((const char *)prow + 16 * g.gl) : "memory");
+                ppx = ppose.x; ppy = ppose.y; ppth = ppose.z; ppt = ppose.w; pplen = (R)0;
+            } else {
+                ppx = prow->x; ppy = prow->y; ppth = prow->th; ppt = prow->t; pplen = prow->len;
             }
-#endif
+            const uint32_t ctr0 = ctr;
             EdgeOut<R> o;
             eval_edge<R, G, true, true, false, false, ONE, ONE && (PlanCta<R, G>::T >= 896)>(g, sc, env, rng, ctr, P.sp, ppx, ppy, ppth, ppt, pplen, P.w3, env.H,
                                                            nullptr, 0, o);
-#if AUV_PLAN_PREFETCH
-            if (ONE && BS && pick_mode == 0 && spec_parent >= 0 && g.gl < 2)
-                asm volatile("prefetch.global.L1 [%0];" ::"l"((const char *)&T.row()[spec_parent] + 32 * g.gl));
-#endif
+            if (POSE) {
+                // the copy is drained on every edge, safe or not: the next iteration's copy rewrites the slot
+                asm volatile("cp.async.wait_all;" ::: "memory");
+                g.sync();
+                prow = &gs.prow;
+                // single chunk: the leaf's length is scan + plen, the same add as inside the edge; no primitive: plen
+                const R plen = prow->len;
+                o.len = o.leaf_moved ? o.len + plen : plen;
+            }
             ctr = o.ctr;
             n_waypoints += o.nwp; n_prims += o.n_exp;
             if (P.trace && g.gl == 0) {
@@ -540,6 +540,7 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
                             }
                             SET_BIN_TAIL(bidx, tl);
                             T.pool()[tl * 32 + (c & 31)] = id;
+                            if (POSE) T.pose()[tl * 32 + (c & 31)] = make_float4((float)o.x, (float)o.y, (float)o.th, (float)o.t);
                             SET_BIN_COUNT(bidx, c + 1);
                         }
                     }

@@ -79,6 +79,7 @@ EXPORTS = [
     "auvrrt_astar_batch_dev", "auvrrt_edges_arc_cost_dev", "auvrrt_edges_arc_cost", "auvrrt_env_host_blob",
     "auvrrt_edges_dubins_cost_dev", "auvrrt_edges_dubins_cost", "auvrrt_occ_create", "auvrrt_occ_destroy", "auvrrt_occ_shape",
     "auvrrt_occ_grid_dev", "auvrrt_env_set_probs", "auvrrt_env_set_probs_dev", "auvrrt_env_get_probs",
+    "auvrrt_plan_group", "auvrrt_plan_best_dev", "auvrrt_materialize_dev",
 ]
 
 _lib = None
@@ -141,6 +142,10 @@ def lib():
                                         vp, vp, vp, C.POINTER(PlanTrace), vp]
     L.auvrrt_materialize.argtypes = [vp, _dp, _u64p, _u32p, _i32p, C.c_int64, C.POINTER(PlanParams), C.c_int,
                                      _dp, _i32p]
+    L.auvrrt_plan_group.argtypes = [C.POINTER(PlanParams), C.c_int64, C.c_int]
+    L.auvrrt_plan_best_dev.argtypes = [vp, C.c_int64, vp, C.c_int64, vp, vp, vp]
+    L.auvrrt_materialize_dev.argtypes = [vp, vp, vp, vp, vp, C.c_int64, vp, C.c_int64, C.POINTER(PlanParams), C.c_int,
+                                         vp, vp, vp]
     L.auvrrt_calibrate_fp32.argtypes = [C.c_int, C.c_int, _dp, _dp]
     _ip = C.POINTER(C.c_int)
     L.auvrrt_occupancy_dims.argtypes = [_dp, C.c_double, C.c_double, _dp, _i64p, C.c_int, _ip, _ip, _ip]

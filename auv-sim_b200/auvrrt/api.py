@@ -349,6 +349,16 @@ def materialize(env: Env, starts, seeds, chain, depth, params: PlanParams, preci
     return path, n_path
 
 
+def plan_group(params: PlanParams, Q, with_path=False):
+    """The planner auvrrt_plan_batch(_dev) runs for a batch of Q queries: 32, 16 or 8 lanes per tree, or 1 (one thread
+    per tree).  with_path: the batch writes paths (an out_path with path_cap > 0).  This is the group
+    materialize / device.materialize_dev need to re-create that batch's plans.  Host logic only."""
+    g = lib().auvrrt_plan_group(C.byref(params), int(Q), int(bool(with_path)))
+    if g < 0:
+        raise _lib.AuvrrtError("libauvrrt: %s" % lib().auvrrt_last_error().decode())
+    return g
+
+
 def calibrate_fp32(device=0, iters=4096):
     f, ms = C.c_double(0), C.c_double(0)
     check(lib().auvrrt_calibrate_fp32(device, iters, C.byref(f), C.byref(ms)))

@@ -10,9 +10,11 @@ import ctypes as C
 import numpy as np
 import torch
 
+import copy
+
 from . import _lib
 from ._lib import F32, F64, PlanRecord, check, lib
-from .api import RECORD_DTYPE, Env, _f64, _p, _prec, flat_polys
+from .api import RECORD_DTYPE, Env, _f64, _p, _prec, flat_polys, plan_group
 
 
 def _rdtype(precision):
@@ -30,7 +32,8 @@ def _vp(t):
 
 class DevicePlanner:
     """Batched RRT.exploring with everything resident in HBM: starts/seeds in, 96-byte records
-    (+ chains of stream positions) out.  One instance owns the tree workspace."""
+    (+ chains of stream positions) out.  One instance owns the tree workspace.  `group` is the planner the last
+    launch ran (api.plan_group), the evaluator best_paths re-creates its paths with."""
 
     def __init__(self, env: Env, params, precision="f32", max_queries=4096, want_chain=True, want_path=False):
         self.env, self.params, self.prec = env, params, _prec(precision)
@@ -48,6 +51,7 @@ class DevicePlanner:
         self.chain = torch.zeros((self.Q, ccap), dtype=torch.int32, device=self.dev) if (want_chain or want_path) else None
         self.path = (torch.zeros((self.Q, params.path_cap, 6), dtype=self.rdtype, device=self.dev)
                      if want_path and params.path_cap > 0 else None)
+        self.group = None
 
     def set_queries(self, starts: np.ndarray, seeds: np.ndarray):
         q = len(seeds)
@@ -58,13 +62,93 @@ class DevicePlanner:
 
     def launch(self, stream=None):
         """enqueue one pass over the current queries on `stream`; no synchronisation"""
+        group = plan_group(self.params, self.n, self.path is not None)
         check(lib().auvrrt_plan_batch_dev(self.env.handle, _vp(self.starts), _vp(self.seeds), self.n,
                                           C.byref(self.params), self.prec, _vp(self.workspace),
                                           self.workspace.numel(), _vp(self.records), _vp(self.chain),
                                           _vp(self.path), None, _stream_ptr(stream)))
+        self.group = group
+
+    def best_paths(self, mission_off, path_cap, stream=None):
+        """Each mission's best plan of the last launch and its path, enqueued on `stream` (default: the current stream)
+        without synchronising.  mission_off int64 [M + 1] on the device: mission m is queries
+        [mission_off[m], mission_off[m + 1]) (plan_best_dev).  Returns dict(best int64 [M] (query index or -1),
+        cost float64 [M] (cost[0] or +inf), path [M, path_cap, 6] in the precision's float type, n_path int32 [M])
+        as device tensors: row m of path re-creates plan best[m] (materialize_dev)."""
+        if self.group is None:
+            raise ValueError("best_paths: nothing launched yet")
+        if self.chain is None:
+            raise ValueError("best_paths: the planner was created without chains (want_chain=False)")
+        n = self.n
+        with torch.cuda.stream(stream if stream is not None else torch.cuda.current_stream(self.dev)):
+            best, cost = plan_best_dev(self.records[:n], mission_off, stream=stream)
+            pp = copy.copy(self.params)
+            pp.group = self.group
+            path, n_path = materialize_dev(self.env, self.starts[:n], self.seeds[:n], self.records[:n], self.chain[:n],
+                                           best, pp, self.prec, path_cap, stream=stream)
+        return {"best": best, "cost": cost, "path": path, "n_path": n_path}
 
     def records_numpy(self):
         return self.records[:self.n].cpu().numpy().view(RECORD_DTYPE).reshape(-1)
+
+
+def plan_best_dev(records, mission_off, out_best=None, out_cost=None, stream=None):
+    """Each mission's best plan (RRT.exploring with replicas: the least cost[0] of the records with status OK, depth
+    >= 0 and a cost that is not NaN; the lowest index on ties, -0.0 == +0.0), enqueued on `stream` (default: the
+    current stream) without synchronising or allocating in the library.  records uint8 [Q, 96] (plan records) and
+    mission_off int64 [M + 1] on one device; mission m is records [mission_off[m], mission_off[m + 1]), offsets
+    clamped into [0, Q].  out_best int64 [M] and out_cost float64 [M], allocated when None.
+    Returns (out_best: global record index or -1, out_cost: its cost[0] or +inf)."""
+    dev = records.device if isinstance(records, torch.Tensor) else None
+    Q = records.shape[0] if isinstance(records, torch.Tensor) and records.dim() == 2 else -1
+    _need("records", records, (torch.uint8,), (Q, C.sizeof(PlanRecord)), dev)
+    M = mission_off.shape[0] - 1 if isinstance(mission_off, torch.Tensor) and mission_off.dim() == 1 else -2
+    _need("mission_off", mission_off, (torch.int64,), (M + 1,), dev)
+    if out_best is None:
+        out_best = torch.empty(max(M, 0), dtype=torch.int64, device=dev)
+    if out_cost is None:
+        out_cost = torch.empty(max(M, 0), dtype=torch.float64, device=dev)
+    _need("out_best", out_best, (torch.int64,), (max(M, 0),), dev)
+    _need("out_cost", out_cost, (torch.float64,), (max(M, 0),), dev)
+    check(lib().auvrrt_plan_best_dev(_vp(records), Q, _vp(mission_off), M, _vp(out_best), _vp(out_cost),
+                                     _stream_on(dev, stream)))
+    return out_best, out_cost
+
+
+def materialize_dev(env: Env, starts, seeds, records, chain, pick, params, precision, path_cap, out=None, out_n=None,
+                    stream=None):
+    """api.materialize on device tensors through a pick list, enqueued on `stream` (default: the current stream)
+    without synchronising: row m of the output re-creates plan pick[m] of one plan_batch_dev launch of Q queries, with
+    the depth of its record.  starts [Q, 5] in the precision's float type, seeds int64 / uint64 [Q], records uint8
+    [Q, 96], chain int32 / uint32 [Q, chain_cap], pick int64 [M]; params.group must name the planner that ran
+    (api.plan_group of that launch; 0 is refused); params.path_cap is replaced by path_cap.
+    out [M, path_cap, 6] in the precision's float type and out_n int32 [M], allocated when None.  n_path is the full
+    row count (only path_cap rows are written); pick -1 gives 0, another pick outside [0, Q) or a depth outside
+    [0, chain_cap] gives -1, and no row.  Returns (out, out_n)."""
+    dev = torch.device("cuda", env.device)
+    prec = _prec(precision)
+    rdt = _rdtype(prec)
+    Q = starts.shape[0] if isinstance(starts, torch.Tensor) and starts.dim() == 2 else -1
+    _need("starts", starts, (rdt,), (Q, 5), dev)
+    _need("seeds", seeds, (torch.int64, torch.uint64), (Q,), dev)
+    _need("records", records, (torch.uint8,), (Q, C.sizeof(PlanRecord)), dev)
+    _need("chain", chain, (torch.int32, torch.uint32), (Q, max(params.chain_cap, 1)), dev)
+    M = pick.shape[0] if isinstance(pick, torch.Tensor) and pick.dim() == 1 else -1
+    _need("pick", pick, (torch.int64,), (M,), dev)
+    path_cap = int(path_cap)
+    if path_cap < 1:
+        raise ValueError("path_cap must be >= 1, got %d" % path_cap)
+    if out is None:
+        out = torch.empty((M, path_cap, 6), dtype=rdt, device=dev)
+    if out_n is None:
+        out_n = torch.empty(M, dtype=torch.int32, device=dev)
+    _need("out", out, (rdt,), (M, path_cap, 6), dev)
+    _need("out_n", out_n, (torch.int32,), (M,), dev)
+    pp = copy.copy(params)
+    pp.path_cap = path_cap
+    check(lib().auvrrt_materialize_dev(env.handle, _vp(starts), _vp(seeds), _vp(records), _vp(chain), Q, _vp(pick), M,
+                                       C.byref(pp), prec, _vp(out), _vp(out_n), _stream_on(dev, stream)))
+    return out, out_n
 
 
 def nn_dev(tree_x, tree_y, qx, qy, out_idx, scratch, precision, stream=None):

@@ -166,10 +166,8 @@ def plan_sharded_device(env, starts, seeds, params, precision="f32", want_path=T
             import copy
             pp = copy.copy(params)
             pp.path_cap = 34 * (int(rec["depth"][0]) + 1)
-            # re-create the path with the evaluator of the kernel that planned it (group 0: one thread per tree from
-            # 32768 queries on, no paths being written)
-            if pp.group == 0 and hi - lo >= 32768 and pp.mode != 3 and planner.path is None:
-                pp.group = 1
+            # re-create the path with the evaluator of the kernel that planned it
+            pp.group = api.plan_group(params, hi - lo, planner.path is not None)
             chain = planner.chain[j:j + 1].cpu().numpy().view(np.uint32)
             rows, n_path = api.materialize(env, starts[best:best + 1], seeds[best:best + 1], chain, rec["depth"], pp, precision)
             rows_dev = torch.from_numpy(np.ascontiguousarray(rows[0, :n_path[0]])).to(dev)

@@ -939,7 +939,7 @@ static int materialize_host(const auvrrt_env *env, const double *starts, const u
     R *dpath = st.out_real<R>(path, 6 * Q * p->path_cap, true);
     int32_t *dn = st.out(n_path, Q);
     AUV_TRY(st.rc);
-    AUV_TRY(launch_materialize<R>(env, ds, dseed, dchain, ddepth, Q, p, dpath, dn, 0));
+    AUV_TRY(launch_materialize<R>(env, ds, dseed, dchain, ddepth, 1, Q, nullptr, Q, p, dpath, dn, 0));
     return st.finish();
 }
 extern "C" int auvrrt_materialize(const auvrrt_env_t *env, const double *starts, const uint64_t *seeds,
@@ -960,6 +960,47 @@ extern "C" int auvrrt_materialize(const auvrrt_env_t *env, const double *starts,
             return set_err(AUVRRT_ERR_ARG, "materialize: depth[%lld] = %d outside [0, chain_cap = %d]", (long long)q, depth[q],
                            params->chain_cap);
     return AUV_DISPATCH(precision, materialize_host, env, starts, seeds, chain, depth, Q, params, out_path, out_n_path);
+}
+
+// ------------------------------------------------------------------ the device end of a planning step
+extern "C" int auvrrt_plan_group(const auvrrt_plan_params_t *p, int64_t Q, int with_path) {
+    if (!p) { set_err(AUVRRT_ERR_ARG, "plan_group: params is NULL"); return -1; }
+    const int G = plan_group(p, Q, with_path != 0);
+    return G < 0 ? -1 : G;
+}
+static int need_a_device() {
+    if (auvrrt_device_count() <= 0) return set_err(AUVRRT_ERR_CUDA, "no CUDA device: libauvrrt has no CPU fallback");
+    return AUVRRT_OK;
+}
+extern "C" int auvrrt_plan_best_dev(const auvrrt_plan_record_t *records, int64_t Q, const int64_t *mission_off, int64_t M,
+                                    int64_t *out_best, double *out_cost, void *stream) {
+    AUV_TRY(need_a_device());
+    if (M <= 0) return AUVRRT_OK;
+    if (!mission_off || !out_best || !out_cost || (Q > 0 && !records)) return set_err(AUVRRT_ERR_ARG, "plan_best: NULL buffer");
+    return launch_plan_best(records, Q, mission_off, M, out_best, out_cost, (cudaStream_t)stream);
+}
+extern "C" int auvrrt_materialize_dev(const auvrrt_env_t *env, const void *starts, const uint64_t *seeds,
+                                      const auvrrt_plan_record_t *records, const uint32_t *chain, int64_t Q,
+                                      const int64_t *pick, int64_t M, const auvrrt_plan_params_t *params, int precision,
+                                      void *out_path, int32_t *out_n_path, void *stream) {
+    AUV_TRY(need_a_device());
+    AUV_TRY(check_precision(precision));
+    if (!env || !params) return set_err(AUVRRT_ERR_ARG, "materialize_dev: NULL env or params");
+    // the evaluator must be the one of the planner that made the chains: group 0 would leave it to a guess
+    if (params->group != 32 && params->group != 16 && params->group != 8 && params->group != 1)
+        return set_err(AUVRRT_ERR_ARG, "materialize_dev: group must name the planner that ran: 32, 16, 8 or 1 (see auvrrt_plan_group)");
+    if (params->path_cap < 1) return set_err(AUVRRT_ERR_ARG, "materialize_dev: path_cap must be >= 1");
+    if (M <= 0) return AUVRRT_OK;
+    if (!pick || !out_path || !out_n_path || (Q > 0 && (!starts || !seeds || !records || !chain)))
+        return set_err(AUVRRT_ERR_ARG, "materialize_dev: NULL buffer");
+    const int32_t *depth = records ? &records->depth : nullptr;
+    const int stride = (int)(sizeof(auvrrt_plan_record_t) / sizeof(int32_t));
+    cudaStream_t s = (cudaStream_t)stream;
+    if (precision == AUVRRT_F32)
+        return launch_materialize<float>(env, (const float *)starts, seeds, chain, depth, stride, Q, pick, M, params,
+                                         (float *)out_path, out_n_path, s);
+    return launch_materialize<double>(env, (const double *)starts, seeds, chain, depth, stride, Q, pick, M, params,
+                                      (double *)out_path, out_n_path, s);
 }
 
 extern "C" int auvrrt_calibrate_fp32(int device, int iters, double *out_flops, double *out_ms) {

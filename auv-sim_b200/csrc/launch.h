@@ -107,9 +107,14 @@ int launch_plan(const auvrrt_env *env, const R *starts, const uint64_t *seeds, i
                 const auvrrt_plan_params_t *p, void *workspace, int64_t workspace_bytes,
                 auvrrt_plan_record_t *records, uint32_t *chain, R *path, const auvrrt_plan_trace_t *trace,
                 cudaStream_t s);
+// the group auvrrt_plan_batch(_dev) runs for Q queries (32, 16, 8 or 1), or -AUVRRT_ERR_* with the message set
+int plan_group(const auvrrt_plan_params_t *p, int64_t Q, bool with_path);
+// output row m re-creates plan pick[m] of Q (row q of Q = M plans when pick is NULL) with depth[q * depth_stride]
 template <typename R>
 int launch_materialize(const auvrrt_env *env, const R *starts, const uint64_t *seeds, const uint32_t *chain,
-                       const int32_t *depth, int64_t Q, const auvrrt_plan_params_t *p, R *path, int32_t *n_path,
-                       cudaStream_t s);
+                       const int32_t *depth, int depth_stride, int64_t Q, const int64_t *pick, int64_t M,
+                       const auvrrt_plan_params_t *p, R *path, int32_t *n_path, cudaStream_t s);
+int launch_plan_best(const auvrrt_plan_record_t *records, int64_t Q, const int64_t *off, int64_t M, int64_t *out_best,
+                     double *out_cost, cudaStream_t s);
 
 }  // namespace auv

@@ -18,6 +18,7 @@
 // `initial` the planner's bin filter (rrt_dubins.py:161-166) never changes a waypoint's first-match
 // bin (every waypoint time lies in [t_initial, t_leaf]).  Totals equal the reference's up to
 // summation order (fp64: <= 1e-12 relative).
+#include <limits.h>
 #include <stdlib.h>
 #include "plan_common.cuh"
 #include "dubins.cuh"
@@ -645,24 +646,35 @@ k_plan(const unsigned char *blob, int hot_bytes, int total_bytes, int stage_mode
 }
 
 // ---- re-create paths from (start, seed, chain of stream positions): no tree needed ------------
+// Output row m re-creates plan q = pick[m] (q = m without a pick list) of the Q plans; its depth is depth[q * depth_stride]
+// (the host entry's int32 array, or the depth field of 96-byte records).  pick[m] == -1 gives n_path 0; another pick
+// outside [0, Q), or a depth outside [0, chain_cap], gives n_path -1.  Neither writes a row.
+// 128 registers (it runs 128-thread CTAs): under ptxas' default register heuristic the fp32 warp variant spilled 20
+// bytes, and the pick indirection made the fp64 one spill.
 template <typename R, int G>
-__global__ void __launch_bounds__(128)
+__global__ void __maxnreg__(128)
 k_materialize(const unsigned char *blob, const R *starts, const uint64_t *seeds, const uint32_t *chain,
-              const int32_t *depth, long long Q, PlanP<R> P, R *path_out, int32_t *n_path_out) {
+              const int32_t *depth, int depth_stride, long long Q, const int64_t *pick, long long M, PlanP<R> P,
+              R *path_out, int32_t *n_path_out) {
     __shared__ GroupScratch<R, G, false> scratch[128 / G];
     EnvView<R> env;
     env.bind(blob, blob);
     env.bind_grid(blob, blob);
     Grp<G> g;
     GroupScratch<R, G, false> &sc = scratch[threadIdx.x / G];
-    const long long groups = (long long)gridDim.x * (128 / G);
-    for (long long q = blockIdx.x * (long long)(128 / G) + threadIdx.x / G; q < Q; q += groups) {
+    const int groups = gridDim.x * (128 / G);
+    for (int m = blockIdx.x * (128 / G) + threadIdx.x / G; m < M; m += groups) {      // (M, Q < 2^31: launch_materialize)
+        const long long pq = pick ? (long long)pick[m] : m;
+        if (pq < 0 || pq >= Q) { if (g.gl == 0) n_path_out[m] = pq == -1 ? 0 : -1; continue; }
+        const int q = (int)pq;
+        const int d = depth[(size_t)q * depth_stride];
+        if (d < 0 || d > P.chain_cap) { if (g.gl == 0) n_path_out[m] = -1; continue; }
         Stream<R> rng;
         rng.key = stream_key(seeds[q]); rng.ext = nullptr; rng.n_ext = 0;
         R x = starts[5 * q], y = starts[5 * q + 1], th = starts[5 * q + 2], t = starts[5 * q + 3], len = starts[5 * q + 4];
-        R *rows = path_out + (size_t)q * P.path_cap * 6;
+        const uint32_t *ch = chain + (size_t)q * P.chain_cap;
+        R *rows = path_out + (size_t)m * P.path_cap * 6;
         int n_path = 0;
-        const int d = depth[q];
         for (int e = 0; e < d; e++) {
             if (g.gl == 0 && n_path < P.path_cap) {
                 R *w = rows + 6 * (size_t)n_path;
@@ -672,7 +684,7 @@ k_materialize(const unsigned char *blob, const R *starts, const uint64_t *seeds,
             int room = P.path_cap - n_path; if (room < 0) room = 0;
             if (P.mode == 3) {                      // every lane re-creates the same Dubins edge; lane 0 writes its rows
                 R smx, smy, smth;
-                dubins_sample_at<R>(env, rng, chain[(size_t)q * P.chain_cap + e], smx, smy, smth);
+                dubins_sample_at<R>(env, rng, ch[e], smx, smy, smth);
                 DubinsEdge<R> de;
                 dubins_edge_eval<R>(env, P, x, y, th, t, len, smx, smy, smth, false,
                                     g.gl == 0 ? rows + 6 * (size_t)(n_path < P.path_cap ? n_path : 0) : nullptr, room, de);
@@ -681,20 +693,18 @@ k_materialize(const unsigned char *blob, const R *starts, const uint64_t *seeds,
                 continue;
             }
             EdgeOut<R> o;
-            eval_edge<R, G, false, false, true>(g, sc, env, rng, chain[(size_t)q * P.chain_cap + e], P.sp, x, y, th, t,
+            eval_edge<R, G, false, false, true>(g, sc, env, rng, ch[e], P.sp, x, y, th, t,
                                                 len, (R)0, 0, rows + 6 * (size_t)(n_path < P.path_cap ? n_path : 0),
                                                 room, o);
             n_path += o.nwp - 1;
             x = o.x; y = o.y; th = o.th; t = o.t; len = o.len;
         }
-        if (d >= 0) {
-            if (g.gl == 0 && n_path < P.path_cap) {
-                R *w = rows + 6 * (size_t)n_path;
-                w[0] = x; w[1] = y; w[2] = th; w[3] = (P.mode == 3 && d > 0) ? P.vel : (R)0; w[4] = t; w[5] = len;
-            }
-            n_path++;
+        if (g.gl == 0 && n_path < P.path_cap) {
+            R *w = rows + 6 * (size_t)n_path;
+            w[0] = x; w[1] = y; w[2] = th; w[3] = (P.mode == 3 && d > 0) ? P.vel : (R)0; w[4] = t; w[5] = len;
         }
-        if (g.gl == 0) n_path_out[q] = n_path;
+        n_path++;
+        if (g.gl == 0) n_path_out[m] = n_path;
     }
 }
 
@@ -800,16 +810,15 @@ int launch_plan(const auvrrt_env *env, const R *starts, const uint64_t *seeds, i
                 cudaStream_t s) {
     // group 0 = automatic: a warp per tree shortens the latency of a few thousand queries; from
     // ~3x10^4 queries on, the queries themselves fill the machine and one thread per tree wins
-    int G = p->group ? p->group : ((Q >= 32768 && !(path && p->path_cap > 0) && p->mode != 3) ? 1 : 32);
-    if (G == 1 && p->mode == 3) return set_err(AUVRRT_ERR_UNSUPPORTED, "plan: mode 3 evaluates one candidate parent per lane; group must be 32, 16 or 8");
+    const int G = plan_group(p, Q, path && p->path_cap > 0);
+    if (G < 0) return -G;
     if (G == 1) {
         if (path && p->path_cap > 0) return set_err(AUVRRT_ERR_UNSUPPORTED, "plan: group 1 (thread per tree) writes no paths; use auvrrt_materialize");
         return launch_plan_tpt<R>(env, starts, seeds, Q, p, workspace, workspace_bytes, records, chain, trace, s, nullptr);
     }
     if (G == 32) return launch_plan_g<R, 32>(env, starts, seeds, Q, p, workspace, workspace_bytes, records, chain, path, trace, s, nullptr);
     if (G == 16) return launch_plan_g<R, 16>(env, starts, seeds, Q, p, workspace, workspace_bytes, records, chain, path, trace, s, nullptr);
-    if (G == 8) return launch_plan_g<R, 8>(env, starts, seeds, Q, p, workspace, workspace_bytes, records, chain, path, trace, s, nullptr);
-    return set_err(AUVRRT_ERR_ARG, "plan: group must be 32, 16, 8 or 1");
+    return launch_plan_g<R, 8>(env, starts, seeds, Q, p, workspace, workspace_bytes, records, chain, path, trace, s, nullptr);
 }
 // Q <= 0: a batch of any size.  Group 0 lets launch_plan pick the kernel per batch (by its size and whether paths are
 // written), so the workspace must hold the largest one it can pick for a batch of at most Q queries.
@@ -817,14 +826,14 @@ template <typename R>
 int64_t plan_workspace_bytes(const auvrrt_env *env, const auvrrt_plan_params_t *p, int64_t Q) {
     int64_t need = -1;
     int rc;
-    const int G = p->group ? p->group : 32;
+    const int G = p->group ? p->group : plan_group(p, Q, true);     // the warp planner every group-0 batch may run
     if (G == 1) rc = launch_plan_tpt<R>(env, nullptr, nullptr, Q, p, nullptr, 0, nullptr, nullptr, nullptr, 0, &need);
     else if (G == 32) rc = launch_plan_g<R, 32>(env, nullptr, nullptr, 0, p, nullptr, 0, nullptr, nullptr, nullptr, nullptr, 0, &need);
     else if (G == 16) rc = launch_plan_g<R, 16>(env, nullptr, nullptr, 0, p, nullptr, 0, nullptr, nullptr, nullptr, nullptr, 0, &need);
     else if (G == 8) rc = launch_plan_g<R, 8>(env, nullptr, nullptr, 0, p, nullptr, 0, nullptr, nullptr, nullptr, nullptr, 0, &need);
     else { set_err(AUVRRT_ERR_ARG, "plan: group must be 32, 16, 8 or 1"); return -1; }
     if (rc) return -1;
-    if (p->group == 0 && p->mode != 3 && (Q <= 0 || Q >= 32768)) {
+    if (p->group == 0 && plan_group(p, Q > 0 ? Q : INT64_MAX, false) == 1) {
         int64_t tpt = -1;
         if (launch_plan_tpt<R>(env, nullptr, nullptr, Q, p, nullptr, 0, nullptr, nullptr, nullptr, 0, &tpt)) return -1;
         if (tpt > need) need = tpt;
@@ -840,9 +849,10 @@ template int64_t plan_workspace_bytes<double>(const auvrrt_env *, const auvrrt_p
 
 template <typename R>
 int launch_materialize(const auvrrt_env *env, const R *starts, const uint64_t *seeds, const uint32_t *chain,
-                       const int32_t *depth, int64_t Q, const auvrrt_plan_params_t *p, R *path, int32_t *n_path,
-                       cudaStream_t s) {
-    if (Q <= 0) return AUVRRT_OK;
+                       const int32_t *depth, int depth_stride, int64_t Q, const int64_t *pick, int64_t M,
+                       const auvrrt_plan_params_t *p, R *path, int32_t *n_path, cudaStream_t s) {
+    if (M <= 0) return AUVRRT_OK;
+    if (M > INT_MAX || Q > INT_MAX) return set_err(AUVRRT_ERR_ARG, "materialize: more than 2^31 - 1 plans or output rows");
     PlanP<R> P;
     int rc = make_planp<R>(env, p, &P);
     if (rc) return rc;
@@ -850,21 +860,159 @@ int launch_materialize(const auvrrt_env *env, const R *starts, const uint64_t *s
     const int G = p->group ? p->group : 32;
     if (G == 1) {
         if (p->mode == 3) return set_err(AUVRRT_ERR_UNSUPPORTED, "materialize: mode 3 has no thread-per-tree plans");
-        return launch_materialize_tpt<R>(env, starts, seeds, chain, depth, Q, P, path, n_path, s);
+        return launch_materialize_tpt<R>(env, starts, seeds, chain, depth, depth_stride, Q, pick, M, P, path, n_path, s);
     }
-    int64_t blocks = (Q * G + 127) / 128;
+    int64_t blocks = (M * G + 127) / 128;
     if (blocks > AUV_SMS * 8) blocks = AUV_SMS * 8;
     const unsigned char *blob = env_blob<R>(env).blob;
-    if (G == 32) k_materialize<R, 32><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
-    else if (G == 16) k_materialize<R, 16><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
-    else if (G == 8) k_materialize<R, 8><<<(unsigned)blocks, 128, 0, s>>>(blob, starts, seeds, chain, depth, (long long)Q, P, path, n_path);
+#define AUV_MAT_ARGS blob, starts, seeds, chain, depth, depth_stride, (long long)Q, pick, (long long)M, P, path, n_path
+    if (G == 32) k_materialize<R, 32><<<(unsigned)blocks, 128, 0, s>>>(AUV_MAT_ARGS);
+    else if (G == 16) k_materialize<R, 16><<<(unsigned)blocks, 128, 0, s>>>(AUV_MAT_ARGS);
+    else if (G == 8) k_materialize<R, 8><<<(unsigned)blocks, 128, 0, s>>>(AUV_MAT_ARGS);
     else return set_err(AUVRRT_ERR_ARG, "materialize: group must be 32, 16, 8 or 1");
+#undef AUV_MAT_ARGS
     AUV_LAUNCH_CHECK();
     return AUVRRT_OK;
 }
-template int launch_materialize<float>(const auvrrt_env *, const float *, const uint64_t *, const uint32_t *, const int32_t *,
-                                       int64_t, const auvrrt_plan_params_t *, float *, int32_t *, cudaStream_t);
-template int launch_materialize<double>(const auvrrt_env *, const double *, const uint64_t *, const uint32_t *, const int32_t *,
-                                        int64_t, const auvrrt_plan_params_t *, double *, int32_t *, cudaStream_t);
+template int launch_materialize<float>(const auvrrt_env *, const float *, const uint64_t *, const uint32_t *, const int32_t *, int,
+                                       int64_t, const int64_t *, int64_t, const auvrrt_plan_params_t *, float *, int32_t *,
+                                       cudaStream_t);
+template int launch_materialize<double>(const auvrrt_env *, const double *, const uint64_t *, const uint32_t *, const int32_t *, int,
+                                        int64_t, const int64_t *, int64_t, const auvrrt_plan_params_t *, double *, int32_t *,
+                                        cudaStream_t);
+
+// ---- each mission's best plan ------------------------------------------------------------------------------------
+// Mission m is records [lo, hi), lo = clamp(off[m], 0, Q), hi = clamp(off[m + 1], lo, Q).  A record is eligible when its
+// status is OK, its depth is >= 0 and cost[0] is not NaN; among those the least cost[0] wins, the lowest index on ties
+// (the reference's strict `<` over the records in order), with -0.0 equal to +0.0.  Only the first two 32-byte sectors
+// of a record are read: status and depth, then cost[0].
+static constexpr unsigned long long BEST_NONE = ~0ull;
+
+__device__ __forceinline__ unsigned long long best_key(const auvrrt_plan_record_t *records, long long i) {
+    const auvrrt_plan_record_t *r = records + i;
+    const int status = __ldg(&r->status), depth = __ldg(&r->depth);
+    double c = __ldg(&r->cost[0]);
+    if (status != AUVRRT_ST_OK || depth < 0 || c != c) return BEST_NONE;
+    if (c == 0.0) c = 0.0;                                   // -0.0 -> +0.0
+    const unsigned long long b = (unsigned long long)__double_as_longlong(c);
+    return (b >> 63) ? ~b : (b | (1ull << 63));             // unsigned order == float order; +inf < BEST_NONE
+}
+
+__device__ __forceinline__ void mission_range(const int64_t *off, long long m, long long Q, long long &lo, long long &hi) {
+    lo = min(max((long long)off[m], 0ll), Q);
+    hi = min(max((long long)off[m + 1], lo), Q);
+}
+
+__device__ __forceinline__ void warp_min(unsigned long long &key, long long &idx) {
+    for (int o = 16; o > 0; o >>= 1) {
+        const unsigned long long k2 = __shfl_xor_sync(0xffffffffu, key, o);
+        const long long i2 = __shfl_xor_sync(0xffffffffu, idx, o);
+        if (k2 < key || (k2 == key && i2 < idx)) { key = k2; idx = i2; }
+    }
+}
+
+// many small missions: one warp per mission, every lane keeps the first minimum of its strided records
+__global__ void __launch_bounds__(256)
+k_best_warp(const auvrrt_plan_record_t *records, long long Q, const int64_t *off, long long M, int64_t *out_best,
+            double *out_cost) {
+    const int lane = threadIdx.x & 31;
+    const long long warps = (long long)gridDim.x * (blockDim.x / 32);
+    for (long long m = (blockIdx.x * (long long)blockDim.x + threadIdx.x) / 32; m < M; m += warps) {
+        long long lo, hi;
+        mission_range(off, m, Q, lo, hi);
+        unsigned long long key = BEST_NONE;
+        long long idx = LLONG_MAX;
+        for (long long i = lo + lane; i < hi; i += 32) {
+            const unsigned long long k = best_key(records, i);
+            if (k < key) { key = k; idx = i; }
+        }
+        warp_min(key, idx);
+        if (lane == 0) {
+            out_best[m] = key == BEST_NONE ? -1 : idx;
+            out_cost[m] = key == BEST_NONE ? (double)INFINITY : records[idx].cost[0];
+        }
+    }
+}
+
+// few large missions: `slices` CTAs per mission; pass 1 takes the least key of the mission with atomicMin into out_cost
+// (as an unsigned key, preset to BEST_NONE), pass 2 the lowest index holding it into out_best (as unsigned, preset to
+// ~0 = -1), then k_best_finish turns the key back into the winner's cost[0].
+template <bool INDEX>
+__global__ void __launch_bounds__(256)
+k_best_split(const auvrrt_plan_record_t *records, long long Q, const int64_t *off, long long M, int slices,
+             int64_t *out_best, double *out_cost) {
+    __shared__ unsigned long long s_key[8];
+    __shared__ long long s_idx[8];
+    unsigned long long *gkey = (unsigned long long *)out_cost;
+    for (long long w = blockIdx.x; w < M * slices; w += gridDim.x) {
+        const long long m = w / slices, s = w % slices;
+        long long lo, hi;
+        mission_range(off, m, Q, lo, hi);
+        const long long a = lo + (hi - lo) * s / slices, b = lo + (hi - lo) * (s + 1) / slices;
+        const unsigned long long want = INDEX ? gkey[m] : 0ull;
+        unsigned long long key = BEST_NONE;
+        long long idx = LLONG_MAX;
+        if (!INDEX || want != BEST_NONE)
+            for (long long i = a + threadIdx.x; i < b; i += blockDim.x) {
+                const unsigned long long k = best_key(records, i);
+                if (INDEX ? k == want && i < idx : k < key) { key = k; idx = i; }
+            }
+        warp_min(key, idx);
+        if ((threadIdx.x & 31) == 0) { s_key[threadIdx.x >> 5] = key; s_idx[threadIdx.x >> 5] = idx; }
+        __syncthreads();
+        if (threadIdx.x < 32) {
+            key = threadIdx.x < blockDim.x / 32 ? s_key[threadIdx.x] : BEST_NONE;
+            idx = threadIdx.x < blockDim.x / 32 ? s_idx[threadIdx.x] : LLONG_MAX;
+            warp_min(key, idx);
+            if (threadIdx.x == 0 && key != BEST_NONE) {
+                if (INDEX) atomicMin((unsigned long long *)&out_best[m], (unsigned long long)idx);
+                else atomicMin(&gkey[m], key);
+            }
+        }
+        __syncthreads();
+    }
+}
+
+__global__ void k_best_finish(const auvrrt_plan_record_t *records, long long M, const int64_t *best, double *out_cost) {
+    for (long long m = blockIdx.x * (long long)blockDim.x + threadIdx.x; m < M; m += (long long)gridDim.x * blockDim.x)
+        out_cost[m] = best[m] < 0 ? (double)INFINITY : records[best[m]].cost[0];
+}
+
+int launch_plan_best(const auvrrt_plan_record_t *records, int64_t Q, const int64_t *off, int64_t M, int64_t *out_best,
+                     double *out_cost, cudaStream_t s) {
+    if (M <= 0) return AUVRRT_OK;
+    // a warp per mission while the average mission fits a few passes of one warp (4096 x 64, 4096 x 256); past that the
+    // records of each mission are split over CTAs of 4096 records (one mission of 2^20 records: 256 CTAs)
+    const int64_t per_cta = 4096;
+    const int64_t slices = Q > 0 ? (Q + M * per_cta - 1) / (M * per_cta) : 1;
+    if (slices <= 1) {
+        int64_t blocks = (M + 7) / 8;
+        if (blocks > AUV_SMS * 16) blocks = AUV_SMS * 16;
+        k_best_warp<<<(unsigned)blocks, 256, 0, s>>>(records, (long long)Q, off, (long long)M, out_best, out_cost);
+        AUV_LAUNCH_CHECK();
+        return AUVRRT_OK;
+    }
+    AUV_CUDA(cudaMemsetAsync(out_cost, 0xFF, 8 * (size_t)M, s));
+    AUV_CUDA(cudaMemsetAsync(out_best, 0xFF, 8 * (size_t)M, s));
+    int64_t blocks = M * slices;
+    if (blocks > AUV_SMS * 8) blocks = AUV_SMS * 8;
+    k_best_split<false><<<(unsigned)blocks, 256, 0, s>>>(records, (long long)Q, off, (long long)M, (int)slices, out_best, out_cost);
+    AUV_LAUNCH_CHECK();
+    k_best_split<true><<<(unsigned)blocks, 256, 0, s>>>(records, (long long)Q, off, (long long)M, (int)slices, out_best, out_cost);
+    AUV_LAUNCH_CHECK();
+    k_best_finish<<<(unsigned)((M + 255) / 256 < AUV_SMS * 8 ? (M + 255) / 256 : AUV_SMS * 8), 256, 0, s>>>(records, (long long)M, out_best, out_cost);
+    AUV_LAUNCH_CHECK();
+    return AUVRRT_OK;
+}
+
+// The planner a batch of Q queries runs: an explicit group passes through; group 0 is one thread per tree from 32768
+// queries on when no paths are written (mode != 3), else a warp per tree.  -AUVRRT_ERR_* (message set) when invalid.
+int plan_group(const auvrrt_plan_params_t *p, int64_t Q, bool with_path) {
+    const int G = p->group ? p->group : ((Q >= 32768 && !with_path && p->mode != 3) ? 1 : 32);
+    if (G == 1 && p->mode == 3)
+        return -set_err(AUVRRT_ERR_UNSUPPORTED, "plan: mode 3 evaluates one candidate parent per lane; group must be 32, 16 or 8");
+    if (G != 32 && G != 16 && G != 8 && G != 1) return -set_err(AUVRRT_ERR_ARG, "plan: group must be 32, 16, 8 or 1");
+    return G;
+}
 
 }  // namespace auv

@@ -99,6 +99,7 @@ int launch_plan_tpt(const auvrrt_env *env, const R *starts, const uint64_t *seed
 // paths of its plans, re-created with its own edge evaluator
 template <typename R>
 int launch_materialize_tpt(const auvrrt_env *env, const R *starts, const uint64_t *seeds, const uint32_t *chain,
-                           const int32_t *depth, int64_t Q, const PlanP<R> &P, R *path, int32_t *n_path, cudaStream_t s);
+                           const int32_t *depth, int depth_stride, int64_t Q, const int64_t *pick, int64_t M,
+                           const PlanP<R> &P, R *path, int32_t *n_path, cudaStream_t s);
 
 }  // namespace auv

@@ -269,6 +269,41 @@ int auvrrt_materialize(const auvrrt_env_t *env, const double *starts, const uint
                        const auvrrt_plan_params_t *params, int precision, double *out_path,
                        int32_t *out_n_path);
 
+/* ---- the device end of a planning step: each mission's best plan and its path, all in HBM ------
+ * auvrrt_plan_group: the group auvrrt_plan_batch(_dev) runs for a batch of Q queries -- 32, 16, 8 or
+ * 1 -- where with_path says whether paths are written (out_path != NULL and path_cap > 0).  An
+ * explicit group passes through; group 0 is 1 for Q >= 32768 without paths and mode != 3, else 32.
+ * -1 (message set) for a bad group or mode 3 with group 1.  Host logic only: needs no device.  It is
+ * the group auvrrt_materialize(_dev) needs to re-create the plans of that batch. */
+int auvrrt_plan_group(const auvrrt_plan_params_t *params, int64_t Q, int with_path);
+/* Each mission's best plan (RRT.exploring with replicas, rrt_dubins.py:169).  Device buffers: records
+ * [Q], mission_off int64 [M + 1]; mission m is records [lo, hi) with lo = clamp(mission_off[m], 0, Q),
+ * hi = clamp(mission_off[m + 1], lo, Q), so no offset reads out of bounds.  A record is eligible when
+ * status == AUVRRT_ST_OK, depth >= 0 and cost[0] is not NaN (a plan made with a chain buffer and
+ * deeper than chain_cap is OVERFLOW, not OK).  Among them the least cost[0] wins as floats compare
+ * (-0.0 == +0.0), the lowest index on ties -- the reference's strict `<`.  out_best int64 [M]: the
+ * global index of the winner, -1 if the mission has none; out_cost double [M]: its cost[0], +inf if
+ * none.  Asynchronous on `stream`: no allocation, no synchronisation (it can be captured in a CUDA
+ * graph).  Reads the first 64 bytes of each record (status, depth, cost[0]).  One kernel while
+ * missions average at most 4096 records; past that 2 memsets and 3 kernels, each mission's records
+ * split over CTAs. */
+int auvrrt_plan_best_dev(const auvrrt_plan_record_t *records, int64_t Q, const int64_t *mission_off,
+                         int64_t M, int64_t *out_best, double *out_cost, void *stream);
+/* auvrrt_materialize on device buffers, through a pick list: output row m re-creates plan pick[m]
+ * of the Q plans (starts [Q][5] in the precision's type, seeds [Q], records [Q], chain
+ * [Q][chain_cap] of one auvrrt_plan_batch_dev call), with the depth of its record.  out_path
+ * [M][path_cap][6] in the precision's type, out_n_path int32 [M] with the full row count (only the
+ * first path_cap rows are written).  pick[m] == -1 (a mission without a plan) gives n_path 0; any
+ * other pick outside [0, Q), or a depth outside [0, chain_cap] (e.g. an OVERFLOW record), gives
+ * n_path -1; neither writes a row.  params->group must name the planner that made the chains: 32,
+ * 16, 8 or 1 (auvrrt_plan_group of that batch); group 0 is AUVRRT_ERR_ARG.  Every argument error is
+ * returned before anything is enqueued.  Rows equal auvrrt_materialize's for the same plans bit for
+ * bit.  Asynchronous on `stream`, no allocation. */
+int auvrrt_materialize_dev(const auvrrt_env_t *env, const void *starts, const uint64_t *seeds,
+                           const auvrrt_plan_record_t *records, const uint32_t *chain, int64_t Q,
+                           const int64_t *pick, int64_t M, const auvrrt_plan_params_t *params,
+                           int precision, void *out_path, int32_t *out_n_path, void *stream);
+
 /* ---- SharkOccupancyGrid.convert (sharkOccupancyGrid.py:47-71): shark tracks -> AUV-detection grids
  * SURVEY.md section 8(f) row N2, the producer of the cost function's probs[T][C] input.
  * cells: C polygons in cell_list order (vertices cell_xy[cell_off[c] .. cell_off[c+1]));

@@ -219,7 +219,9 @@ def cost(env: Env, paths_xyt, t_total, weights, bin_mask=None, n_habitats=-1, pr
     tt = _f64(t_total, (-1,))
     w = _f64(weights, (3,))
     out = np.zeros((len(paths_xyt), 4))
-    mask = None if bin_mask is None else np.ascontiguousarray(np.asarray(bin_mask, dtype=np.uint8))
+    mask = None if bin_mask is None else np.ascontiguousarray(np.asarray(bin_mask, dtype=np.uint8)).reshape(-1)
+    if mask is not None and len(mask) < len(env.bins):       # the library reads one byte per time bin
+        raise ValueError("bin_mask needs one entry per time bin (%d), got %d" % (len(env.bins), len(mask)))
     check(lib().auvrrt_cost(env.handle, _p(flat), _p(off, C.c_int64), len(paths_xyt), _p(tt), _p(w),
                             _p(mask, C.c_uint8) if mask is not None else None, int(n_habitats),
                             _prec(precision), _p(out)))
@@ -228,7 +230,9 @@ def cost(env: Env, paths_xyt, t_total, weights, bin_mask=None, n_habitats=-1, pr
 
 def cost_point(env: Env, points_xy, visited, tb, weights, precision="f64"):
     pts = _f64(points_xy, (-1, 2))
-    vis = np.ascontiguousarray(np.asarray(visited, dtype=np.uint8))
+    vis = np.ascontiguousarray(np.asarray(visited, dtype=np.uint8)).reshape(-1)
+    if len(vis) < len(env.habitats):                         # the library reads one byte per habitat
+        raise ValueError("visited needs one entry per habitat (%d), got %d" % (len(env.habitats), len(vis)))
     w = _f64(weights, (3,))
     out = np.zeros(len(pts))
     check(lib().auvrrt_cost_point(env.handle, _p(pts), len(pts), _p(vis, C.c_uint8), int(tb), _p(w),

@@ -247,10 +247,11 @@ __device__ __forceinline__ int find_cell_rare(const EnvView<R> &env, int lo, R x
 template <typename R, bool HAS_XB = false>
 __device__ __forceinline__ int find_cell(const EnvView<R> &env, R x, R y) {
     if (!HAS_XB && env.nxb == 0) return env.NB == 0 ? -1 : find_cell_walk<R>(env.brk, env.piece, env.c1, env.cell, env.NB, 0, x, y);
+    // the first and last buckets lie outside every cell.  A NaN x goes to the first bucket, where it matches no piece
+    // (fmaxf(NaN, 0) = 0; without it the fp32 form sent NaN to the last bucket and the piece before the last breakpoint)
     int b;
-    if (sizeof(R) == 4) b = __float_as_int(__fadd_rd(fmaf((float)x, (float)env.xbinv, (float)env.xbo), 8388608.f)) - 0x4B000000;
+    if (sizeof(R) == 4) b = min(__float_as_int(__fadd_rd(fmaxf(fmaf((float)x, (float)env.xbinv, (float)env.xbo), 0.f), 8388608.f)) - 0x4B000000, env.nxb - 1);
     else { const R fb = (x - env.xb0) * env.xbinv; b = fb >= (R)0 ? (fb < (R)env.nxb ? (int)fb : env.nxb - 1) : 0; }
-    b = min(max(b, 0), env.nxb - 1);             // the first and last buckets lie outside every cell
     const int e = (int)env.xb[b];
     int lo = (e & 0x7FFF) - 1;                   // last breakpoint left of the bucket (-1: none)
     if (__builtin_expect(e & 0x8000, 0)) return find_cell_rare<R, HAS_XB>(env, lo, x, y);

@@ -63,3 +63,15 @@ def test_product_never_imports_oracle():
             if fn.endswith((".py", ".cu", ".cuh", ".h")):
                 with open(os.path.join(d, fn)) as f:
                     assert not bad.search(f.read()), (d, fn)
+
+
+def test_cost_wrappers_reject_short_mask_and_visited(auvrrt):
+    """auvrrt_cost reads one bin_mask byte per time bin and auvrrt_cost_point one visited byte per habitat: the
+    wrappers refuse shorter lists before the library is called (longer ones stay valid)"""
+    import types
+    import numpy as np
+    env = types.SimpleNamespace(bins=np.zeros((10, 2)), habitats=np.zeros((10, 3)), handle=None)
+    with pytest.raises(ValueError, match="bin_mask"):
+        auvrrt.api.cost(env, [np.zeros((1, 3))], [1.0], [-3.0, -3.0, -4.0], bin_mask=[1] * 9)
+    with pytest.raises(ValueError, match="visited"):
+        auvrrt.api.cost_point(env, np.zeros((1, 2)), [0] * 9, 0, [-3.0, -3.0, -4.0])

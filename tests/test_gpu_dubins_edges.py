@@ -17,6 +17,7 @@ import numpy as np
 import pytest
 
 import envelope_worlds as ew
+from fp32_exact import bound as _bound, f32 as _f32, ring as _ring, table as _table
 
 pytestmark = pytest.mark.gpu
 
@@ -24,8 +25,6 @@ from oracle import orc  # noqa: E402
 
 TOL64 = 1e-9
 RHO = 1.0
-U = 2.0 ** -24          # unit roundoff of fp32
-POLY_TOL = 0.01         # m: a waypoint closer than this to the ring has no certain fp32 polygon answer
 ED_MAX_CTAS = 148 * 12  # the all-pairs launch's grid: at most 12 CTAs of 256 threads per SM
 
 
@@ -60,10 +59,6 @@ def _edges(n, seed, origin=(0.0, 0.0), dist=(2.0, 40.0), circles=None):
     ang, d = rs.uniform(-np.pi, np.pi, n), rs.uniform(dist[0], dist[1], n)
     q1 = np.stack([q0[:, 0] + d * np.cos(ang), q0[:, 1] + d * np.sin(ang), rs.uniform(-np.pi, np.pi, n)], 1)
     return q0, q1
-
-
-def _f32(a):
-    return np.asarray(a, np.float64).astype(np.float32).astype(np.float64)
 
 
 def _near_tie(q0, q1, rho):
@@ -189,47 +184,6 @@ def test_allpairs_rejects_waypoint_counts(api, brute):
 
 
 # ------------------------------------------------------------------------------------ (2) fp32, exact decisions
-def _bound(d, a):
-    """Bound on |q - d^2|, q the fp32 evaluation of the squared distance d^2 between a waypoint p and a circle centre c
-    (both fp32), as the kernels compute it: q = fma(dy, dy, dx * dx) with
-        culled kernel:                    dx = fl(px - cx)                               (a = 0)
-        all-pairs direct formula:         dx = fl(fl(px - ox) - fl(cx - ox)), o = the edge's waypoint 0
-                                                                                          (a = |p - o| + |c - o|)
-    Each difference carries a relative error <= u, so |dx^ - dx| <= e = u (a + d)(1 + 2u), likewise dy.  Then
-        |dx^2 + dy^2 - d^2| <= 2 e (|dx| + |dy|) + 2 e^2 <= 2 sqrt(2) d e + 2 e^2,
-    and the rounded square and the fma add a relative (2u + u^2) of dx^2 + dy^2 <= (d + sqrt(2) e)^2.  The all-pairs
-    kernel's expansion path decides only outside its guard, where it must agree with this (that is what the guard is
-    for); inside, the direct formula decides.  1 % on top for the fp64 evaluation of the bound itself."""
-    e = U * (a + d) * (1 + 2 * U)
-    return 1.01 * (2 * np.sqrt(2) * d * e + 2 * e * e + (2 * U + U * U) * (d + np.sqrt(2) * e) ** 2)
-
-
-def _table(world):
-    """the fp32 circle table (cx, cy, creff2) and ring the kernels read: the running-minimum radius folded in"""
-    h, raw = ew.header(dict(world, habitats=(), bins=(), cells=(), probs=None), "f32")
-    def arr(off, n):
-        return raw[off:off + 4 * n].view(np.float32).astype(np.float64)
-    K, E = h["K"], h["E"]
-    return dict(cx=arr(h["off_cx"], K), cy=arr(h["off_cy"], K), cr=arr(h["off_cr"], K),
-                creff=arr(h["off_creff"], K), creff2=arr(h["off_creff2"], K), px=arr(h["off_px"], E), py=arr(h["off_py"], E))
-
-
-def _ring(t, x, y, tol=POLY_TOL):
-    """crossing-number inside test against the fp32 ring, and whether the point is farther than `tol` from it"""
-    px, py = t["px"], t["py"]
-    inside, dmin = np.zeros(x.shape, bool), np.full(x.shape, np.inf)
-    for i in range(len(px)):
-        ax, ay, bx, by = px[i], py[i], px[(i + 1) % len(px)], py[(i + 1) % len(px)]
-        cross = (ay > y) != (by > y)
-        with np.errstate(divide="ignore", invalid="ignore"):
-            xi = ax + (y - ay) * (bx - ax) / (by - ay)
-        inside ^= cross & (x < xi)
-        ex, ey = bx - ax, by - ay
-        s = np.clip(((x - ax) * ex + (y - ay) * ey) / (ex * ex + ey * ey), 0.0, 1.0)
-        dmin = np.minimum(dmin, np.hypot(x - ax - s * ex, y - ay - s * ey))
-    return inside, dmin > tol
-
-
 def _margins(t, wp, o):
     """m = d^2 - creff2 for every (waypoint, circle) pair of the fp32 inputs (differences of fp32 values are exact in
     fp64; the fp64 squares and sum add at most 2^-51 (d^2 + creff2), added to both bounds), and the two bounds"""
